@@ -19,6 +19,14 @@ text of configs[3]) and the batched search of configs[4] sharded over N replicas
   cpu_baseline = the oracle port (single thread, like divsufsort) on a bounded prefix of the text
   verified     = the benchmarked output checked once, outside the timed region (sab200_check on the GPU,
                  oracle sufcheck on the CPU for the 1 GiB text)
+
+--dump-outputs DIR writes what the timed path returned in its last step as DIR/<name>.npy (float64, exact for
+32-bit values), so that two builds can be compared output for output on the same inputs (the texts and patterns
+are pure functions of their seeds):
+  suffix_array                      the suffix array (n + 1 entries) at sampled positions
+  search_<set>_lo / search_<set>_hi the batched search_all ranges of each pattern set, at sampled queries
+A sample is the sorted distinct positions np.unique(gen.splitmix64(DUMP_SEED, 0, k) % size); an output of at most
+k entries is written whole.  At most 48 MiB in all.
 """
 import argparse
 import ctypes
@@ -46,6 +54,9 @@ WORKLOADS = {
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md, used only if MEASURED_PEAKS.json is absent
 METRIC = "sa_construction_throughput"
 DTYPE = "u8 text / u64 keys / u32 ranks"
+DUMP_SEED = 0xD0D0
+DUMP_SA_ENTRIES = 4 << 20       # 32 MiB of float64
+DUMP_SEARCH_QUERIES = 1 << 19   # 4 MiB per array, four arrays
 
 
 def make_text(workload, n, seed_shift=0):
@@ -70,6 +81,20 @@ def hbm_peak():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return FALLBACK_HBM_GBS, "fallback (B200_PROFILING.md)"
+
+
+def dump_positions(size, k):
+    """The fixed sample of an output of `size` entries that --dump-outputs writes (see the module docstring)."""
+    from suffix_array_b200 import gen
+    if size <= k:
+        return np.arange(size, dtype=np.int64)
+    return np.unique(gen.splitmix64(DUMP_SEED, 0, k) % np.uint64(size)).astype(np.int64)
+
+
+def write_outputs(path, outputs):
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
 
 
 def pinned(n, dtype):
@@ -233,12 +258,13 @@ def search_bytes(bkt, pats, offs, n):
     return algo, sector, int(probes.sum())
 
 
-def bench_search(L, _lib, torch, dev, text, sa, n, ngpus, npat, sample=1_000_000):
+def bench_search(L, _lib, torch, dev, text, sa, n, ngpus, npat, outputs, sample=1_000_000):
     """BASELINE.json configs[4]: batched search_all of `npat` patterns (len 8..64) on the finished index with
     enable_buckets, sharded over `ngpus` replicas (one process, no collective).  Two pattern sets (SURVEY.md 8d):
     half substrings + half hybrids whose second half is random symbols of the text's alphabet, and the
     reference's own hybrid (raw random bytes, benches/utils.rs:193-197).  (lo, hi) of a sample is compared
-    with the oracle's restatement of src/sa.rs:173-204."""
+    with the oracle's restatement of src/sa.rs:173-204.  The host-ABI ranges of the last call go to `outputs`
+    (None: not kept)."""
     from suffix_array_b200 import gen
     from oracle import oracle
     bkt = np.empty(_lib.BKT_LEN, dtype=np.uint32)
@@ -266,6 +292,10 @@ def bench_search(L, _lib, torch, dev, text, sa, n, ngpus, npat, sample=1_000_000
             t0 = time.perf_counter()
             _lib.check(L.sab200_search_all_batch(ix, hp.ctypes.data, ho.ctypes.data, npat, lo.ctypes.data, hi.ctypes.data), "search")
             host_s = min(host_s, time.perf_counter() - t0)
+        if outputs is not None:
+            q = dump_positions(npat, DUMP_SEARCH_QUERIES)
+            outputs["search_%s_lo" % name] = lo[q]
+            outputs["search_%s_hi" % name] = hi[q]
         rec = {"hit_fraction": round(float((hi > lo).mean()), 3), "queries_per_s_host_abi": round(npat / host_s, 1),
                "h2d_bytes": int(pats.size + 8 * offs.size), "d2h_bytes": 8 * npat}
         if ngpus == 1:
@@ -363,6 +393,8 @@ def run_single_c4(args, L, _lib, torch, dev):
         launches += st["kernel_launches"]
     sampler.end()
     sampler.join(timeout=2)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"suffix_array": sa[dump_positions(n + 1, DUMP_SA_ENTRIES)]})
     ver = verify_host(L, _lib, text, sa, n, with_oracle=False)
     d, e = float(np.mean(dev_ms)), float(np.mean(e2e_ms))
     print(json.dumps({
@@ -398,7 +430,13 @@ def main():
     ap.add_argument("--api-gpus", type=int, default=1,
                     help="N=1 process: the ngpus argument of the host-buffer leg, sab200_saca(s, n, sa, ngpus) -- "
                          "one process driving several GPUs through the reference seam")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of what the timed path returned in its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -459,6 +497,10 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     dev_ms = e0.elapsed_time(e1) / args.steps
+    outputs = None
+    if args.dump_outputs:
+        pos = torch.from_numpy(dump_positions(n + 1, DUMP_SA_ENTRIES)).to(dev)
+        outputs = {"suffix_array": d_sa.index_select(0, pos).cpu().numpy().view(np.uint32)}
     # per-launch CUDA events of the radix passes: separate steps (the events cost a few %)
     L.sab200_set_profiling(1)
     pass_ms = pass_bytes = pass_launches = 0
@@ -505,7 +547,9 @@ def main():
     if not args.no_search:
         del d_sa
         torch.cuda.empty_cache()
-        search = bench_search(L, _lib, torch, dev, text, h_sa, n, 1, args.patterns)
+        search = bench_search(L, _lib, torch, dev, text, h_sa, n, 1, args.patterns, outputs)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
 
     cpu = None
     if not args.no_cpu_baseline:
@@ -679,6 +723,9 @@ def run_distributed(args, L, _lib, torch, dist, rank, local_rank, world):
                                                oracle_verify=(args.workload == "c2" and not args.n_mib and not args.no_oracle_verify))
     if rank == 0:
         sampler.join(timeout=2)
+    outputs = None
+    if rank == 0 and args.dump_outputs:  # the suffix array assembled from the slices of the last host-buffer step
+        outputs = {"suffix_array": sa_full[dump_positions(n + 1, DUMP_SA_ENTRIES)]}
     c4 = None
     if args.workload != "c4" and not args.no_c4 and not args.n_mib:
         c4, _ = dist_case(L, _lib, torch, dist, gloo, comm, rank, local_rank, world, "c4", C4_BYTES, 2, 1, None, False)
@@ -696,7 +743,9 @@ def run_distributed(args, L, _lib, torch, dist, rank, local_rank, world):
     dist.barrier()
     search = None
     if rank == 0 and not args.no_search and args.workload == "c2":
-        search = bench_search(L, _lib, torch, dev, text_full, sa_full, n, world, args.patterns)
+        search = bench_search(L, _lib, torch, dev, text_full, sa_full, n, world, args.patterns, outputs)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     dist.barrier()
     peak, peak_src = hbm_peak()
     if rank == 0:
