@@ -128,7 +128,7 @@ int sab_arena_reserve(SabContext* c, size_t bytes) {
 // Status words of one radix pass over `tiles` tiles: one per tile and bin, followed by one per group of
 // SAB_LB_GROUP tiles and bin (two-level look-back).  lookback_tiles counts allocated 256-word rows.
 int sab_ensure_lookback(SabContext* c, size_t tiles) {
-    tiles += tiles / (SAB_LB_GROUP > 0 ? SAB_LB_GROUP : 8) + 2;
+    tiles += tiles / SAB_LB_GROUP + 2;
     if (c->lookback_tiles >= tiles) return SAB_OK;
     if (c->d_lookback) {
         SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));

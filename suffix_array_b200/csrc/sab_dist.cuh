@@ -869,7 +869,7 @@ static int sab_dist_saca(sab200_comm* cm, SabContext* c, DistArena A0, const u8*
         }
         bool lead_barrier = false;  // the first gather is ordered by the row exchange above
         const int rank_bits = sab_ceil_log2_u64(n + 2);
-        bool group_sort_on = SAB_GROUP_SORT != 0;
+        bool group_sort_on = true;  // until most records are in large groups
         u64 h = (u64)k;
         while (tot > 0) {
             ++round;

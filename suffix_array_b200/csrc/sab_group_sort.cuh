@@ -38,9 +38,6 @@
 #ifndef SAB_GSORT_MID
 #define SAB_GSORT_MID 512  // largest group ordered by one warp in registers (64, 128, 256 or 512)
 #endif
-#ifndef SAB_GSORT_DYNAMIC
-#define SAB_GSORT_DYNAMIC 0  // 1: the warps of a tile take the moderate groups from a shared counter (A/B: no gain)
-#endif
 #define SAB_GSORT_THREADS 256
 #define SAB_GSORT_ITEMS 8
 #define SAB_GSORT_TILE (SAB_GSORT_THREADS * SAB_GSORT_ITEMS)
@@ -150,9 +147,6 @@ group_sort_kernel(const u64* __restrict__ kin, const u32* __restrict__ vin, u64 
     u16* s_mid = s_heads + SAB_GSORT_TILE + 8;      // groups of moderate size (all but the tile's last group)
     SAB_SHARED_ARRAY(u32, s_edge, 4);           // tail length, tail group is big, leading records to skip, ... are big
     SAB_SHARED_VAR(u32, s_nmid);
-#if SAB_GSORT_DYNAMIC
-    SAB_SHARED_VAR(u32, s_next);
-#endif
     const u32 tile = blockIdx.x, tid = threadIdx.x, lane = lane_id(), w = warp_id();
     const u64 base = (u64)tile * SAB_GSORT_TILE;
     const u32 valid = (m - base < (u64)SAB_GSORT_TILE) ? (u32)(m - base) : (u32)SAB_GSORT_TILE;
@@ -168,9 +162,6 @@ group_sort_kernel(const u64* __restrict__ kin, const u32* __restrict__ vin, u64 
     if (tid == 0) {
         s_key[0] = base > 0 ? kin[base - 1] : none;
         s_nmid = 0;
-#if SAB_GSORT_DYNAMIC
-        s_next = 0;
-#endif
     }
     // the 32 records behind the tile (warp 0) and the 32 keys in front of it (warp 1) are requested together with
     // the tile: step 2 below normally needs no more than these, so it adds no round trip of its own
@@ -303,17 +294,10 @@ group_sort_kernel(const u64* __restrict__ kin, const u32* __restrict__ vin, u64 
     // the fetched tail of the last group (a group that is small or of moderate size: never "big")
     if (tid < ext) gsort_place(s_key, s_val, s_or2, s_oval, s_heads, valid + tid, (int)G - 1, G, tail_big, lead_big);
 
-    // 4. groups of moderate size: one warp each, in registers
+    // 4. groups of moderate size: one warp each, in registers (taking them from a shared counter instead of
+    // striding by warp measured neutral, r02_ab_final_1gpu.txt _dyn)
     const u32 nmid = s_nmid;
-#if SAB_GSORT_DYNAMIC
-    for (;;) {  // the warps take the groups from a shared counter
-        u32 t = 0;
-        if (lane == 0) t = atomicAdd(&s_next, 1u);
-        t = __shfl_sync(SAB_FULL, t, 0);
-        if (t > nmid) break;
-#else
     for (u32 t = w; t <= nmid; t += SAB_SCAN_WARPS) {
-#endif
         u32 g;
         if (t < nmid) {
             g = s_mid[t];

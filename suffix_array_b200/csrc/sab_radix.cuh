@@ -105,39 +105,8 @@ radix_scan_kernel(const u64* __restrict__ ghist, u64 n, int npass, u64* __restri
 }
 
 // Lanes of the warp holding the same 8-bit digit.  Eight ballots beat the hardware MATCH.ANY
-// instruction here: profiling showed ~45 % of the pass stalled on MATCH results (profiles/).
-#ifndef SAB_MATCH_HW
-#define SAB_MATCH_HW 0
-#endif
-// every SAB_HW_MATCH_EVERY-th item of a thread uses the MATCH unit instead (0 = never): lets the
-// otherwise idle MATCH pipe take part of the ranking work off the issue slots
-#ifndef SAB_HW_MATCH_EVERY
-#define SAB_HW_MATCH_EVERY 0
-#endif
-// tiles per look-back group (two-level status words); 0 = single-level look-back over tiles
-#ifndef SAB_LB_GROUP
-#define SAB_LB_GROUP 8
-#endif
-#ifndef SAB_LB_DEPTH
-#define SAB_LB_DEPTH 4
-#endif
-// 1: a record goes to its shared-memory slot as soon as it is ranked (the slot does not depend on the
-// look-back), so the ranks[] array and one block barrier disappear and keys[] / vals[] die item by item:
-// no register spills under __launch_bounds__(256, 3).  0: rank all items, look back, then scatter (round 1).
-#ifndef SAB_FUSED_SCATTER
-#define SAB_FUSED_SCATTER 1
-#endif
-// 1: the ballot matching runs ONCE, in the histogram phase: the leader's atomic returns the first slot of the
-// digit group inside the warp's share of the bin, every lane keeps its 10-bit local rank, and after the block
-// scan the final slot is one shared-memory read (warp offset of the bin) + the local rank.  0: plain atomics
-// for the histogram, matching in the ranking phase.
-#ifndef SAB_RANK_ONCE
-#define SAB_RANK_ONCE 0
-#endif
+// instruction here: profiling showed ~45 % of the pass stalled on MATCH results (profiles/r01_variants.md §2).
 __device__ __forceinline__ u32 match_digit(u32 d) {
-#if SAB_MATCH_HW
-    return __match_any_sync(SAB_FULL, d);
-#else
     u32 peers = SAB_FULL;
 #pragma unroll
     for (int bit = 0; bit < SAB_RADIX_BITS; ++bit) {
@@ -146,8 +115,14 @@ __device__ __forceinline__ u32 match_digit(u32 d) {
         peers &= p ? m : ~m;
     }
     return peers;
-#endif
 }
+
+// tiles per look-back group (two-level status words); the single-level look-back over tiles measured
+// slower, profiles/r01_variants.md §3b
+#define SAB_LB_GROUP 8
+#ifndef SAB_LB_DEPTH
+#define SAB_LB_DEPTH 4
+#endif
 
 // ------------------------------------------------------------------ one onesweep pass
 template <typename KeyT, bool HAS_VAL, bool IOTA_VAL, int THREADS, int ITEMS>
@@ -267,9 +242,6 @@ onesweep_kernel(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out, c
     // ---- load (warp-striped: item k of lane l is record w*WTILE + k*32 + l of the tile)
     KeyT keys[ITEMS];
     u32 vals[ITEMS];
-#if !SAB_FUSED_SCATTER
-    u32 ranks[ITEMS];
-#endif
     const u32 wofs = w * WTILE + lane;
     const KeyT* kin = keys_in + tile_base + wofs;
     const u32* vin = IOTA_VAL ? nullptr : vals_in + tile_base + wofs;
@@ -295,32 +267,15 @@ onesweep_kernel(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out, c
     // ---- tile histogram first (plain shared-memory atomics, order irrelevant), so the tile's partial is
     // published a whole ranking phase before its successors look back: they never find it missing.
     u32* wh = s_whist + w * SAB_RADIX_BINS;
-#if SAB_RANK_ONCE
-    u32 lrank[(ITEMS + 1) / 2];  // two 16-bit local ranks (position inside the warp's share of the bin) per word
-#pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
-        const u32 d = dop(keys[k]);
-        const u32 peers = match_digit(d);
-        const u32 leader = (u32)(__ffs((int)peers) - 1);
-        u32 old = 0;
-        if (lane == leader) old = atomicAdd(&wh[d], (u32)__popc(peers));  // same-address atomics of a warp retire in order
-        old = __shfl_sync(SAB_FULL, old, (int)leader) + (u32)__popc(peers & lanemask_lt());
-        if (k & 1) lrank[k / 2] |= old << 16;
-        else lrank[k / 2] = old;
-    }
-#else
 #pragma unroll
     for (int k = 0; k < ITEMS; ++k) atomicAdd(&wh[dop(keys[k])], 1u);
-#endif
     __syncthreads();
     u32 my_count = 0;
     u64* lb = lookback + (u64)tile * SAB_RADIX_BINS + tid;
     const u64 etag = (u64)epoch << SAB_LB_EPOCH_SHIFT;
-#if SAB_LB_GROUP
     const u32 grp = tile / SAB_LB_GROUP, gr = tile % SAB_LB_GROUP;
     // group status words live behind the tile status words of this launch
     u64* lb2 = lookback + ((n + (u64)TILE - 1) / (u64)TILE + grp) * SAB_RADIX_BINS + tid;
-#endif
     if (tid < SAB_RADIX_BINS) {
         u32 run = 0;
 #pragma unroll
@@ -330,7 +285,6 @@ onesweep_kernel(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out, c
             run += c;
         }
         my_count = run;
-#if SAB_LB_GROUP
         // Two-level status: tile partials (never upgraded) + one word per group of SAB_LB_GROUP tiles, owned by
         // the group's last tile: PARTIAL = sum of the group's tile counts (published here, early), later
         // INCLUSIVE = prefix through the end of the group.  A look-back is then the tile's in-group
@@ -354,9 +308,6 @@ onesweep_kernel(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out, c
             } while (!ok);
             st_relaxed_u64(lb2, etag | (grp == 0 ? SAB_LB_FLAG_INCLUSIVE : SAB_LB_FLAG_PARTIAL) | (agg + (u64)my_count));
         }
-#else
-        st_relaxed_u64(lb, etag | (tile == 0 ? SAB_LB_FLAG_INCLUSIVE : SAB_LB_FLAG_PARTIAL) | (u64)my_count);
-#endif
     }
     // block-exclusive scan of the 256 bin counts; the bin start is folded into the per-warp offsets, so
     // the ranking atomics below return final shared-memory slots
@@ -378,27 +329,17 @@ onesweep_kernel(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out, c
 #pragma unroll
     for (int k = 0; k < ITEMS; ++k) {
         const u32 d = dop(keys[k]);
-#if SAB_RANK_ONCE
-        const u32 pos = wh[d] + ((k & 1) ? (lrank[k / 2] >> 16) : (lrank[k / 2] & 0xffffu));
-#else
-        const u32 peers = (SAB_HW_MATCH_EVERY > 0 && (k % (SAB_HW_MATCH_EVERY > 0 ? SAB_HW_MATCH_EVERY : 1)) == 0)
-                              ? __match_any_sync(SAB_FULL, d)
-                              : match_digit(d);
+        const u32 peers = match_digit(d);
         const u32 leader = (u32)(__ffs((int)peers) - 1);
         // Atomics of one warp on one address retire in program order, so item k+1 sees item k's update.
         u32 old = 0;
         if (lane == leader) old = atomicAdd(&wh[d], (u32)__popc(peers));
         old = __shfl_sync(SAB_FULL, old, (int)leader);
         const u32 pos = old + (u32)__popc(peers & lanemask_lt());
-#endif
-#if SAB_FUSED_SCATTER
+        // staged as soon as ranked; a scatter loop after the look-back measured slower, r02_ab_radix_variants.txt _unf
         s_keys[pos] = keys[k];
         if (HAS_VAL) s_vals[pos] = vals[k];
-#else
-        ranks[k] = pos;
-#endif
     }
-#if SAB_LB_GROUP
     // ---- two-level look-back, one lane per bin: in-group tile partials and the first batch of group words
     // are requested together, so the common case is a single L2 round trip
     if (tid < SAB_RADIX_BINS) {
@@ -452,52 +393,10 @@ onesweep_kernel(const KeyT* __restrict__ keys_in, KeyT* __restrict__ keys_out, c
             }
             if (gr == SAB_LB_GROUP - 1 && grp > 0) st_relaxed_u64(lb2, etag | SAB_LB_FLAG_INCLUSIVE | (excl + (u64)my_count));
         }
-        s_goff[tid] = (u32)(gbase[tid] + excl) - my_start;
-    }
-    __syncthreads();
-#else
-    // ---- decoupled look-back, one lane per bin
-    if (tid < SAB_RADIX_BINS) {
-        u64 excl = 0;
-        if (tile > 0) {
-            // Walk the predecessors SAB_LB_DEPTH at a time: the status loads of one batch are independent,
-            // so a long chain of PARTIAL tiles costs one L2 round trip per batch instead of one per tile.
-            i64 t = (i64)tile - 1;
-            bool done = false;
-            while (!done) {
-                u64 v[SAB_LB_DEPTH];
-#pragma unroll
-                for (int j = 0; j < SAB_LB_DEPTH; ++j)
-                    v[j] = (t - j >= 0) ? ld_relaxed_u64(lookback + (u64)(t - j) * SAB_RADIX_BINS + tid) : 0ull;
-#pragma unroll
-                for (int j = 0; j < SAB_LB_DEPTH; ++j) {
-                    if (done) break;
-                    const u64 f = v[j] & SAB_LB_FLAG_MASK;
-                    if ((v[j] >> SAB_LB_EPOCH_SHIFT) != (u64)epoch || f == 0) break;  // not published yet: reload from here
-                    excl += v[j] & SAB_LB_VALUE_MASK;
-                    --t;
-                    if (f == SAB_LB_FLAG_INCLUSIVE) done = true;
-                }
-                if (!done) SAB_SPIN_PAUSE();
-            }
-            st_relaxed_u64(lb, etag | SAB_LB_FLAG_INCLUSIVE | (excl + (u64)my_count));
-        }
         // record indices are < 2^32 (N <= 2^32 - 1): keep the per-bin offset as a wrapping u32
         s_goff[tid] = (u32)(gbase[tid] + excl) - my_start;
     }
     __syncthreads();
-
-#endif
-#if !SAB_FUSED_SCATTER
-    // ---- scatter into shared memory in sorted order
-#pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
-        const u32 pos = ranks[k];
-        s_keys[pos] = keys[k];
-        if (HAS_VAL) s_vals[pos] = vals[k];
-    }
-    __syncthreads();
-#endif
 
     // ---- coalesced write-out: consecutive shared slots of one bin are consecutive in global memory
     if (full) {

@@ -29,20 +29,12 @@
 // The bucket directory of the lazy inverse suffix array has 2^(ceil(log2 n) - SAB_DIR_SHIFT) entries (at most
 // 2^28): ~2^SAB_DIR_SHIFT sorted keys per entry for the gallop + bisect that follows the jump.  Measured on the
 // 1 GiB DNA-like text (profiles/r02_ab_round2.txt): shift 4 -> 2 takes the gathers from 6.9 to 6.2 ms.
-#ifndef SAB_GS_REQUIRE_SORTED
-#define SAB_GS_REQUIRE_SORTED 0  // debugging aid: 1 = the in-group sort only runs on lists ascending in r1
-#endif
 #ifndef SAB_DIR_SHIFT
 #define SAB_DIR_SHIFT 2
 #endif
 
 #define SAB_RANK_EMPTY 0xffffffffu
 #define SAB_PAD(o) ((o) + ((o) >> 5))  // shared-memory padding, one word per 32; NB: evaluates its argument twice
-// 1: the records of a round are ordered inside their groups by sab_group_sort (one sweep + a radix sort
-// of the large groups only) instead of a radix sort of every record
-#ifndef SAB_GROUP_SORT
-#define SAB_GROUP_SORT 1
-#endif
 #ifdef SAB_EMU
 #ifndef SAB_FILTER_MIN
 #define SAB_FILTER_MIN ((u64)3000)
@@ -225,8 +217,7 @@ static int sab_launch_pack(SabContext* c, const u8* d_text, u64 n, u64 count, co
     const int ka = (k + 1) / 2;
     unsigned __int128 lim = 1;
     for (int t = 0; t < ka; ++t) lim *= base;
-    const char* off = getenv("SAB_PACK_SPLIT");
-    if (k >= 2 && ka <= 32 && lim < ((unsigned __int128)1 << 32) && !(off && off[0] == '0')) {
+    if (k >= 2 && ka <= 32 && lim < ((unsigned __int128)1 << 32)) {
         const u32 wtop = (u32)sab_pow_u64(base, ka - 1);
         const u32 wmul = (u32)sab_pow_u64(base, (k & 1) ? ka - 1 : ka);
         SAB_LAUNCH(pack_keys_split_kernel, (unsigned)div_up64(count, SAB_PACK_TILE), SAB_PACK_THREADS, 0, c->stream, d_text, n, count,
@@ -643,7 +634,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     const int rank_bits = sab_ceil_log2_u64(n + 2);
     // the split filter (5c) pays off while few groups split: repetitive texts, early rounds
     bool filter_on = (z.sorted_keys == nullptr) && m >= SAB_FILTER_MIN;
-    bool group_sort_on = SAB_GROUP_SORT != 0;
+    bool group_sort_on = true;  // 5d, until most records are in large groups
     // The active list leaves init_ranks ascending in r1.  A round of the split filter parks the unsplit
     // groups in front of the re-ranked ones, so the next list is two ascending runs: groups stay contiguous
     // (all the scan kernels need) but the list is no longer monotone -- sab_group_sort is told, because it
@@ -696,7 +687,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
             // 5d. small groups are ordered in one sweep; the spare buffers for the records of big groups are
             // the unused tails of the round buffers (keys, payloads) and of r1buf (positions)
             int sorted = 0;
-            if (group_sort_on && (list_sorted || !SAB_GS_REQUIRE_SORTED)) {
+            if (group_sort_on) {
                 const u64 used = sab_align_up(n_sort, 64);
                 const u64 cap_keys = key_cap > used ? key_cap - used : 0;
                 const u64 cap_vals = n + 8 > n_stay + used ? n + 8 - n_stay - used : 0;

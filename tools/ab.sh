@@ -1,6 +1,6 @@
 #!/bin/bash
 # developer tool: A/B the variant builds of libsab200 on one box (device-resident bench)
-#   AB_VARIANTS="_gs0 _x"  suffixes of suffix_array_b200/libsab200<suffix>.so (built with `make variant`)
+#   AB_VARIANTS="_i16 _x"  suffixes of suffix_array_b200/libsab200<suffix>.so (built with `make variant`)
 #   AB_MIB=256  AB_WORKLOAD=c2
 for v in "" ${AB_VARIANTS}; do
   lib=suffix_array_b200/libsab200$v.so
