@@ -427,45 +427,6 @@ static int32_t saca_host(const uint8_t* s, uint64_t n, uint32_t* sa, uint32_t* b
 }  // extern "C"
 
 // ---- buckets -------------------------------------------------------------------------------
-static int buckets_device(SabContext* c, const u8* d_text, u64 n, u32* d_bkt) {
-    cudaStream_t st = c->stream;
-    SAB_CUDA_TRY(cudaMemsetAsync(d_bkt, 0, SAB_BKT_LEN * sizeof(u32), st));
-    if (n > 0) {
-        u32* d_hist = c->d_counters + 16;
-        SAB_CUDA_TRY(cudaMemsetAsync(d_hist, 0, 256 * sizeof(u32), st));
-        u64 blocks = div_up64(n, 256 * 64);
-        const u64 bmax = (u64)c->sm_count * 8;
-        if (blocks > bmax) blocks = bmax;
-        SAB_LAUNCH(alphabet_hist_kernel, (unsigned)blocks, 256, 0, st, d_text, n, d_hist);
-        SAB_LAUNCH_CHECK();
-        SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small + 64, d_hist, 256 * sizeof(u32), cudaMemcpyDeviceToHost, st));
-        SAB_CUDA_TRY(cudaStreamSynchronize(st));
-        u16 lut[256];
-        u32 sigma = 0;
-        for (int ch = 0; ch < 256; ++ch) {
-            if (c->h_small[64 + ch]) ++sigma;
-            lut[ch] = (u16)(c->h_small[64 + ch] ? sigma : 0);
-        }
-        u16* d_lut = (u16*)(c->d_counters + 16 + 256);
-        memcpy(c->h_small + 384, lut, sizeof(lut));
-        SAB_CUDA_TRY(cudaMemcpyAsync(d_lut, c->h_small + 384, sizeof(lut), cudaMemcpyHostToDevice, st));
-        const size_t tab_bytes = (size_t)sigma * (sigma + 1) * sizeof(u32);
-        const int dense = tab_bytes <= 160 * 1024;
-        const size_t smem = dense ? tab_bytes : 0;
-#ifndef SAB_EMU
-        SAB_CUDA_TRY(cudaFuncSetAttribute(bucket_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-#endif
-        u64 pblocks = div_up64(n, 256 * 64);
-        const u64 pmax = (u64)c->sm_count * (smem > 64 * 1024 ? 1 : 4);
-        if (pblocks > pmax) pblocks = pmax;
-        SAB_LAUNCH(bucket_pairs_kernel, (unsigned)pblocks, 256, smem, st, d_text, n, (const u16*)d_lut, sigma, dense, d_bkt);
-        SAB_LAUNCH_CHECK();
-    }
-    SAB_LAUNCH(bucket_scan_kernel, 1, 1024, 0, st, d_bkt);
-    SAB_LAUNCH_CHECK();
-    return SAB_OK;
-}
-
 extern "C" int32_t sab200_enable_buckets(const uint8_t* s, uint64_t n, uint32_t* bkt) {
     if (!bkt || (n > 0 && !s) || n > SAB200_MAX_LENGTH) {
         sab_set_error("sab200_enable_buckets: bad arguments");
@@ -476,12 +437,14 @@ extern "C" int32_t sab200_enable_buckets(const uint8_t* s, uint64_t n, uint32_t*
     std::lock_guard<std::mutex> lk(c->mu);
     SAB_CUDA_TRY(cudaSetDevice(c->device));
     const size_t text_bytes = sab_align_up((size_t)n + 64, 256);
-    SAB_TRY(sab_arena_reserve(c, text_bytes + SAB_BKT_LEN * sizeof(u32) + 1024));
+    SAB_TRY(sab_arena_reserve(c, text_bytes + SAB200_BKT_LEN * sizeof(u32) + 1024));
     u8* d_s = (u8*)c->arena;
     u32* d_bkt = (u32*)(c->arena + text_bytes);
     if (n) SAB_CUDA_TRY(cudaMemcpyAsync(d_s, s, n, cudaMemcpyHostToDevice, c->stream));
-    SAB_TRY(buckets_device(c, d_s, n, d_bkt));
-    SAB_CUDA_TRY(cudaMemcpyAsync(bkt, d_bkt, SAB_BKT_LEN * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+    SabAlphabet al = {};
+    if (n) SAB_TRY(sab_alphabet_local(c, d_s, n, &al));
+    SAB_TRY(sab_pair_buckets(c, d_s, n, al.d_lut, al.sigma, d_bkt));
+    SAB_CUDA_TRY(cudaMemcpyAsync(bkt, d_bkt, SAB200_BKT_LEN * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
     SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
     return SAB_OK;
 }
@@ -664,8 +627,8 @@ static int replica_init(SabReplica& r, int device, const u8* s, u64 n, const u32
     if (n) SAB_CUDA_TRY(cudaMemcpyAsync(r.d_text, s, n, cudaMemcpyHostToDevice, st));
     SAB_CUDA_TRY(cudaMemcpyAsync(r.d_sa, sa, ((size_t)n + 1) * sizeof(u32), cudaMemcpyHostToDevice, st));
     if (bkt) {
-        SAB_CUDA_TRY(cudaMalloc(&r.d_bkt, SAB_BKT_LEN * sizeof(u32)));
-        SAB_CUDA_TRY(cudaMemcpyAsync(r.d_bkt, bkt, SAB_BKT_LEN * sizeof(u32), cudaMemcpyHostToDevice, st));
+        SAB_CUDA_TRY(cudaMalloc(&r.d_bkt, SAB200_BKT_LEN * sizeof(u32)));
+        SAB_CUDA_TRY(cudaMemcpyAsync(r.d_bkt, bkt, SAB200_BKT_LEN * sizeof(u32), cudaMemcpyHostToDevice, st));
     }
     SAB_CUDA_TRY(cudaStreamSynchronize(st));
     memset(&r.pd, 0, sizeof(r.pd));

@@ -192,12 +192,23 @@ dist_lazy_fill_kernel(const u32* __restrict__ slot, const u32* __restrict__ rank
 }
 
 // ------------------------------------------------------------------ host helpers
-static inline unsigned sab_grid(SabContext* c, u64 n, u64 per_block, int waves) {
-    u64 g = div_up64(n, per_block);
-    const u64 gmax = (u64)c->sm_count * (u64)waves;
-    if (g > gmax) g = gmax;
-    return (unsigned)(g ? g : 1);
+// Rank g of P owns the text positions [lo, hi), B = ceil(n / P) of them (the last ranks fewer, or none).  Its shard
+// holds len readable bytes from lo on: its own positions and SAB200_SHARD_HALO bytes of the next shard, cut at n.
+struct ShardBounds {
+    u64 B, lo, hi, len;
+};
+static inline ShardBounds sab_shard_bounds(u64 n, int P, int g) {
+    ShardBounds s;
+    s.B = n ? div_up64(n, (u64)P) : 1;
+    s.lo = (u64)g * s.B < n ? (u64)g * s.B : n;
+    s.hi = s.lo + s.B < n ? s.lo + s.B : n;
+    s.len = (n - s.lo) < (s.hi - s.lo) + SAB200_SHARD_HALO ? (n - s.lo) : (s.hi - s.lo) + SAB200_SHARD_HALO;
+    return s;
 }
+
+// Directory shift of the lazy inverse suffix array on a multi-GPU rank.  One GPU uses SAB_DIR_SHIFT = 2; that value
+// was measured on one GPU only, so the multi-GPU driver keeps its own.
+#define SAB_DIST_DIR_SHIFT 4
 
 // Plans one variable all-to-all with a single host synchronisation:
 //   per-destination counts of keys[0..count) (count read from *d_count32 when given; `count` is then its bound)
@@ -234,17 +245,6 @@ static int sab_plan_exchange(sab200_comm* cm, SabContext* c, const KeyT* d_keys,
         pl->rtotal += pl->rcount[d];
     }
     return SAB_OK;
-}
-
-// host mirror of RankLayout::owner / slot (sab_radix.cuh)
-static inline u32 sab_layout_owner_host(const RankLayout& L, u64 q) {
-    if (L.cyc) return (u32)((q >> L.shift) % (L.pmax + 1u));
-    const u32 o = (u32)(q / L.B);
-    return o < L.pmax ? o : L.pmax;
-}
-static inline u64 sab_layout_slot_host(const RankLayout& L, u64 q, u32 o) {
-    if (L.cyc) return (((q >> L.shift) / (L.pmax + 1u)) << L.shift) | (q & (u64)(L.B - 1u));
-    return q - (u64)o * L.B;
 }
 
 // Two-ended bump allocator over the context arena: long-lived arrays grow from the bottom, the temporaries of
@@ -408,19 +408,66 @@ static int sab_peers_update(sab200_comm* cm, SabContext* c, const u64* rows, int
 }
 #endif
 
+// Phases of a construction: the indices of sab200_dist_stats::phase_ms (include/sab200.h); PH_END closes the last one
+enum DistPhase {
+    PH_ALPHABET, PH_SPLITTERS, PH_PARTITION, PH_KEY_EXCHANGE, PH_LOCAL_SORT, PH_INIT_RANKS, PH_RANKS_TO_OWNERS, PH_REBALANCE,
+    PH_REQUESTS, PH_LAZY, PH_ROUND_SORT, PH_RERANK, PH_RANK_UPDATES, PH_NEW_SA, PH_H2D, PH_D2H, PH_END = -1
+};
+static_assert(PH_D2H + 1 == SAB200_PHASES, "one phase per slot of sab200_dist_stats::phase_ms");
+
+// One rank's construction, phase by phase (sab_dist_saca runs them; the file header numbers the steps).  The
+// members are what one phase leaves for the later ones.
 struct DistRun {
     sab200_comm* cm;
     SabContext* c;
+    cudaStream_t st;
+    sab200_dist_stats* ds;
     DistArena A;
+    size_t top0;  // A.hi at the start: the temporaries of the key exchange are released down to it
+    int P, g;
+    u64 n;
+    ShardBounds sh;  // this rank's text positions
+    u64 count;       // own positions: sh.hi - sh.lo
+    const u8* d_text;
     DistPhases ph;
+    SabAlphabet al;
+    SplitterDigit sdop;  // slice that holds a key
+    SliceDigit slices;   // slice that holds an SA position
+    u64 R, sa_off;       // this rank's slice: SA positions [sa_off, sa_off + R)
+    bool fused;          // the key exchange went peer to peer (so can the rounds)
+    // 5, 6: the slice, its sorted keys and bucket directory (dir[0] is entry dlo), the active list (r1buf, rb.v)
+    SortBuffers<u64> buf;
+    u32 *sa_local, *r1buf, *rank_seq, *dir;
+    const u64* sortedK;
+    const u32* sortedI;
+    u64 dlo;
+    int dir_shift;
+    u64 m, tot;  // active records here / over all ranks
+    // 7: rank[] at the owners; the buffers of the rounds
+    bool lazy = false, rebalanced = false;
+    int layout_cyc = 0;
     RankLayout lay;
-    u32* rank_local;
-    u64 lo;  // first text position of this rank
+    u32* rank_local = nullptr;
+    SortBuffers<u64> rb;
+    u64 key_cap, val_cap;  // records each key / payload buffer of rb can hold
+    bool p2p_ready = false;  // 7c: peer-to-peer rounds
+    bool lead_barrier = false;  // the first gather is ordered by the row exchange of the peer table
+    P2PTable pt;
+    bool group_sort_on = true;  // the in-group sort, until most records are in large groups
+    // the current round: what the re-rank leaves for the new SA entries and the rank updates
+    u32 *upd_idx, *upd_r, *set_pos;
+    const u32* sorted_idx;
+    int sorted_in;  // which of the two index buffers holds the sorted list
+
+    DistRun(sab200_comm* cm_, SabContext* c_, sab200_dist_stats* ds_, DistArena A0, const u8* text, u64 n_)
+        : cm(cm_), c(c_), st(c_->stream), ds(ds_), A(A0), top0(A0.hi), P(cm_->P), g(cm_->rank), n(n_),
+          sh(sab_shard_bounds(n_, cm_->P, cm_->rank)), count(sh.hi - sh.lo), d_text(text) { ph.c = c_; }
+
+    static constexpr int PTILE = PassShape<u64>::THREADS * PassShape<u64>::ITEMS;
 
     // rank[idx[t]] = val[t] on the GPU that owns text position idx[t]; records with idx = 0xFFFFFFFF are dropped.
     // d_extra32 / rows: nd device-side u32 values ride along with the count exchange (rows[s*(P+nd) + P + e]).
     int send_ranks(const u32* idx, const u32* val, u64 cnt, const u32* d_extra32 = nullptr, int nd = 0, u64* rows = nullptr) {
-        cudaStream_t st = c->stream;
         const size_t mark = A.hi;
         u32* kp = A.top<u32>(cnt + 8);
         u32* vp = A.top<u32>(cnt + 8);
@@ -441,262 +488,197 @@ struct DistRun {
         SAB_TRY(sab_comm_exchange(cm, st, pl, vp, rr, sizeof(u32)));
         if (pl.rtotal) {
             SAB_LAUNCH(dist_scatter_kernel, (unsigned)div_up64(pl.rtotal, 256), 256, 0, st, (const u32*)ri, (const u32*)rr, pl.rtotal,
-                       (u32)lo, lay, rank_local);
+                       (u32)sh.lo, lay, rank_local);
             SAB_LAUNCH_CHECK();
             c->stats.kernel_launches++;
         }
         A.hi = mark;
         return SAB_OK;
     }
-};
 
-// d_text: this rank's shard + halo on the device (text_len bytes).  The arena `A0` starts behind whatever the
-// caller placed at its bottom.  Enqueues on c->stream; the stream is idle when the function returns.
-static int sab_dist_saca(sab200_comm* cm, SabContext* c, DistArena A0, const u8* d_text, u64 text_len, u64 n, DistResult* res,
-                         sab200_dist_stats* ds) {
-    const int P = cm->P, g = cm->rank;
-    cudaStream_t st = c->stream;
-    SabStats& S = c->stats;
-    S.n = n;
-    cm->bytes_sent = 0;
-    cm->collectives = 0;
-    const u64 B = n ? div_up64(n, (u64)P) : 1;
-    const u64 lo = (u64)g * B < n ? (u64)g * B : n;
-    const u64 hi = lo + B < n ? lo + B : n;
-    const u64 count = hi - lo;
-    res->d_slice = nullptr;
-    res->slice_len = 0;
-    res->sa_off = 1;
-    ds->nranks = (u32)P;
-    ds->rank = (u32)g;
-    if (n == 0) return SAB_OK;  // the suffix array is the sentinel alone
-    const u64 avail = (n - lo) < count + SAB200_SHARD_HALO ? (n - lo) : count + SAB200_SHARD_HALO;
-    if (text_len < avail) {
-        sab_set_error("rank %d: shard of %llu bytes, need %llu (own positions + halo)", g, (unsigned long long)text_len,
-                      (unsigned long long)avail);
-        return SAB_ERR_ARGS;
-    }
-    DistRun R_;
-    R_.cm = cm;
-    R_.c = c;
-    R_.A = A0;
-    R_.ph.c = c;
-    R_.lo = lo;
-    R_.rank_local = nullptr;
-    DistArena& A = R_.A;
-    DistPhases& ph = R_.ph;
-    SAB_TRY(sab_ensure_scan(c, (size_t)div_up64(count + count / 2 + 4096, SAB_GSORT_TILE)));
-
-    // ---- 1. common alphabet / key shape
-    ph.mark(0);
-    u32* d_h32 = c->d_counters + 16;
-    SAB_CUDA_TRY(cudaMemsetAsync(d_h32, 0, 256 * sizeof(u32), st));
-    if (count) {
-        SAB_LAUNCH(alphabet_hist_kernel, sab_grid(c, count, 256 * 64, 8), 256, 0, st, d_text, count, d_h32);
+    // ---- 1. common alphabet / key shape: the byte histograms of all shards add up
+    int alphabet() {
+        ph.mark(PH_ALPHABET);
+        u32* d_h32 = c->d_counters + 16;
+        SAB_TRY(sab_launch_alphabet_hist(c, d_text, count, d_h32));
+        SAB_LAUNCH(hist_widen_kernel, 1, 256, 0, st, (const u32*)d_h32, c->d_ghist);
         SAB_LAUNCH_CHECK();
-        S.kernel_launches++;
-    }
-    SAB_LAUNCH(hist_widen_kernel, 1, 256, 0, st, (const u32*)d_h32, c->d_ghist);
-    SAB_LAUNCH_CHECK();
-    SAB_TRY(sab_comm_all_reduce_u64(cm, st, c->d_ghist, 256));
-    u64* h64 = (u64*)(c->h_small + 1024);
-    SAB_CUDA_TRY(cudaMemcpyAsync(h64, c->d_ghist, 256 * sizeof(u64), cudaMemcpyDeviceToHost, st));
-    SAB_CUDA_TRY(cudaStreamSynchronize(st));
-    u16 lut[256];
-    u32 sigma = 0, base = 2;
-    int k = 1, key_bits = 1;
-    {
-        u64 hh[256];
-        memcpy(hh, h64, sizeof(hh));
-        sab_plan_alphabet(hh, n, lut, &sigma, &base, &k, &key_bits);
-    }
-    S.sigma = sigma;
-    S.bits_per_symbol = (u32)sab_ceil_log2_u64(base);
-    S.symbols_per_key = (u32)k;
-    u16* d_lut = (u16*)(c->d_counters + 16 + 256);
-    memcpy(c->h_small + 384, lut, sizeof(lut));
-    SAB_CUDA_TRY(cudaMemcpyAsync(d_lut, c->h_small + 384, sizeof(lut), cudaMemcpyHostToDevice, st));
-
-    // ---- 2. keys of own positions, splitters from a sample
-    ph.mark(1);
-    u64* keysA = A.top<u64>(count + 8);
-    SAB_ARENA_CHECK(A);
-    if (count) {
-        sab_prof_begin(c, 2);
-        SAB_TRY(sab_launch_pack(c, d_text, avail, count, (const u16*)d_lut, base, k, keysA));
-        sab_prof_end(c);
-    }
-    u64 splitters[SAB_MAX_RANKS];
-    for (int i = 0; i < SAB_MAX_RANKS; ++i) splitters[i] = ~0ull;
-    if (P > 1) {
-        // ~8 Ki samples over all ranks (slice sizes within a few per cent); the pool is sorted on the host
-        const u32 NS = 8192 / (u32)P < 512 ? 512u : (8192 / (u32)P > 2048 ? 2048u : 8192 / (u32)P);
-        const u64 step = count / NS ? count / NS : 1;
-        u64* d_sample = cm->d_small;
-        SAB_LAUNCH(sample_keys_kernel, (NS + 255) / 256, 256, 0, st, (const u64*)keysA, count, step, NS, d_sample);
-        SAB_LAUNCH_CHECK();
-        SAB_TRY(sab_comm_all_gather(cm, st, d_sample, d_sample + (NS + 1), (NS + 1) * sizeof(u64)));
-        SAB_CUDA_TRY(cudaMemcpyAsync(cm->h_small, d_sample + (NS + 1), (size_t)P * (NS + 1) * sizeof(u64), cudaMemcpyDeviceToHost, st));
+        SAB_TRY(sab_comm_all_reduce_u64(cm, st, c->d_ghist, 256));
+        u64* h64 = (u64*)(c->h_small + 1024);
+        SAB_CUDA_TRY(cudaMemcpyAsync(h64, c->d_ghist, 256 * sizeof(u64), cudaMemcpyDeviceToHost, st));
         SAB_CUDA_TRY(cudaStreamSynchronize(st));
-        std::vector<u64> pool;
-        pool.reserve((size_t)P * NS);
-        for (int r = 0; r < P; ++r) {
-            const u64* row = cm->h_small + (size_t)r * (NS + 1);
-            const u64 have = row[NS] <= NS ? row[NS] : NS;
-            pool.insert(pool.end(), row, row + have);
-        }
-        std::sort(pool.begin(), pool.end());
-        for (int i = 0; i + 1 < P; ++i) {
-            size_t at = (size_t)(i + 1) * pool.size() / (size_t)P;
-            if (at >= pool.size()) at = pool.size() - 1;
-            splitters[i] = pool.empty() ? 0 : pool[at];
-        }
+        return sab_plan_alphabet(c, h64, n, &al);
     }
 
-    // ---- 3. partition by destination (digit = number of splitters <= key), payload = global position
-    ph.mark(2);
-    SplitterDigit sdop;
-    sdop.np = P - 1;
-    for (int i = 0; i < SAB_MAX_RANKS - 1; ++i) sdop.s[i] = i < P - 1 ? splitters[i] : ~0ull;
-    A2APlan pk;
-    u64 mat[SAB_MAX_RANKS * SAB_MAX_RANKS];
-    // the count exchange also carries what the peers need to address this rank's receive buffers directly
-    // (fused exchange, below): process, device, arena, offset of the key buffer inside it
-    const u64 k0_off = sab_align_up(A.lo, 256);
-    u64 extra[5] = {(u64)getpid(), (u64)c->device, (u64)(uintptr_t)c->arena, (u64)c->arena_bytes, k0_off};
-    constexpr int NX = 5;
-    u64 rows[SAB_MAX_RANKS * 32];
-    SAB_TRY((sab_plan_exchange<u64, SplitterDigit>(cm, c, keysA, count, nullptr, sdop, nullptr, 0, extra, NX, &pk, rows)));
-    const int W = P + NX;
-    for (int s = 0; s < P; ++s)
-        for (int d = 0; d < P; ++d) mat[(size_t)s * P + d] = rows[(size_t)s * W + d];
-    const u64 R = pk.rtotal;
-    u64 sa_off = 1;
-    for (int r = 0; r < g; ++r)
-        for (int s = 0; s < P; ++s) sa_off += mat[(size_t)s * P + r];
-    constexpr int PTILE = PassShape<u64>::THREADS * PassShape<u64>::ITEMS;
-    SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64((count > R ? count : R) + 1, PTILE)));
-    SAB_TRY(sab_ensure_scan(c, (size_t)div_up64(R + 4096, SAB_GSORT_TILE)));
-    u64* K0 = A.bot<u64>(R + 8);
-    u32* V0 = A.bot<u32>(R + 8);
-    SAB_ARENA_CHECK(A);
-    bool fused = false;
-#ifndef SAB_EMU
-    if (P > 1 && cm->kind == 0 && sab_env_int("SAB_DIST_P2P", 1) != 0) {
-        SAB_TRY(sab_peers_update(cm, c, rows, W));
-        fused = cm->peers_ok;
-    }
-#endif
-    if (fused) {
-        // ---- 3+4 fused: the partition pass stores every record straight into its destination GPU's receive
-        // buffers over NVLink (rank s writes behind the records of the ranks before it): no staging copy, no
-        // all-to-all; the transfer overlaps the ranking tile by tile.  Every rank entered this call (alphabet
-        // all_reduce) before anybody stores, and the all_reduce below orders the stores before the local sort.
-        PeerOut po;
-        memset(&po, 0, sizeof(po));
-        u64* h = (u64*)(c->h_small + 1024);
-        for (int i = 0; i < 256; ++i) h[i] = 0;
-        for (int d = 0; d < P; ++d) {
-            u64 Rd = 0, before = 0;
-            for (int s = 0; s < P; ++s) {
-                Rd += mat[(size_t)s * P + d];
-                if (s < g) before += mat[(size_t)s * P + d];
-            }
-            const u64 koff = rows[(size_t)d * W + P + 4];
-            const u64 voff = sab_align_up(koff + (Rd + 8) * sizeof(u64), 256);
-            char* base = d == g ? c->arena : (char*)cm->peers[d].base;
-            po.k[d] = (u64)(uintptr_t)(base + koff);
-            po.v[d] = (u64)(uintptr_t)(base + voff);
-            h[d] = before;
-        }
-        SAB_CUDA_TRY(cudaMemcpyAsync(c->d_gbase, h, 256 * sizeof(u64), cudaMemcpyHostToDevice, st));
-        if (count)
-            SAB_TRY((sab_launch_pass_op<u64, true, SplitterDigit, true>(c, keysA, (u64*)nullptr, nullptr, (u32*)nullptr, count, sdop,
-                                                                       c->d_gbase, &po, (u32)lo)));
-        ph.mark(3);
-        SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small, 1));  // barrier: all peers' stores have landed
-        for (int d = 0; d < P; ++d)
-            if (d != g) cm->bytes_sent += mat[(size_t)g * P + d] * 12;
-    } else {
-        u64* partK = A.top<u64>(count + 8);
-        u32* partI = A.top<u32>(count + 8);
+    // ---- 2. keys of own positions (into *keys_out), splitters from a sample
+    int keys_and_splitters(u64** keys_out) {
+        ph.mark(PH_SPLITTERS);
+        u64* keysA = A.top<u64>(count + 8);
         SAB_ARENA_CHECK(A);
-        if (count)
-            SAB_TRY((sab_launch_pass_op<u64, true, SplitterDigit>(c, keysA, partK, nullptr, partI, count, sdop, c->d_gbase, nullptr, (u32)lo)));
-        // ---- 4. key exchange
-        ph.mark(3);
-        SAB_TRY(sab_comm_exchange(cm, st, pk, partK, K0, sizeof(u64)));
-        SAB_TRY(sab_comm_exchange(cm, st, pk, partI, V0, sizeof(u32)));
+        if (count) {
+            sab_prof_begin(c, 2);
+            SAB_TRY(sab_launch_pack(c, d_text, sh.len, count, al.d_lut, al.base, al.k, keysA));
+            sab_prof_end(c);
+        }
+        sdop.np = P - 1;
+        for (int i = 0; i < SAB_MAX_RANKS - 1; ++i) sdop.s[i] = ~0ull;
+        if (P > 1) {
+            // ~8 Ki samples over all ranks (slice sizes within a few per cent); the pool is sorted on the host
+            const u32 NS = 8192 / (u32)P < 512 ? 512u : (8192 / (u32)P > 2048 ? 2048u : 8192 / (u32)P);
+            const u64 step = count / NS ? count / NS : 1;
+            u64* d_sample = cm->d_small;
+            SAB_LAUNCH(sample_keys_kernel, (NS + 255) / 256, 256, 0, st, (const u64*)keysA, count, step, NS, d_sample);
+            SAB_LAUNCH_CHECK();
+            SAB_TRY(sab_comm_all_gather(cm, st, d_sample, d_sample + (NS + 1), (NS + 1) * sizeof(u64)));
+            SAB_CUDA_TRY(cudaMemcpyAsync(cm->h_small, d_sample + (NS + 1), (size_t)P * (NS + 1) * sizeof(u64), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaStreamSynchronize(st));
+            std::vector<u64> pool;
+            pool.reserve((size_t)P * NS);
+            for (int r = 0; r < P; ++r) {
+                const u64* row = cm->h_small + (size_t)r * (NS + 1);
+                const u64 have = row[NS] <= NS ? row[NS] : NS;
+                pool.insert(pool.end(), row, row + have);
+            }
+            std::sort(pool.begin(), pool.end());
+            for (int i = 0; i + 1 < P; ++i) {
+                size_t at = (size_t)(i + 1) * pool.size() / (size_t)P;
+                if (at >= pool.size()) at = pool.size() - 1;
+                sdop.s[i] = pool.empty() ? 0 : pool[at];
+            }
+        }
+        *keys_out = keysA;
+        return SAB_OK;
     }
-    A.hi = A0.hi;  // keysA, partK, partI are dead once the exchange has run (stream order)
 
-    // ---- 5. local sort: this rank's slice of the suffix array
-    ph.mark(4);
-    SortBuffers<u64> buf;
-    buf.k[0] = K0;
-    buf.v[0] = V0;
-    buf.k[1] = A.bot<u64>(R + 8);
-    buf.v[1] = A.bot<u32>(R + 8);
-    buf.cur = 0;
-    u32* sa_local = A.bot<u32>(R + 8);
-    u32* r1buf = A.bot<u32>(R + 8);
-    SAB_ARENA_CHECK(A);
-    bool sa_written = false;  // the last pass writes the sorted indices straight into the slice of sa[]
-    SAB_TRY(sab_radix_sort<u64>(c, buf, R, 0, key_bits, /*iota=*/false, &S.passes[0], sa_local, &sa_written));
-
-    // ---- 6. ranks, slice of sa[], active list, bucket directory over the slice's keys
-    ph.mark(5);
-    const u64* sortedK = buf.k[buf.cur];
-    if (c->want_bkt) SAB_TRY(sab_fused_buckets(c, d_text, n, sortedK, R, (const u16*)d_lut, sigma, base, k));  // this slice's share
-    const u32* sortedI = sa_written ? sa_local : buf.v[buf.cur];
-    u64* freeK = buf.k[buf.cur ^ 1];
-    u32* act_idx = buf.v[buf.cur ^ 1];
-    u32* rank_seq = (u32*)freeK;
-    int dir_bits = sab_ceil_log2_u64(n) - 4;
-    if (dir_bits > 28) dir_bits = 28;
-    if (dir_bits > key_bits) dir_bits = key_bits;
-    if (dir_bits < 1) dir_bits = 1;
-    const int dir_shift = key_bits - dir_bits;
-    const u64 kmax = key_bits >= 64 ? ~0ull : ((1ull << key_bits) - 1ull);
-    const u64 klo = g > 0 ? splitters[g - 1] : 0ull;
-    u64 khi = g < P - 1 ? splitters[g] : kmax;
-    if (khi > kmax) khi = kmax;
-    if (khi < klo) khi = klo;
-    const u64 dlo = klo >> dir_shift;
-    const u64 dir_len = (khi >> dir_shift) - dlo + 2;
-    u32* dir = A.bot<u32>(dir_len + 8);
-    SAB_ARENA_CHECK(A);
-    u32* dir_shifted = dir - dlo;  // indexed by key >> dir_shift
-    u32* d_m = c->d_counters;
-    u64 m = 0;
-    if (R) {
-        const u64 tiles = div_up64(R, SAB_SCAN_TILE);
-        TileState<RankScan> ts = sab_tile_state<RankScan>(c, tiles);
-        sab_prof_begin(c, 3);
-        SAB_LAUNCH(init_ranks_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, st, sortedK, sortedI, R, (u32)sa_off, (u32*)nullptr, rank_seq,
-                   sa_written ? (u32*)nullptr : sa_local, r1buf, act_idx, d_m, dir_shifted, dir_shift, ts);
-        sab_prof_end(c);
-        SAB_LAUNCH_CHECK();
-        S.kernel_launches++;
-        SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
-        SAB_CUDA_TRY(cudaStreamSynchronize(st));
-        m = c->h_small[0];
+    // ---- 3, 4. partition by destination (digit = number of splitters <= key), payload = global position; the records
+    // land in buf.k[0] / buf.v[0], either stored straight into the destination over NVLink (fused) or by all-to-all
+    int key_exchange(const u64* keysA) {
+        ph.mark(PH_PARTITION);
+        A2APlan pk;
+        u64 mat[SAB_MAX_RANKS * SAB_MAX_RANKS];
+        // the count exchange also carries what the peers need to address this rank's receive buffers directly
+        // (fused exchange, below): process, device, arena, offset of the key buffer inside it
+        const u64 k0_off = sab_align_up(A.lo, 256);
+        u64 extra[5] = {(u64)getpid(), (u64)c->device, (u64)(uintptr_t)c->arena, (u64)c->arena_bytes, k0_off};
+        constexpr int NX = 5;
+        u64 rows[SAB_MAX_RANKS * 32];
+        SAB_TRY((sab_plan_exchange<u64, SplitterDigit>(cm, c, keysA, count, nullptr, sdop, nullptr, 0, extra, NX, &pk, rows)));
+        const int W = P + NX;
+        for (int s = 0; s < P; ++s)
+            for (int d = 0; d < P; ++d) mat[(size_t)s * P + d] = rows[(size_t)s * W + d];
+        R = pk.rtotal;
+        u64 run = 1;  // first SA position of every slice
+        for (int r = 0; r < SAB_MAX_RANKS; ++r) {
+            slices.start[r] = r < P ? (u32)run : 0xffffffffu;
+            if (r == g) sa_off = run;
+            if (r < P)
+                for (int s = 0; s < P; ++s) run += mat[(size_t)s * P + r];
+        }
+        slices.pmax = (u32)P - 1;
+        SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64((count > R ? count : R) + 1, PTILE)));
+        SAB_TRY(sab_ensure_scan(c, (size_t)div_up64(R + 4096, SAB_GSORT_TILE)));
+        buf.k[0] = A.bot<u64>(R + 8);
+        buf.v[0] = A.bot<u32>(R + 8);
+        SAB_ARENA_CHECK(A);
+        fused = false;
+#ifndef SAB_EMU
+        if (P > 1 && cm->kind == 0 && sab_env_int("SAB_DIST_P2P", 1) != 0) {
+            SAB_TRY(sab_peers_update(cm, c, rows, W));
+            fused = cm->peers_ok;
+        }
+#endif
+        if (fused) {
+            // the partition pass stores every record straight into its destination GPU's receive buffers over NVLink
+            // (rank s writes behind the records of the ranks before it): no staging copy, no all-to-all; the transfer
+            // overlaps the ranking tile by tile.  Every rank entered this call (alphabet all_reduce) before anybody
+            // stores, and the all_reduce below orders the stores before the local sort.
+            PeerOut po;
+            memset(&po, 0, sizeof(po));
+            u64* h = (u64*)(c->h_small + 1024);
+            for (int i = 0; i < 256; ++i) h[i] = 0;
+            for (int d = 0; d < P; ++d) {
+                u64 Rd = 0, before = 0;
+                for (int s = 0; s < P; ++s) {
+                    Rd += mat[(size_t)s * P + d];
+                    if (s < g) before += mat[(size_t)s * P + d];
+                }
+                const u64 koff = rows[(size_t)d * W + P + 4];
+                const u64 voff = sab_align_up(koff + (Rd + 8) * sizeof(u64), 256);
+                char* base = d == g ? c->arena : (char*)cm->peers[d].base;
+                po.k[d] = (u64)(uintptr_t)(base + koff);
+                po.v[d] = (u64)(uintptr_t)(base + voff);
+                h[d] = before;
+            }
+            SAB_CUDA_TRY(cudaMemcpyAsync(c->d_gbase, h, 256 * sizeof(u64), cudaMemcpyHostToDevice, st));
+            if (count)
+                SAB_TRY((sab_launch_pass_op<u64, true, SplitterDigit, true>(c, keysA, (u64*)nullptr, nullptr, (u32*)nullptr, count, sdop,
+                                                                           c->d_gbase, &po, (u32)sh.lo)));
+            ph.mark(PH_KEY_EXCHANGE);
+            SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small, 1));  // barrier: all peers' stores have landed
+            for (int d = 0; d < P; ++d)
+                if (d != g) cm->bytes_sent += mat[(size_t)g * P + d] * 12;
+        } else {
+            u64* partK = A.top<u64>(count + 8);
+            u32* partI = A.top<u32>(count + 8);
+            SAB_ARENA_CHECK(A);
+            if (count)
+                SAB_TRY((sab_launch_pass_op<u64, true, SplitterDigit>(c, keysA, partK, nullptr, partI, count, sdop, c->d_gbase, nullptr,
+                                                                     (u32)sh.lo)));
+            ph.mark(PH_KEY_EXCHANGE);
+            SAB_TRY(sab_comm_exchange(cm, st, pk, partK, buf.k[0], sizeof(u64)));
+            SAB_TRY(sab_comm_exchange(cm, st, pk, partI, buf.v[0], sizeof(u32)));
+        }
+        A.hi = top0;  // keysA, partK, partI are dead once the exchange has run (stream order)
+        return SAB_OK;
     }
-    // In lazy mode the round keys ping-pong inside ONE key buffer (the other keeps the sorted keys): the local
-    // list must fit its halves.
-    const u64 half = sab_align_up((size_t)(R + 8) / 2, 32);
-    u64 sums[2] = {m, (m > (R + 8) - half) ? 1ull : 0ull};
-    SAB_TRY(sab_comm_sum_u64(cm, st, sums, 2));
-    u64 tot = sums[0];
-    S.active[0] = m;
-    ds->active[0] = tot;
-    u32 round = 0;
-    bool lazy = false, rebalanced = false;
-    int layout_cyc = 0;
-    if (tot > 0) {
-        // ---- 7. inverse suffix array at the owners
-        ph.mark(6);
-        lazy = tot <= n / 4 && sums[1] == 0 && sab_env_int("SAB_DIST_LAZY", 1) != 0;
+
+    // ---- 5, 6. local sort -> this rank's slice of the suffix array; init_ranks: ranks, slice of sa[], active list,
+    // bucket directory over the slice's keys.  Ends with the active count over all ranks (tot).
+    int local_slice(bool* halves_fit) {
+        ph.mark(PH_LOCAL_SORT);
+        buf.k[1] = A.bot<u64>(R + 8);
+        buf.v[1] = A.bot<u32>(R + 8);
+        buf.cur = 0;
+        sa_local = A.bot<u32>(R + 8);
+        r1buf = A.bot<u32>(R + 8);
+        SAB_ARENA_CHECK(A);
+        bool sa_written = false;  // the last pass writes the sorted indices straight into the slice of sa[]
+        SAB_TRY(sab_radix_sort<u64>(c, buf, R, 0, al.key_bits, /*iota=*/false, &c->stats.passes[0], sa_local, &sa_written));
+
+        ph.mark(PH_INIT_RANKS);
+        sortedK = buf.k[buf.cur];
+        if (c->want_bkt) SAB_TRY(sab_fused_buckets(c, d_text, n, sortedK, R, al));  // this slice's share
+        sortedI = sa_written ? sa_local : buf.v[buf.cur];
+        u32* act_idx = buf.v[buf.cur ^ 1];
+        rank_seq = (u32*)buf.k[buf.cur ^ 1];
+        dir_shift = al.key_bits - sab_dir_bits(n, al.key_bits, SAB_DIST_DIR_SHIFT);
+        const u64 kmax = al.key_bits >= 64 ? ~0ull : ((1ull << al.key_bits) - 1ull);
+        const u64 klo = g > 0 ? sdop.s[g - 1] : 0ull;
+        u64 khi = g < P - 1 ? sdop.s[g] : kmax;
+        if (khi > kmax) khi = kmax;
+        if (khi < klo) khi = klo;
+        dlo = klo >> dir_shift;
+        const u64 dir_len = (khi >> dir_shift) - dlo + 2;
+        dir = A.bot<u32>(dir_len + 8);
+        SAB_ARENA_CHECK(A);
+        m = 0;
+        if (R)
+            SAB_TRY(sab_init_ranks(c, sortedK, sortedI, R, (u32)sa_off, nullptr, rank_seq, sa_written ? nullptr : sa_local, r1buf, act_idx,
+                                   dir - dlo, dir_shift, &m));
+        const u64 half = sab_align_up((size_t)(R + 8) / 2, 32);  // lazy mode: the local list must fit a half (sab_round_buffers)
+        u64 sums[2] = {m, (m > (R + 8) - half) ? 1ull : 0ull};
+        SAB_TRY(sab_comm_sum_u64(cm, st, sums, 2));
+        tot = sums[0];
+        *halves_fit = sums[1] == 0;
+        c->stats.active[0] = m;
+        ds->active[0] = tot;
+        return SAB_OK;
+    }
+
+    // ---- 7. inverse suffix array at the owners (file header, step 6), and the buffers of the rounds
+    int ranks_to_owners(bool halves_fit) {
+        ph.mark(PH_RANKS_TO_OWNERS);
+        lazy = tot <= n / 4 && halves_fit && sab_env_int("SAB_DIST_LAZY", 1) != 0;
         const char* lenv = getenv("SAB_RANK_LAYOUT");
         layout_cyc = lazy ? 0 : 1;  // lazy look-ups pack keys from the owner's text shard: block ownership
         if (!lazy && lenv && !strcmp(lenv, "block")) layout_cyc = 0;
@@ -708,418 +690,427 @@ static int sab_dist_saca(sab200_comm* cm, SabContext* c, DistArena A0, const u8*
             const u64 width = 1ull << shift;
             const u64 blocks = div_up64(n + 1, width);
             local_len = div_up64(blocks, (u64)P) << shift;
-            sab_rank_layout((u32)width, P, shift, &R_.lay);
+            sab_rank_layout((u32)width, P, shift, &lay);
         } else {
-            local_len = B + 1;  // the last GPU also owns position n
-            sab_rank_layout((u32)B, P, -1, &R_.lay);
+            local_len = sh.B + 1;  // the last GPU also owns position n
+            sab_rank_layout((u32)sh.B, P, -1, &lay);
         }
-        const RankLayout lay = R_.lay;
-        u32* rank_local = A.bot<u32>(local_len + 8);
+        rank_local = A.bot<u32>(local_len + 8);
         SAB_ARENA_CHECK(A);
-        R_.rank_local = rank_local;
         if (lazy) SAB_CUDA_TRY(cudaMemsetAsync(rank_local, 0xff, local_len * sizeof(u32), st));
-        {
-            const u32 on = sab_layout_owner_host(lay, n);  // the empty suffix has rank 0
-            if ((int)on == g) SAB_CUDA_TRY(cudaMemsetAsync(rank_local + sab_layout_slot_host(lay, n, on), 0, sizeof(u32), st));
-        }
-        if (lazy) SAB_TRY(R_.send_ranks(act_idx, r1buf, m));
-        else SAB_TRY(R_.send_ranks(sortedI, rank_seq, R));
+        const u32 on = lay.owner(n);  // the empty suffix has rank 0
+        if ((int)on == g) SAB_CUDA_TRY(cudaMemsetAsync(rank_local + lay.slot(n, on), 0, sizeof(u32), st));
+        if (lazy) SAB_TRY(send_ranks(buf.v[buf.cur ^ 1], r1buf, m));
+        else SAB_TRY(send_ranks(sortedI, rank_seq, R));
+        rb = sab_round_buffers(buf, R, lazy, &key_cap);
+        val_cap = R + 8;
+        return SAB_OK;
+    }
 
-        // ---- 8. doubling rounds
-        SortBuffers<u64> rb;
-        u32 slice_start[SAB_MAX_RANKS];  // first SA position of every slice
-        {
-            u64 run = 1;
-            for (int r = 0; r < SAB_MAX_RANKS; ++r) {
-                slice_start[r] = r < P ? (u32)run : 0xffffffffu;
-                if (r < P)
-                    for (int s = 0; s < P; ++s) run += mat[(size_t)s * P + r];
-            }
+    // ---- 7b. even out the active lists.  The slices hold equal numbers of SUFFIXES, not of active ones (on the
+    // mixed text the English-like key ranges hold nearly all of them) and a round costs what its longest list
+    // costs.  The lists are globally sorted by rank and groups never straddle GPUs: cut points move to group
+    // boundaries and contiguous chunks are shipped, which keeps both properties.  A suffix that becomes unique
+    // on a GPU that does not hold its SA position is then routed to the slice owner (new_sa_entries).
+    int rebalance() {
+        ph.mark(PH_REBALANCE);
+        if (P == 1) return SAB_OK;
+        u64 mine[SAB_MAX_RANKS], mm[SAB_MAX_RANKS * SAB_MAX_RANKS];
+        for (int d = 0; d < P; ++d) mine[d] = m;
+        SAB_TRY(sab_comm_count_matrix(cm, st, mine, mm));  // mm[s*P + *] = list length of rank s
+        u64 M = 0, mx = 0, off = 0;
+        for (int s = 0; s < P; ++s) {
+            const u64 v = mm[(size_t)s * P];
+            M += v;
+            if (v > mx) mx = v;
+            if (s < g) off += v;
         }
-        u64 key_cap;
-        if (lazy) {
-            rb.k[0] = freeK;
-            rb.k[1] = freeK + half;
-            key_cap = (R + 8) - half;
-        } else {
-            rb.k[0] = freeK;
-            rb.k[1] = buf.k[buf.cur];
-            key_cap = R + 8;
+        const u64 rebal_min = (u64)sab_env_int("SAB_REBALANCE_MIN", 1 << 20);
+        if (M < rebal_min * (u64)P || (double)mx * P <= 1.1 * (double)M) return SAB_OK;
+        const u64 Q = div_up64(M, (u64)P);
+        u64* h = (u64*)(c->h_small + 1024);
+        u64 cuts[SAB_MAX_RANKS], found[SAB_MAX_RANKS];
+        for (int j = 1; j < P; ++j) {
+            const u64 want = (u64)j * Q;
+            cuts[j - 1] = want <= off ? 0 : (want - off >= m ? m : want - off);
+            found[j - 1] = (cuts[j - 1] == 0 || cuts[j - 1] >= m) ? cuts[j - 1] : ~0ull;
         }
-        rb.v[0] = act_idx;
-        rb.v[1] = buf.v[buf.cur];
-        rb.cur = 0;
-        const u64 val_cap = R + 8;
-        u32* sa_shifted = sa_local - (size_t)sa_off;  // ranks are global SA positions
-        // ---- 7b. even out the active lists.  The slices hold equal numbers of SUFFIXES, not of active ones (on the
-        // mixed text the English-like key ranges hold nearly all of them) and a round costs what its longest list
-        // costs.  The lists are globally sorted by rank and groups never straddle GPUs: cut points move to group
-        // boundaries and contiguous chunks are shipped, which keeps both properties.  A suffix that becomes unique
-        // on a GPU that does not hold its SA position is then routed to the slice owner (step f of a round).
-        ph.mark(7);
-        if (P > 1) {
-            u64 mine[SAB_MAX_RANKS], mm[SAB_MAX_RANKS * SAB_MAX_RANKS];
-            for (int d = 0; d < P; ++d) mine[d] = m;
-            SAB_TRY(sab_comm_count_matrix(cm, st, mine, mm));  // mm[s*P + *] = list length of rank s
-            u64 M = 0, mx = 0, off = 0;
-            for (int s = 0; s < P; ++s) {
-                const u64 v = mm[(size_t)s * P];
-                M += v;
-                if (v > mx) mx = v;
-                if (s < g) off += v;
+        u64* d_cuts = c->d_ghist;  // [P-1] cuts, then [P-1] results
+        unsigned long long* d_found = (unsigned long long*)(c->d_ghist + SAB_MAX_RANKS);
+        memcpy(h, cuts, sizeof(u64) * (P - 1));
+        SAB_CUDA_TRY(cudaMemcpyAsync(d_cuts, h, sizeof(u64) * (P - 1), cudaMemcpyHostToDevice, st));
+        u64 woff = 0, window = 1 << 16;
+        for (;;) {
+            bool open = false;
+            for (int j = 0; j < P - 1; ++j) open = open || found[j] == ~0ull;
+            if (!open) break;
+            SAB_CUDA_TRY(cudaMemsetAsync(d_found, 0xff, sizeof(u64) * (P - 1), st));
+            const u32 bpc = (u32)div_up64(window, 256);
+            SAB_LAUNCH(find_boundary_kernel, bpc * (unsigned)(P - 1), 256, 0, st, (const u32*)r1buf, m, (const u64*)d_cuts, bpc, woff,
+                       window, d_found);
+            SAB_LAUNCH_CHECK();
+            SAB_CUDA_TRY(cudaMemcpyAsync(h + 32, d_found, sizeof(u64) * (P - 1), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaStreamSynchronize(st));
+            for (int j = 0; j < P - 1; ++j) {
+                if (found[j] != ~0ull) continue;
+                if (h[32 + j] != ~0ull) found[j] = h[32 + j];
+                else if (cuts[j] + woff + window >= m) found[j] = m;  // the group runs to the end of the list
             }
-            const u64 rebal_min = (u64)sab_env_int("SAB_REBALANCE_MIN", 1 << 20);
-            if (M >= rebal_min * (u64)P && (double)mx * P > 1.1 * (double)M) {
-                const u64 Q = div_up64(M, (u64)P);
-                u64* h = (u64*)(c->h_small + 1024);
-                u64 cuts[SAB_MAX_RANKS], found[SAB_MAX_RANKS];
-                for (int j = 1; j < P; ++j) {
-                    const u64 want = (u64)j * Q;
-                    cuts[j - 1] = want <= off ? 0 : (want - off >= m ? m : want - off);
-                    found[j - 1] = (cuts[j - 1] == 0 || cuts[j - 1] >= m) ? cuts[j - 1] : ~0ull;
-                }
-                u64* d_cuts = c->d_ghist;             // [P-1] cuts, then [P-1] results
-                unsigned long long* d_found = (unsigned long long*)(c->d_ghist + SAB_MAX_RANKS);
-                memcpy(h, cuts, sizeof(u64) * (P - 1));
-                SAB_CUDA_TRY(cudaMemcpyAsync(d_cuts, h, sizeof(u64) * (P - 1), cudaMemcpyHostToDevice, st));
-                u64 woff = 0, window = 1 << 16;
-                for (;;) {
-                    bool open = false;
-                    for (int j = 0; j < P - 1; ++j) open = open || found[j] == ~0ull;
-                    if (!open) break;
-                    SAB_CUDA_TRY(cudaMemsetAsync(d_found, 0xff, sizeof(u64) * (P - 1), st));
-                    const u32 bpc = (u32)div_up64(window, 256);
-                    SAB_LAUNCH(find_boundary_kernel, bpc * (unsigned)(P - 1), 256, 0, st, (const u32*)r1buf, m, (const u64*)d_cuts, bpc, woff,
-                               window, d_found);
-                    SAB_LAUNCH_CHECK();
-                    SAB_CUDA_TRY(cudaMemcpyAsync(h + 32, d_found, sizeof(u64) * (P - 1), cudaMemcpyDeviceToHost, st));
-                    SAB_CUDA_TRY(cudaStreamSynchronize(st));
-                    for (int j = 0; j < P - 1; ++j) {
-                        if (found[j] != ~0ull) continue;
-                        if (h[32 + j] != ~0ull) found[j] = h[32 + j];
-                        else if (cuts[j] + woff + window >= m) found[j] = m;  // the group runs to the end of the list
-                    }
-                    woff += window;
-                    window *= 8;
-                }
-                u64 bounds[SAB_MAX_RANKS + 1], sendc[SAB_MAX_RANKS];
-                bounds[0] = 0;
-                for (int j = 1; j < P; ++j) bounds[j] = found[j - 1] > bounds[j - 1] ? found[j - 1] : bounds[j - 1];
-                bounds[P] = m;
-                for (int j = 0; j < P; ++j) sendc[j] = bounds[j + 1] - bounds[j];
-                A2APlan pb;
-                SAB_TRY(sab_comm_plan(cm, st, sendc, &pb, nullptr));
-                const u64 cap = key_cap < val_cap ? key_cap : val_cap;
-                u64 bad = pb.rtotal + 64 > cap ? 1 : 0;
-                SAB_TRY(sab_comm_sum_u64(cm, st, &bad, 1));
-                if (bad == 0) {
-                    const size_t mark = A.hi;
-                    u32* t1 = A.top<u32>(pb.rtotal + 8);
-                    u32* t2 = A.top<u32>(pb.rtotal + 8);
-                    SAB_ARENA_CHECK(A);
-                    SAB_TRY(sab_comm_exchange(cm, st, pb, r1buf, t1, sizeof(u32)));
-                    SAB_TRY(sab_comm_exchange(cm, st, pb, rb.v[rb.cur], t2, sizeof(u32)));
-                    m = pb.rtotal;
-                    if (m) {
-                        SAB_CUDA_TRY(cudaMemcpyAsync(r1buf, t1, m * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-                        SAB_CUDA_TRY(cudaMemcpyAsync(rb.v[rb.cur], t2, m * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-                    }
-                    A.hi = mark;
-                    rebalanced = true;
-                }
-            }
+            woff += window;
+            window *= 8;
         }
-        // ---- 7c. peer table of the peer-to-peer rounds (same precondition as the fused key exchange)
-        bool p2p_ready = false;
-        P2PTable pt;
+        u64 bounds[SAB_MAX_RANKS + 1], sendc[SAB_MAX_RANKS];
+        bounds[0] = 0;
+        for (int j = 1; j < P; ++j) bounds[j] = found[j - 1] > bounds[j - 1] ? found[j - 1] : bounds[j - 1];
+        bounds[P] = m;
+        for (int j = 0; j < P; ++j) sendc[j] = bounds[j + 1] - bounds[j];
+        A2APlan pb;
+        SAB_TRY(sab_comm_plan(cm, st, sendc, &pb, nullptr));
+        const u64 cap = key_cap < val_cap ? key_cap : val_cap;
+        u64 bad = pb.rtotal + 64 > cap ? 1 : 0;
+        SAB_TRY(sab_comm_sum_u64(cm, st, &bad, 1));
+        if (bad != 0) return SAB_OK;
+        const size_t mark = A.hi;
+        u32* t1 = A.top<u32>(pb.rtotal + 8);
+        u32* t2 = A.top<u32>(pb.rtotal + 8);
+        SAB_ARENA_CHECK(A);
+        SAB_TRY(sab_comm_exchange(cm, st, pb, r1buf, t1, sizeof(u32)));
+        SAB_TRY(sab_comm_exchange(cm, st, pb, rb.v[rb.cur], t2, sizeof(u32)));
+        m = pb.rtotal;
+        if (m) {
+            SAB_CUDA_TRY(cudaMemcpyAsync(r1buf, t1, m * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+            SAB_CUDA_TRY(cudaMemcpyAsync(rb.v[rb.cur], t2, m * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+        }
+        A.hi = mark;
+        rebalanced = true;
+        return SAB_OK;
+    }
+
+    // ---- 7c. peer table of the peer-to-peer rounds (same precondition as the fused key exchange)
+    int peer_table() {
         memset(&pt, 0, sizeof(pt));
+        if (!fused || rebalanced) return SAB_OK;
+        // row: offsets of rank_local, text, sorted keys, directory inside the arena; directory origin, slice length, offset
+        u64* hrow = cm->h_small + 32;
+        hrow[0] = (u64)((char*)rank_local - c->arena);
+        hrow[1] = (u64)((const char*)d_text - c->arena);
+        hrow[2] = (u64)((const char*)sortedK - c->arena);
+        hrow[3] = (u64)((char*)dir - c->arena);
+        hrow[4] = dlo;
+        hrow[5] = R;
+        hrow[6] = sa_off;
+        hrow[7] = ((const char*)d_text >= c->arena && (const char*)d_text < c->arena + c->arena_bytes) ? 1 : 0;
+        SAB_CUDA_TRY(cudaMemcpyAsync(cm->d_small, hrow, 8 * sizeof(u64), cudaMemcpyHostToDevice, st));
+        u64 prow[SAB_MAX_RANKS * 8];
+        SAB_TRY(sab_comm_gather_rows(cm, st, 8, prow));  // also orders every rank's ISA scatter before the first gather
+        bool ok = true;
+        for (int d = 0; d < P; ++d) {
+            const u64* r = prow + (size_t)d * 8;
+            char* pb = d == g ? c->arena : (char*)cm->peers[d].base;
+            ok = ok && r[7] == 1 && pb != nullptr;
+            pt.rank_local[d] = (u32*)(pb + r[0]);
+            pt.text[d] = (const u8*)(pb + r[1]);
+            pt.sorted[d] = (const u64*)(pb + r[2]);
+            pt.dir[d] = (const u32*)(pb + r[3]) - r[4];
+            pt.R[d] = r[5];
+            pt.sa_off[d] = (u32)r[6];
+            pt.n_rel[d] = sab_shard_bounds(n, P, d).len;
+        }
+        p2p_ready = ok;
+        return SAB_OK;
+    }
+
+    // ---- round, a. (peer to peer): rank[i + h] loaded straight from the owner GPU
+    int second_ranks_p2p(u64 h) {
+        ph.mark(PH_REQUESTS);
+        if (lead_barrier) {  // the owners' scatters of an all-to-all round must have finished everywhere
+            SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small + 8, 1));
+            lead_barrier = false;
+        }
+        if (m) {
+            sab_prof_begin(c, 4);
+            SAB_LAUNCH(dist_gather_p2p_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)r1buf, (const u32*)rb.v[rb.cur], m,
+                       (u32)h, lay, pt, lazy ? 1 : 0, al.d_lut, al.base, al.k, dir_shift, sdop, rb.k[rb.cur]);
+            sab_prof_end(c);
+            SAB_LAUNCH_CHECK();
+            c->stats.kernel_launches++;
+        }
+        return SAB_OK;
+    }
+
+    // ---- round, a + b. (all-to-all): requests i + h to the owners (payload = list position), answers back in the same
+    // order.  The buffers are temporaries at the top of the arena; the caller releases them.
+    int second_ranks_a2a(u64 h) {
+        ph.mark(PH_REQUESTS);
+        u32* cur_idx = rb.v[rb.cur];
+        u32* ipart = A.top<u32>(m + 8);
+        u32* ppart = A.top<u32>(m + 8);
+        SAB_ARENA_CHECK(A);
+        OwnerDigit odop;
+        odop.add = (u32)h;
+        odop.lay = lay;
+        A2APlan pr;
+        SAB_TRY((sab_plan_exchange<u32, OwnerDigit>(cm, c, cur_idx, m, nullptr, odop, nullptr, 0, nullptr, 0, &pr, nullptr)));
+        if (m) {
+            SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64(m, PTILE)));
+            SAB_TRY((sab_launch_pass_op<u32, true, OwnerDigit>(c, cur_idx, ipart, nullptr, ppart, m, odop, c->d_gbase)));
+        }
+        const u64 nq = pr.rtotal;
+        u32* q = A.top<u32>(nq + 8);
+        u32* ans = A.top<u32>(nq + 8);
+        SAB_ARENA_CHECK(A);
+        SAB_TRY(sab_comm_exchange(cm, st, pr, ipart, q, sizeof(u32)));
+        if (nq) {
+            sab_prof_begin(c, 4);
+            SAB_LAUNCH(dist_gather_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, (const u32*)q, nq, (u32)h, (u32)sh.lo, lay,
+                       (const u32*)rank_local, ans);
+            sab_prof_end(c);
+            SAB_LAUNCH_CHECK();
+            c->stats.kernel_launches++;
+        }
+        if (lazy) {
+            // b. requests that found EMPTY: key at the owner -> slice that holds the key -> rank back.  Their
+            // number stays on the device until it comes back with the count exchange (one synchronisation).
+            ph.mark(PH_LAZY);
+            u64* keys_u = A.top<u64>(nq + 8);
+            u32* slot_u = A.top<u32>(nq + 8);
+            SAB_ARENA_CHECK(A);
+            u32* d_nu = c->d_counters + 12;
+            SAB_CUDA_TRY(cudaMemsetAsync(d_nu, 0, sizeof(u32), st));
+            if (nq) {
+                SAB_LAUNCH(dist_lazy_collect_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, q, (const u32*)ans, nq, (u32)h, sh.lo, d_text,
+                           sh.len, al.d_lut, al.base, al.k, keys_u, slot_u, d_nu);
+                SAB_LAUNCH_CHECK();
+                c->stats.kernel_launches++;
+            }
+            A2APlan pu;
+            u64 rows_u[SAB_MAX_RANKS * 32];
+            SAB_TRY((sab_plan_exchange<u64, SplitterDigit>(cm, c, keys_u, nq, d_nu, sdop, d_nu, 1, nullptr, 0, &pu, rows_u)));
+            const u64 nu = rows_u[(size_t)g * (P + 1) + P];
+            ds->resolved_empty += nu;
+            u64* kp = A.top<u64>(nu + 8);
+            u32* sp = A.top<u32>(nu + 8);
+            SAB_ARENA_CHECK(A);
+            if (nu) {
+                SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64(nu, PTILE)));
+                SAB_TRY((sab_launch_pass_op<u64, false, SplitterDigit>(c, keys_u, kp, slot_u, sp, nu, sdop, c->d_gbase)));
+            }
+            u64* kq = A.top<u64>(pu.rtotal + 8);
+            u32* rk = A.top<u32>(pu.rtotal + 8);
+            u32* back = A.top<u32>(nu + 8);
+            SAB_ARENA_CHECK(A);
+            SAB_TRY(sab_comm_exchange(cm, st, pu, kp, kq, sizeof(u64)));
+            if (pu.rtotal) {
+                SAB_LAUNCH(dist_lookup_kernel, (unsigned)div_up64(pu.rtotal, 256), 256, 0, st, sortedK, R, (const u32*)(dir - dlo), dir_shift,
+                           (const u64*)kq, pu.rtotal, (u32)sa_off, rk);
+                SAB_LAUNCH_CHECK();
+                c->stats.kernel_launches++;
+            }
+            SAB_TRY(sab_comm_exchange_back(cm, st, pu, rk, back, sizeof(u32)));
+            if (nu) {
+                SAB_LAUNCH(dist_lazy_fill_kernel, (unsigned)div_up64(nu, 256), 256, 0, st, (const u32*)sp, (const u32*)back, nu, q, (u32)h,
+                           (u32)sh.lo, ans, rank_local);
+                SAB_LAUNCH_CHECK();
+                c->stats.kernel_launches++;
+            }
+            ph.mark(PH_REQUESTS);
+        }
+        u32* r2 = A.top<u32>(m + 8);
+        SAB_ARENA_CHECK(A);
+        SAB_TRY(sab_comm_exchange_back(cm, st, pr, ans, r2, sizeof(u32)));
+        if (m) {
+            SAB_LAUNCH(dist_place_keys_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)r1buf, (const u32*)ppart, (const u32*)r2,
+                       m, rb.k[rb.cur]);
+            SAB_LAUNCH_CHECK();
+            c->stats.kernel_launches++;
+        }
+        return SAB_OK;
+    }
+
+    // ---- round, c + d. order inside the groups (as on one GPU: the list is still grouped by r1, ascending), then
+    // re-rank: newly unique suffixes go to sa[], changed ranks are collected for their owners (upd_idx, upd_r); the
+    // number of survivors stays on the device and comes back with the count exchange of the rank updates
+    int refine(u32 round) {
+        ph.mark(PH_ROUND_SORT);
+        upd_idx = A.top<u32>(m + 8);
+        upd_r = A.top<u32>(m + 8);
+        set_pos = rebalanced ? A.top<u32>(m + 8) : nullptr;
+        sorted_idx = nullptr;
+        sorted_in = 0;
+        SAB_ARENA_CHECK(A);
+        SAB_CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, sizeof(u32), st));  // kept = 0 unless the re-rank says otherwise
+        if (m == 0) return SAB_OK;
+        const int rank_bits = sab_ceil_log2_u64(n + 2);
+        SortBuffers<u64> sb;
+        sb.k[0] = rb.k[rb.cur];
+        sb.k[1] = rb.k[rb.cur ^ 1];
+        sb.v[0] = rb.v[rb.cur];
+        sb.v[1] = rb.v[rb.cur ^ 1];
+        sb.cur = 0;
+        int sorted = 0;
+        if (group_sort_on) {
+            // the first ranks live in the key words until the re-rank writes them back: r1buf holds the positions
+            const GroupSortSpare sp = sab_group_sort_spare(sb, m, key_cap, val_cap, r1buf);
+            if (sp.cap * 8 >= m) {
+                u64 nbig = 0;
+                sorted = sab_group_sort(c, sb, m, 32 + rank_bits, sp, &c->stats.passes[round], &nbig);
+                if (sorted < 0) return sorted;
+                if (nbig * 2 > m) group_sort_on = false;
+            }
+        }
+        if (!sorted) SAB_TRY(sab_radix_sort<u64>(c, sb, m, 0, 32 + rank_bits, /*iota=*/false, &c->stats.passes[round]));
+        ph.mark(PH_RERANK);
+        u32* out_idx = (sb.cur == 0) ? rb.v[rb.cur ^ 1] : rb.v[rb.cur];
+        // ranks are global SA positions
+        SAB_TRY(sab_launch_rerank(c, sb, m, nullptr, sa_local - (size_t)sa_off, r1buf, out_idx, upd_idx, upd_r, set_pos));
+        sorted_idx = sb.v[sb.cur];
+        sorted_in = sb.cur;
+        return SAB_OK;
+    }
+
+    // ---- round, f. (rebalanced lists) new SA entries to the GPUs that hold their positions, before the buffer of the
+    // sorted indices is reused for the next list; a rank with an empty list still takes part in the exchange
+    int new_sa_entries() {
+        ph.mark(PH_NEW_SA);
+        const size_t mark = A.hi;
+        u32* kp = A.top<u32>(m + 8);
+        u32* vp = A.top<u32>(m + 8);
+        SAB_ARENA_CHECK(A);
+        A2APlan ps;
+        SAB_TRY((sab_plan_exchange<u32, SliceDigit>(cm, c, set_pos, m, nullptr, slices, nullptr, 0, nullptr, 0, &ps, nullptr)));
+        if (m) {
+            SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64(m, PTILE)));
+            SAB_TRY((sab_launch_pass_op<u32, false, SliceDigit>(c, set_pos, kp, sorted_idx, vp, m, slices, c->d_gbase)));
+        }
+        u32* rp = A.top<u32>(ps.rtotal + 8);
+        u32* ri = A.top<u32>(ps.rtotal + 8);
+        SAB_ARENA_CHECK(A);
+        SAB_TRY(sab_comm_exchange(cm, st, ps, kp, rp, sizeof(u32)));
+        SAB_TRY(sab_comm_exchange(cm, st, ps, vp, ri, sizeof(u32)));
+        if (ps.rtotal) {
+            SAB_LAUNCH(dist_store_sa_kernel, (unsigned)div_up64(ps.rtotal, 256), 256, 0, st, (const u32*)rp, (const u32*)ri, ps.rtotal,
+                       (u32)sa_off, sa_local);
+            SAB_LAUNCH_CHECK();
+            c->stats.kernel_launches++;
+        }
+        A.hi = mark;
+        return SAB_OK;
+    }
+
+    // ---- round, e. changed ranks to their owners; the same exchange returns every rank's number of survivors (tot
+    // over all ranks).  The survivors here become the next list.
+    int rank_updates(bool p2p_round) {
+        u64 kept = 0;
+        u32* d_m = c->d_counters;
+        ph.mark(PH_RANK_UPDATES);
+        if (p2p_round) {
+            // all_reduce #1: the survivors add up (termination) and every rank has finished LOADING ranks;
+            // then the stores go straight into the owners' blocks; all_reduce #2: every store has landed
+            SAB_LAUNCH(put_u64_kernel, 1, 1, 0, st, cm->d_small, (const u32*)d_m);
+            SAB_LAUNCH_CHECK();
+            SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small, 1));
+            if (m) {
+                SAB_LAUNCH(dist_scatter_p2p_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)upd_idx, (const u32*)upd_r, m, lay, pt);
+                SAB_LAUNCH_CHECK();
+                c->stats.kernel_launches++;
+            }
+            SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small + 8, 1));
+            SAB_CUDA_TRY(cudaMemcpyAsync(cm->h_small, cm->d_small, sizeof(u64), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaStreamSynchronize(st));
+            tot = cm->h_small[0];
+            kept = c->h_small[0];
+            ds->p2p_rounds++;
+        } else {
+            u64 rows_k[SAB_MAX_RANKS * 32];
+            SAB_TRY(send_ranks(upd_idx, upd_r, m, d_m, 1, rows_k));
+            kept = rows_k[(size_t)g * (P + 1) + P];
+            tot = 0;
+            for (int s2 = 0; s2 < P; ++s2) tot += rows_k[(size_t)s2 * (P + 1) + P];
+            lead_barrier = true;
+        }
+        if (m && sorted_in != 0 && kept > 0)
+            SAB_CUDA_TRY(cudaMemcpyAsync(rb.v[rb.cur ^ 1], rb.v[rb.cur], kept * sizeof(u32), cudaMemcpyDeviceToDevice, st));
+        rb.cur ^= 1;
+        m = kept;
+        return SAB_OK;
+    }
+};
+
+// d_text: this rank's shard + halo on the device (text_len bytes).  The arena `A0` starts behind whatever the
+// caller placed at its bottom.  Enqueues on c->stream; the stream is idle when the function returns.
+static int sab_dist_saca(sab200_comm* cm, SabContext* c, DistArena A0, const u8* d_text, u64 text_len, u64 n, DistResult* res,
+                         sab200_dist_stats* ds) {
+    cudaStream_t st = c->stream;
+    SabStats& S = c->stats;
+    S.n = n;
+    cm->bytes_sent = 0;
+    cm->collectives = 0;
+    DistRun run(cm, c, ds, A0, d_text, n);
+    *res = DistResult{nullptr, 0, 1};
+    ds->nranks = (u32)run.P;
+    ds->rank = (u32)run.g;
+    if (n == 0) return SAB_OK;  // the suffix array is the sentinel alone
+    if (text_len < run.sh.len) {
+        sab_set_error("rank %d: shard of %llu bytes, need %llu (own positions + halo)", run.g, (unsigned long long)text_len,
+                      (unsigned long long)run.sh.len);
+        return SAB_ERR_ARGS;
+    }
+    SAB_TRY(sab_ensure_scan(c, (size_t)div_up64(run.count + run.count / 2 + 4096, SAB_GSORT_TILE)));
+
+    u64* keysA = nullptr;
+    SAB_TRY(run.alphabet());
+    SAB_TRY(run.keys_and_splitters(&keysA));
+    SAB_TRY(run.key_exchange(keysA));
+    bool halves_fit = false;
+    SAB_TRY(run.local_slice(&halves_fit));
+    u32 round = 0;
+    if (run.tot > 0) {
+        SAB_TRY(run.ranks_to_owners(halves_fit));
+        SAB_TRY(run.rebalance());
+        SAB_TRY(run.peer_table());
         // records per rank; above it the all-to-all form wins (measured on 8 B200, 1 GiB text: every round peer to peer
         // 20.3 ms, limit 2 Mi 18.8 ms; on 2 GPUs limits of 4 Mi .. 16 Mi are within 1 % of each other)
         const u64 p2p_max = (u64)sab_env_int("SAB_P2P_MAX_RECORDS", 2 << 20);
-        if (fused && !rebalanced) {
-            // row: offsets of rank_local, text, sorted keys, directory inside the arena; directory origin, slice length, offset
-            u64* hrow = cm->h_small + 32;
-            hrow[0] = (u64)((char*)rank_local - c->arena);
-            hrow[1] = (u64)((const char*)d_text - c->arena);
-            hrow[2] = (u64)((const char*)sortedK - c->arena);
-            hrow[3] = (u64)((char*)dir - c->arena);
-            hrow[4] = dlo;
-            hrow[5] = R;
-            hrow[6] = sa_off;
-            hrow[7] = ((const char*)d_text >= c->arena && (const char*)d_text < c->arena + c->arena_bytes) ? 1 : 0;
-            SAB_CUDA_TRY(cudaMemcpyAsync(cm->d_small, hrow, 8 * sizeof(u64), cudaMemcpyHostToDevice, st));
-            u64 prow[SAB_MAX_RANKS * 8];
-            SAB_TRY(sab_comm_gather_rows(cm, st, 8, prow));  // also orders every rank's ISA scatter before the first gather
-            bool ok = true;
-            for (int d = 0; d < P; ++d) {
-                const u64* r = prow + (size_t)d * 8;
-                char* pb = d == g ? c->arena : (char*)cm->peers[d].base;
-                ok = ok && r[7] == 1 && pb != nullptr;
-                pt.rank_local[d] = (u32*)(pb + r[0]);
-                pt.text[d] = (const u8*)(pb + r[1]);
-                pt.sorted[d] = (const u64*)(pb + r[2]);
-                pt.dir[d] = (const u32*)(pb + r[3]) - r[4];
-                pt.R[d] = r[5];
-                pt.sa_off[d] = (u32)r[6];
-                const u64 lo_d = (u64)d * B < n ? (u64)d * B : n;
-                const u64 hi_d = lo_d + B < n ? lo_d + B : n;
-                pt.n_rel[d] = (n - lo_d) < (hi_d - lo_d) + SAB200_SHARD_HALO ? (n - lo_d) : (hi_d - lo_d) + SAB200_SHARD_HALO;
-            }
-            p2p_ready = ok;
-        }
-        bool lead_barrier = false;  // the first gather is ordered by the row exchange above
-        const int rank_bits = sab_ceil_log2_u64(n + 2);
-        bool group_sort_on = true;  // until most records are in large groups
-        u64 h = (u64)k;
-        while (tot > 0) {
+        u64 h = (u64)run.al.k;
+        while (run.tot > 0) {
             ++round;
             if (round >= SAB_MAX_ROUNDS || h > n) {
                 sab_set_error("prefix doubling did not converge (round %u, h=%llu, active=%llu)", round, (unsigned long long)h,
-                              (unsigned long long)tot);
+                              (unsigned long long)run.tot);
                 return SAB_ERR_INTERNAL;
             }
-            const size_t topmark = A.hi;
+            const size_t topmark = run.A.hi;
             // Small rounds go peer to peer (no exchange step, one host round trip); large ones through partition +
             // all-to-all (bulk NVLink transfers, local random access).  Same decision on every rank.
-            const bool p2p_round = p2p_ready && tot <= p2p_max * (u64)P;
-            if (p2p_round) {
-                ph.mark(8);
-                if (lead_barrier) {  // the owners' scatters of an all-to-all round must have finished everywhere
-                    SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small + 8, 1));
-                    lead_barrier = false;
-                }
-                if (m) {
-                    sab_prof_begin(c, 4);
-                    SAB_LAUNCH(dist_gather_p2p_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)r1buf, (const u32*)rb.v[rb.cur], m,
-                               (u32)h, lay, pt, lazy ? 1 : 0, (const u16*)d_lut, base, k, dir_shift, sdop, rb.k[rb.cur]);
-                    sab_prof_end(c);
-                    SAB_LAUNCH_CHECK();
-                    S.kernel_launches++;
-                }
-            } else {
-            // a. requests i + h to the owners (payload = list position), answers back in the same order
-            ph.mark(8);
-            u32* cur_idx = rb.v[rb.cur];
-            u32* ipart = A.top<u32>(m + 8);
-            u32* ppart = A.top<u32>(m + 8);
-            SAB_ARENA_CHECK(A);
-            OwnerDigit odop;
-            odop.add = (u32)h;
-            odop.lay = lay;
-            A2APlan pr;
-            SAB_TRY((sab_plan_exchange<u32, OwnerDigit>(cm, c, cur_idx, m, nullptr, odop, nullptr, 0, nullptr, 0, &pr, nullptr)));
-            if (m) {
-                SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64(m, PTILE)));
-                SAB_TRY((sab_launch_pass_op<u32, true, OwnerDigit>(c, cur_idx, ipart, nullptr, ppart, m, odop, c->d_gbase)));
-            }
-            const u64 nq = pr.rtotal;
-            u32* q = A.top<u32>(nq + 8);
-            u32* ans = A.top<u32>(nq + 8);
-            SAB_ARENA_CHECK(A);
-            SAB_TRY(sab_comm_exchange(cm, st, pr, ipart, q, sizeof(u32)));
-            if (nq) {
-                sab_prof_begin(c, 4);
-                SAB_LAUNCH(dist_gather_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, (const u32*)q, nq, (u32)h, (u32)lo, lay,
-                           (const u32*)rank_local, ans);
-                sab_prof_end(c);
-                SAB_LAUNCH_CHECK();
-                S.kernel_launches++;
-            }
-            if (lazy) {
-                // b. requests that found EMPTY: key at the owner -> slice that holds the key -> rank back.  Their
-                // number stays on the device until it comes back with the count exchange (one synchronisation).
-                ph.mark(9);
-                u64* keys_u = A.top<u64>(nq + 8);
-                u32* slot_u = A.top<u32>(nq + 8);
-                SAB_ARENA_CHECK(A);
-                u32* d_nu = c->d_counters + 12;
-                SAB_CUDA_TRY(cudaMemsetAsync(d_nu, 0, sizeof(u32), st));
-                if (nq) {
-                    SAB_LAUNCH(dist_lazy_collect_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, (const u32*)q, (const u32*)ans, nq, (u32)h,
-                               lo, d_text, avail, (const u16*)d_lut, base, k, keys_u, slot_u, d_nu);
-                    SAB_LAUNCH_CHECK();
-                    S.kernel_launches++;
-                }
-                A2APlan pu;
-                u64 rows_u[SAB_MAX_RANKS * 32];
-                SAB_TRY((sab_plan_exchange<u64, SplitterDigit>(cm, c, keys_u, nq, d_nu, sdop, d_nu, 1, nullptr, 0, &pu, rows_u)));
-                const u64 nu = rows_u[(size_t)g * (P + 1) + P];
-                ds->resolved_empty += nu;
-                u64* kp = A.top<u64>(nu + 8);
-                u32* sp = A.top<u32>(nu + 8);
-                SAB_ARENA_CHECK(A);
-                if (nu) {
-                    SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64(nu, PTILE)));
-                    SAB_TRY((sab_launch_pass_op<u64, false, SplitterDigit>(c, keys_u, kp, slot_u, sp, nu, sdop, c->d_gbase)));
-                }
-                u64* kq = A.top<u64>(pu.rtotal + 8);
-                u32* rk = A.top<u32>(pu.rtotal + 8);
-                u32* back = A.top<u32>(nu + 8);
-                SAB_ARENA_CHECK(A);
-                SAB_TRY(sab_comm_exchange(cm, st, pu, kp, kq, sizeof(u64)));
-                if (pu.rtotal) {
-                    SAB_LAUNCH(dist_lookup_kernel, (unsigned)div_up64(pu.rtotal, 256), 256, 0, st, sortedK, R, (const u32*)dir_shifted,
-                               dir_shift, (const u64*)kq, pu.rtotal, (u32)sa_off, rk);
-                    SAB_LAUNCH_CHECK();
-                    S.kernel_launches++;
-                }
-                SAB_TRY(sab_comm_exchange_back(cm, st, pu, rk, back, sizeof(u32)));
-                if (nu) {
-                    SAB_LAUNCH(dist_lazy_fill_kernel, (unsigned)div_up64(nu, 256), 256, 0, st, (const u32*)sp, (const u32*)back, nu,
-                               (const u32*)q, (u32)h, (u32)lo, ans, rank_local);
-                    SAB_LAUNCH_CHECK();
-                    S.kernel_launches++;
-                }
-                ph.mark(8);
-            }
-            u32* r2 = A.top<u32>(m + 8);
-            SAB_ARENA_CHECK(A);
-            SAB_TRY(sab_comm_exchange_back(cm, st, pr, ans, r2, sizeof(u32)));
-            if (m) {
-                SAB_LAUNCH(dist_place_keys_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)r1buf, (const u32*)ppart,
-                           (const u32*)r2, m, rb.k[rb.cur]);
-                SAB_LAUNCH_CHECK();
-                S.kernel_launches++;
-            }
-            }  // all-to-all form of steps a, b
-            A.hi = topmark;  // requests, answers and look-up buffers are dead (stream order)
-
-            // c. order inside the groups (as on one GPU: the list is still grouped by r1, ascending)
-            ph.mark(10);
-            u32* upd_idx = A.top<u32>(m + 8);
-            u32* upd_r = A.top<u32>(m + 8);
-            u32* set_pos = rebalanced ? A.top<u32>(m + 8) : nullptr;
-            const u32* sorted_idx = nullptr;
-            int sorted_in = 0;  // which of the two index buffers holds the sorted list
-            SAB_ARENA_CHECK(A);
-            SAB_CUDA_TRY(cudaMemsetAsync(d_m, 0, sizeof(u32), st));  // kept = 0 unless the re-rank says otherwise
-            if (m) {
-                SortBuffers<u64> sb;
-                sb.k[0] = rb.k[rb.cur];
-                sb.k[1] = rb.k[rb.cur ^ 1];
-                sb.v[0] = rb.v[rb.cur];
-                sb.v[1] = rb.v[rb.cur ^ 1];
-                sb.cur = 0;
-                int sorted = 0;
-                if (group_sort_on) {
-                    const u64 used = sab_align_up(m, 64);
-                    const u64 cap_keys = key_cap > used ? key_cap - used : 0;
-                    const u64 cap_vals = val_cap > used ? val_cap - used : 0;
-                    GroupSortSpare sp_;
-                    sp_.k[0] = sb.k[0] + used;
-                    sp_.k[1] = sb.k[1] + used;
-                    sp_.v[0] = sb.v[0] + used;
-                    sp_.v[1] = sb.v[1] + used;
-                    sp_.pos = r1buf;  // the first ranks live in the key words until the re-rank writes them back
-                    sp_.cap = cap_keys < cap_vals ? cap_keys : cap_vals;
-                    if (sp_.cap > val_cap) sp_.cap = val_cap;
-                    if (sp_.cap * 8 >= m) {
-                        u64 nbig = 0;
-                        sorted = sab_group_sort(c, sb, m, 32 + rank_bits, sp_, &S.passes[round], &nbig);
-                        if (sorted < 0) return sorted;
-                        if (nbig * 2 > m) group_sort_on = false;
-                    }
-                }
-                if (!sorted) SAB_TRY(sab_radix_sort<u64>(c, sb, m, 0, 32 + rank_bits, /*iota=*/false, &S.passes[round]));
-                // d. re-rank; newly unique suffixes go to sa[], changed ranks are collected for their owners; the
-                // number of survivors stays on the device and comes back with the count exchange of step e
-                ph.mark(11);
-                u32* out_idx = (sb.cur == 0) ? rb.v[rb.cur ^ 1] : rb.v[rb.cur];
-                const u64 tiles = div_up64(m, SAB_SCAN_TILE);
-                TileState<RerankScan> ts = sab_tile_state<RerankScan>(c, tiles);
-                sab_prof_begin(c, 3);
-                SAB_LAUNCH(rerank_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, st, (const u64*)sb.k[sb.cur], (const u32*)sb.v[sb.cur], m,
-                           (u32*)nullptr, sa_shifted, r1buf, out_idx, upd_idx, upd_r, set_pos, d_m, ts);
-                sab_prof_end(c);
-                SAB_LAUNCH_CHECK();
-                S.kernel_launches++;
-                sorted_idx = sb.v[sb.cur];
-                sorted_in = sb.cur;
-            }
-            if (rebalanced) {
-                // f. new SA entries to the GPUs that hold their positions (before the buffer of the sorted indices
-                // is reused for the next list); a rank with an empty list still takes part in the exchange
-                ph.mark(13);
-                const size_t mark2 = A.hi;
-                u32* kp = A.top<u32>(m + 8);
-                u32* vp = A.top<u32>(m + 8);
-                SAB_ARENA_CHECK(A);
-                SliceDigit sld;
-                for (int i = 0; i < SAB_MAX_RANKS; ++i) sld.start[i] = slice_start[i];
-                sld.pmax = (u32)P - 1;
-                A2APlan ps;
-                SAB_TRY((sab_plan_exchange<u32, SliceDigit>(cm, c, set_pos, m, nullptr, sld, nullptr, 0, nullptr, 0, &ps, nullptr)));
-                if (m) {
-                    SAB_TRY(sab_ensure_lookback(c, (size_t)div_up64(m, PTILE)));
-                    SAB_TRY((sab_launch_pass_op<u32, false, SliceDigit>(c, set_pos, kp, sorted_idx, vp, m, sld, c->d_gbase)));
-                }
-                u32* rp = A.top<u32>(ps.rtotal + 8);
-                u32* ri = A.top<u32>(ps.rtotal + 8);
-                SAB_ARENA_CHECK(A);
-                SAB_TRY(sab_comm_exchange(cm, st, ps, kp, rp, sizeof(u32)));
-                SAB_TRY(sab_comm_exchange(cm, st, ps, vp, ri, sizeof(u32)));
-                if (ps.rtotal) {
-                    SAB_LAUNCH(dist_store_sa_kernel, (unsigned)div_up64(ps.rtotal, 256), 256, 0, st, (const u32*)rp, (const u32*)ri,
-                               ps.rtotal, (u32)sa_off, sa_local);
-                    SAB_LAUNCH_CHECK();
-                    S.kernel_launches++;
-                }
-                A.hi = mark2;
-            }
-            // e. changed ranks to their owners; the same exchange returns every rank's number of survivors
-            ph.mark(12);
-            u64 kept = 0;
-            if (p2p_round) {
-                // all_reduce #1: the survivors add up (termination) and every rank has finished LOADING ranks;
-                // then the stores go straight into the owners' blocks; all_reduce #2: every store has landed
-                SAB_LAUNCH(put_u64_kernel, 1, 1, 0, st, cm->d_small, (const u32*)d_m);
-                SAB_LAUNCH_CHECK();
-                SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small, 1));
-                if (m) {
-                    SAB_LAUNCH(dist_scatter_p2p_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)upd_idx, (const u32*)upd_r, m, lay, pt);
-                    SAB_LAUNCH_CHECK();
-                    S.kernel_launches++;
-                }
-                SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small + 8, 1));
-                SAB_CUDA_TRY(cudaMemcpyAsync(cm->h_small, cm->d_small, sizeof(u64), cudaMemcpyDeviceToHost, st));
-                SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
-                SAB_CUDA_TRY(cudaStreamSynchronize(st));
-                tot = cm->h_small[0];
-                kept = c->h_small[0];
-                ds->p2p_rounds++;
-            } else {
-                u64 rows_k[SAB_MAX_RANKS * 32];
-                SAB_TRY(R_.send_ranks(upd_idx, upd_r, m, d_m, 1, rows_k));
-                kept = rows_k[(size_t)g * (P + 1) + P];
-                tot = 0;
-                for (int s2 = 0; s2 < P; ++s2) tot += rows_k[(size_t)s2 * (P + 1) + P];
-                lead_barrier = true;
-            }
-            if (m && sorted_in != 0 && kept > 0)
-                SAB_CUDA_TRY(cudaMemcpyAsync(rb.v[rb.cur ^ 1], rb.v[rb.cur], kept * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-            A.hi = topmark;
-            rb.cur ^= 1;
-            m = kept;
-            S.active[round] = m;
-            ds->active[round] = tot;
+            const bool p2p_round = run.p2p_ready && run.tot <= p2p_max * (u64)run.P;
+            if (p2p_round) SAB_TRY(run.second_ranks_p2p(h));
+            else SAB_TRY(run.second_ranks_a2a(h));
+            run.A.hi = topmark;  // requests, answers and look-up buffers are dead (stream order)
+            SAB_TRY(run.refine(round));
+            if (run.rebalanced) SAB_TRY(run.new_sa_entries());
+            SAB_TRY(run.rank_updates(p2p_round));
+            run.A.hi = topmark;
+            S.active[round] = run.m;
+            ds->active[round] = run.tot;
             h *= 2;
         }
     }
-    ph.mark(-1);
+    run.ph.mark(PH_END);
     SAB_CUDA_TRY(cudaStreamSynchronize(st));
-    ph.collect(ds->phase_ms, &ds->total_ms);
+    run.ph.collect(ds->phase_ms, &ds->total_ms);
     S.rounds = round;
     S.total_ms = ds->total_ms;
-    res->d_slice = sa_local;
-    res->slice_len = R;
-    res->sa_off = sa_off;
+    res->d_slice = run.sa_local;
+    res->slice_len = run.R;
+    res->sa_off = run.sa_off;
     ds->rounds = round;
-    ds->lazy_isa = lazy ? 1u : 0u;
-    ds->rank_layout = (u32)layout_cyc;
-    ds->rebalanced = rebalanced ? 1u : 0u;
-    ds->fused_exchange = fused ? 1u : 0u;
-    ds->slice_len = R;
-    ds->sa_off = sa_off;
+    ds->lazy_isa = run.lazy ? 1u : 0u;
+    ds->rank_layout = (u32)run.layout_cyc;
+    ds->rebalanced = run.rebalanced ? 1u : 0u;
+    ds->fused_exchange = run.fused ? 1u : 0u;
+    ds->slice_len = run.R;
+    ds->sa_off = run.sa_off;
     ds->all_to_all_bytes = cm->bytes_sent;
     ds->collectives = cm->collectives;
     return SAB_OK;
@@ -1230,7 +1221,7 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
     c->profiling = g_profiling;
     sab200_dist_stats& ds = cm->last;
     memset(&ds, 0, sizeof(ds));
-    const u64 B = n ? div_up64(n, (u64)cm->P) : 1;
+    const u64 B = sab_shard_bounds(n, cm->P, cm->rank).B;
     if (cm->last_want != sab_dist_want(B)) {
         // another text size than last time (every rank sees the same change): arenas may be re-allocated, so all
         // peer mappings are closed first, on every rank, before anybody frees
@@ -1305,11 +1296,11 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
     SAB_CUDA_TRY(cudaStreamSynchronize(st));
     float ms = 0.f;
     cudaEventElapsedTime(&ms, e0, e1);
-    ds.phase_ms[14] = ms;
+    ds.phase_ms[PH_H2D] = ms;
     cudaEventElapsedTime(&ms, e2, e3);
-    ds.phase_ms[15] = ms;
-    c->stats.h2d_ms = ds.phase_ms[14];
-    c->stats.d2h_ms = ds.phase_ms[15];
+    ds.phase_ms[PH_D2H] = ms;
+    c->stats.h2d_ms = ds.phase_ms[PH_H2D];
+    c->stats.d2h_ms = ds.phase_ms[PH_D2H];
     c->event_pool.push_back(e0);
     c->event_pool.push_back(e1);
     c->event_pool.push_back(e2);
@@ -1442,13 +1433,10 @@ static int sab_saca_multi(const u8* s, u64 n, u32* sa, int P, u32* bkt) {
     std::vector<std::thread> th;
     std::vector<u32> parts;
     if (bkt) parts.assign((size_t)P * SAB200_BKT_LEN, 0u);
-    const u64 B = n ? div_up64(n, (u64)P) : 1;
     for (int g = 0; g < P; ++g) {
         th.emplace_back([&, g]() {
-            const u64 lo = (u64)g * B < n ? (u64)g * B : n;
-            const u64 hi = lo + B < n ? lo + B : n;
-            const u64 len = (n - lo) < (hi - lo) + SAB200_SHARD_HALO ? (n - lo) : (hi - lo) + SAB200_SHARD_HALO;
-            rcs[g] = sab_sharded_run(g_multi_comms[g], s + lo, len, n, 0, nullptr, 0, 0, sa, nullptr, nullptr, nullptr,
+            const ShardBounds sh = sab_shard_bounds(n, P, g);
+            rcs[g] = sab_sharded_run(g_multi_comms[g], s + sh.lo, sh.len, n, 0, nullptr, 0, 0, sa, nullptr, nullptr, nullptr,
                                      bkt ? parts.data() + (size_t)g * SAB200_BKT_LEN : nullptr);
         });
     }

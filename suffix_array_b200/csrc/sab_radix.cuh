@@ -158,12 +158,12 @@ struct SplitterDigit {  // destination rank of a key: number of splitters <= key
 //                     all GPUs, so the requests of a round do not pile up on the owners of one region
 struct RankLayout {
     u32 B, pmax, cyc, shift;
-    __device__ __forceinline__ u32 owner(u64 q) const {
+    __host__ __device__ __forceinline__ u32 owner(u64 q) const {
         if (cyc) return (u32)((q >> shift) % (pmax + 1u));
         const u32 o = (u32)(q / B);
         return o < pmax ? o : pmax;
     }
-    __device__ __forceinline__ u64 slot(u64 q, u32 o) const {
+    __host__ __device__ __forceinline__ u64 slot(u64 q, u32 o) const {
         if (cyc) return (((q >> shift) / (pmax + 1u)) << shift) | (q & (u64)(B - 1u));
         return q - (u64)o * B;
     }

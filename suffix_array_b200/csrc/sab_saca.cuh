@@ -79,6 +79,24 @@ __global__ void __launch_bounds__(256) alphabet_hist_kernel(const u8* __restrict
     if (c) atomicAdd(&hist[threadIdx.x], c);
 }
 
+// blocks for n items of per_block each, at most `waves` blocks per SM (grid-stride kernels), at least 1
+static inline unsigned sab_grid(SabContext* c, u64 n, u64 per_block, int waves) {
+    u64 g = div_up64(n, per_block);
+    const u64 gmax = (u64)c->sm_count * (u64)waves;
+    if (g > gmax) g = gmax;
+    return (unsigned)(g ? g : 1);
+}
+
+// byte histogram of text[0..n) into the 256 words at d_hist (zeroed first)
+static int sab_launch_alphabet_hist(SabContext* c, const u8* d_text, u64 n, u32* d_hist) {
+    SAB_CUDA_TRY(cudaMemsetAsync(d_hist, 0, 256 * sizeof(u32), c->stream));
+    if (n == 0) return SAB_OK;
+    SAB_LAUNCH(alphabet_hist_kernel, sab_grid(c, n, 256 * 64, 8), 256, 0, c->stream, d_text, n, d_hist);
+    SAB_LAUNCH_CHECK();
+    c->stats.kernel_launches++;
+    return SAB_OK;
+}
+
 static inline u64 sab_pow_u64(u64 b, int e) {
     u64 r = 1;
     for (int i = 0; i < e; ++i) r *= b;
@@ -306,7 +324,7 @@ bucket_from_keys_kernel(const u64* __restrict__ sorted_keys, u64 cnt, const u16*
     }
     __syncthreads();
     const u32 slot = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot >= 65793u) return;
+    if (slot >= SAB200_BKT_LEN) return;
     if (slot == 0) {
         out[0] = add_one;  // "$": the empty suffix alone
         return;
@@ -374,16 +392,24 @@ static inline int sab_ceil_log2_u64(u64 x) {  // smallest b with 2^b >= x
     return b;
 }
 
-// Code table and key shape from the byte histogram: codes 1..sigma in byte order (0 = absent byte /
-// past the end).  Keys are mixed-radix numbers in base sigma+1 (dense: no bit is wasted on unused
+// What sab_plan_alphabet decided, with its code table on the device.
+struct SabAlphabet {
+    u32 sigma, base;
+    int k, key_bits;
+    const u16* d_lut;
+};
+
+// Code table and key shape from the byte histogram of the whole text (n bytes): codes 1..sigma in byte order (0 =
+// absent byte / past the end).  Keys are mixed-radix numbers in base sigma+1 (dense: no bit is wasted on unused
 // codes, so more symbols fit a radix pass and the key space is evenly filled), k symbols per key,
-// key_bits = bits needed for base^k - 1.
+// key_bits = bits needed for base^k - 1.  The code table goes to the device, the key shape to c->stats.
 //
 // Cost model, in bytes moved per suffix: P radix passes of 24 B each, plus ~SAB_ACTIVE_COST bytes over
 // all doubling rounds for every suffix still tied after the initial sort; a suffix stays tied with
 // probability ~ n * 2^-(k*H2) (H2 = order-0 collision entropy; higher-order structure only makes the
 // estimate optimistic, never the result wrong).
-static void sab_plan_alphabet(const u64* hist, u64 n, u16* lut, u32* sigma_out, u32* base_out, int* k_out, int* key_bits_out) {
+static int sab_plan_alphabet(SabContext* c, const u64* hist, u64 n, SabAlphabet* a) {
+    u16 lut[256];
     u32 sigma = 0;
     double sum_p2 = 0.0;
     for (int ch = 0; ch < 256; ++ch) {
@@ -437,24 +463,74 @@ static void sab_plan_alphabet(const u64* hist, u64 n, u16* lut, u32* sigma_out, 
         }
     }
     if (k < 1) k = 1;
-    *sigma_out = sigma;
-    *base_out = base;
-    *k_out = k;
-    *key_bits_out = bits_of_k[k];
+    a->sigma = sigma;
+    a->base = base;
+    a->k = k;
+    a->key_bits = bits_of_k[k];
+    c->stats.sigma = sigma;
+    c->stats.bits_per_symbol = (u32)sab_ceil_log2_u64(base);
+    c->stats.symbols_per_key = (u32)k;
+    u16* d_lut = (u16*)(c->d_counters + 16 + 256);
+    memcpy(c->h_small + 384, lut, sizeof(lut));  // pinned staging: the async copy must not read the stack later
+    SAB_CUDA_TRY(cudaMemcpyAsync(d_lut, c->h_small + 384, sizeof(lut), cudaMemcpyHostToDevice, c->stream));
+    a->d_lut = d_lut;
+    return SAB_OK;
+}
+
+// The alphabet of a text of n > 0 bytes resident on this GPU.
+static int sab_alphabet_local(SabContext* c, const u8* d_text, u64 n, SabAlphabet* a) {
+    u32* d_hist = c->d_counters + 16;  // 256 words inside the counters block
+    SAB_TRY(sab_launch_alphabet_hist(c, d_text, n, d_hist));
+    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small + 64, d_hist, 256 * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    u64 hist[256];
+    for (int ch = 0; ch < 256; ++ch) hist[ch] = c->h_small[64 + ch];
+    return sab_plan_alphabet(c, hist, n, a);
+}
+
+// Bits of the bucket directory of the lazy inverse suffix array over keys of key_bits bits:
+// 2^(ceil(log2 n) - shift) entries, at most 2^28 and 2^key_bits, at least 2.
+static inline int sab_dir_bits(u64 n, int key_bits, int shift) {
+    int dir_bits = sab_ceil_log2_u64(n) - shift;
+    if (dir_bits > 28) dir_bits = 28;
+    if (dir_bits > key_bits) dir_bits = key_bits;
+    if (dir_bits < 1) dir_bits = 1;
+    return dir_bits;
 }
 
 __global__ void bucket_pairs_kernel(const u8* __restrict__ text, u64 n, const u16* __restrict__ lut, u32 sigma, int dense,
                                     u32* __restrict__ cnt);  // sab_search.cuh
 __global__ void bucket_scan_kernel(u32* __restrict__ bkt);
 
+// The bucket table (SAB200_BKT_LEN inclusive boundaries, + 1 for the empty suffix) into d_bkt by counting the byte
+// pairs of text[0..n); d_lut, sigma: the code table of the text.
+static int sab_pair_buckets(SabContext* c, const u8* d_text, u64 n, const u16* d_lut, u32 sigma, u32* d_bkt) {
+    cudaStream_t st = c->stream;
+    SAB_CUDA_TRY(cudaMemsetAsync(d_bkt, 0, SAB200_BKT_LEN * sizeof(u32), st));
+    if (n > 0) {
+        const size_t tab_bytes = (size_t)sigma * (sigma + 1) * sizeof(u32);
+        const int dense = tab_bytes <= 160 * 1024;
+        const size_t smem = dense ? tab_bytes : 0;
+#ifndef SAB_EMU
+        SAB_CUDA_TRY(cudaFuncSetAttribute(bucket_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+#endif
+        SAB_LAUNCH(bucket_pairs_kernel, sab_grid(c, n, 256 * 64, smem > 64 * 1024 ? 1 : 4), 256, smem, st, d_text, n, d_lut, sigma,
+                   dense, d_bkt);
+        SAB_LAUNCH_CHECK();
+        c->stats.kernel_launches++;
+    }
+    SAB_LAUNCH(bucket_scan_kernel, 1, 1024, 0, st, d_bkt);
+    SAB_LAUNCH_CHECK();
+    c->stats.kernel_launches++;
+    return SAB_OK;
+}
+
 // The bucket table of the running construction into c->want_bkt: from the sorted initial keys (k >= 2), else by
 // the pair-counting kernels over the resident text (tiny texts with large alphabets; single GPU only).
-static int sab_fused_buckets(SabContext* c, const u8* d_text, u64 n, const u64* sortedK, u64 cnt, const u16* d_lut, u32 sigma,
-                             u32 base, int k) {
-    cudaStream_t st = c->stream;
-    if (k >= 2) {
-        SAB_LAUNCH(bucket_from_keys_kernel, (65793u + 255u) / 256u, 256, 0, st, sortedK, cnt, d_lut, base, sab_pow_u64(base, k - 2),
-                   c->bkt_add_one, c->want_bkt);
+static int sab_fused_buckets(SabContext* c, const u8* d_text, u64 n, const u64* sortedK, u64 cnt, const SabAlphabet& al) {
+    if (al.k >= 2) {
+        SAB_LAUNCH(bucket_from_keys_kernel, (SAB200_BKT_LEN + 255u) / 256u, 256, 0, c->stream, sortedK, cnt, al.d_lut, al.base,
+                   sab_pow_u64(al.base, al.k - 2), c->bkt_add_one, c->want_bkt);
         SAB_LAUNCH_CHECK();
         c->stats.kernel_launches++;
         return SAB_OK;
@@ -463,29 +539,76 @@ static int sab_fused_buckets(SabContext* c, const u8* d_text, u64 n, const u64* 
         sab_set_error("fused bucket table: keys of one symbol on a multi-GPU rank");
         return SAB_ERR_INTERNAL;
     }
-    SAB_CUDA_TRY(cudaMemsetAsync(c->want_bkt, 0, 65793u * sizeof(u32), st));
-    const size_t tab_bytes = (size_t)sigma * (sigma + 1) * sizeof(u32);
-    const int dense = tab_bytes <= 160 * 1024;
-#ifndef SAB_EMU
-    SAB_CUDA_TRY(cudaFuncSetAttribute(bucket_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-#endif
-    u64 pblocks = div_up64(n, 256 * 64);
-    const u64 pmax = (u64)c->sm_count * ((dense ? tab_bytes : 0) > 64 * 1024 ? 1 : 4);
-    if (pblocks > pmax) pblocks = pmax;
-    SAB_LAUNCH(bucket_pairs_kernel, (unsigned)pblocks, 256, dense ? tab_bytes : 0, st, d_text, n, d_lut, sigma, dense, c->want_bkt);
+    return sab_pair_buckets(c, d_text, n, al.d_lut, al.sigma, c->want_bkt);
+}
+
+// The spare buffers of the in-group sort (sab_group_sort) of `count` records at the front of sb: the unused tails of
+// the round's buffers behind the first align_up(count, 64) records (sb.k[*] hold key_cap records, sb.v[*] val_cap),
+// and the position list `pos`.
+static inline GroupSortSpare sab_group_sort_spare(const SortBuffers<u64>& sb, u64 count, u64 key_cap, u64 val_cap, u32* pos) {
+    const u64 used = sab_align_up(count, 64);
+    const u64 cap_keys = key_cap > used ? key_cap - used : 0;
+    const u64 cap_vals = val_cap > used ? val_cap - used : 0;
+    GroupSortSpare sp;
+    sp.k[0] = sb.k[0] + used;
+    sp.k[1] = sb.k[1] + used;
+    sp.v[0] = sb.v[0] + used;
+    sp.v[1] = sb.v[1] + used;
+    sp.pos = pos;
+    sp.cap = cap_keys < cap_vals ? cap_keys : cap_vals;
+    return sp;
+}
+
+// The buffers of the doubling rounds, taken from those of the initial sort of cnt records (result in buf.cur): the
+// round keys ping-pong inside the two halves of the free key buffer while the sorted keys are kept (lazy inverse
+// suffix array), else over both key buffers.  *key_cap = records each round key buffer holds.
+static inline SortBuffers<u64> sab_round_buffers(const SortBuffers<u64>& buf, u64 cnt, bool keep_sorted, u64* key_cap) {
+    const u64 half = sab_align_up((size_t)(cnt + 8) / 2, 32);
+    SortBuffers<u64> rb;
+    rb.k[0] = buf.k[buf.cur ^ 1];
+    rb.k[1] = keep_sorted ? buf.k[buf.cur ^ 1] + half : buf.k[buf.cur];
+    *key_cap = keep_sorted ? (cnt + 8) - half : cnt + 8;
+    rb.v[0] = buf.v[buf.cur ^ 1];
+    rb.v[1] = buf.v[buf.cur];
+    rb.cur = 0;
+    return rb;
+}
+
+// init_ranks (4) over the cnt sorted records; *m = the number of records left active
+static int sab_init_ranks(SabContext* c, const u64* sortedK, const u32* sortedI, u64 cnt, u32 rank_base, u32* rank, u32* rank_seq,
+                          u32* sa_out, u32* act_r1, u32* act_idx, u32* dir, int dir_shift, u64* m) {
+    const u64 tiles = div_up64(cnt, SAB_SCAN_TILE);
+    TileState<RankScan> ts = sab_tile_state<RankScan>(c, tiles);
+    sab_prof_begin(c, 3);
+    SAB_LAUNCH(init_ranks_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, c->stream, sortedK, sortedI, cnt, rank_base, rank, rank_seq,
+               sa_out, act_r1, act_idx, c->d_counters, dir, dir_shift, ts);
+    sab_prof_end(c);
     SAB_LAUNCH_CHECK();
-    SAB_LAUNCH(bucket_scan_kernel, 1, 1024, 0, st, c->want_bkt);
+    c->stats.kernel_launches++;
+    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, c->d_counters, sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    *m = c->h_small[0];
+    return SAB_OK;
+}
+
+// re-rank (5) of the cnt sorted records of a round; the number of survivors is left in c->d_counters[0]
+static int sab_launch_rerank(SabContext* c, const SortBuffers<u64>& sb, u64 cnt, u32* rank, u32* sa, u32* out_r1, u32* out_idx,
+                             u32* upd_idx, u32* upd_r, u32* set_pos) {
+    const u64 tiles = div_up64(cnt, SAB_SCAN_TILE);
+    TileState<RerankScan> ts = sab_tile_state<RerankScan>(c, tiles);
+    sab_prof_begin(c, 3);
+    SAB_LAUNCH(rerank_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, c->stream, (const u64*)sb.k[sb.cur], (const u32*)sb.v[sb.cur], cnt,
+               rank, sa, out_r1, out_idx, upd_idx, upd_r, set_pos, c->d_counters, ts);
+    sab_prof_end(c);
     SAB_LAUNCH_CHECK();
-    c->stats.kernel_launches += 2;
+    c->stats.kernel_launches++;
     return SAB_OK;
 }
 
 // bytes of arena needed for a text of n bytes (excluding text and sa, which the caller provides)
 static inline size_t sab_saca_workspace_bytes(u64 n) {
     const size_t N = (size_t)n + 8;
-    int dir_bits = sab_ceil_log2_u64(n) - SAB_DIR_SHIFT;
-    if (dir_bits > 28) dir_bits = 28;
-    if (dir_bits < 1) dir_bits = 1;
+    const int dir_bits = sab_dir_bits(n, 64, SAB_DIR_SHIFT);
     return 2 * sab_align_up(N * 8, 256) + 3 * sab_align_up(N * 4, 256) + sab_align_up((N + 1) * 4, 256) +
            sab_align_up((((size_t)1 << dir_bits) + 8) * 4, 256) + sab_align_up((N / 32 + 8) * 4, 256) + 4096;
 }
@@ -517,76 +640,34 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
 
     // 1. alphabet
     sab_prof_begin(c, 2);
-    u32* d_hist = c->d_counters + 16;  // 256 words inside the counters block
-    SAB_CUDA_TRY(cudaMemsetAsync(d_hist, 0, 256 * sizeof(u32), st));
-    {
-        u64 blocks = div_up64(n, 256 * 64);
-        const u64 bmax = (u64)c->sm_count * 8;
-        if (blocks > bmax) blocks = bmax;
-        SAB_LAUNCH(alphabet_hist_kernel, (unsigned)blocks, 256, 0, st, d_text, n, d_hist);
-        SAB_LAUNCH_CHECK();
-        S.kernel_launches++;
-    }
-    u32 h_hist[256];
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small + 64, d_hist, 256 * sizeof(u32), cudaMemcpyDeviceToHost, st));
-    SAB_CUDA_TRY(cudaStreamSynchronize(st));
-    memcpy(h_hist, c->h_small + 64, sizeof(h_hist));
-    u16 lut[256];
-    u32 sigma = 0;
-    u32 base = 2;
-    int k = 1, key_bits = 1;
-    {
-        u64 h64[256];
-        for (int ch = 0; ch < 256; ++ch) h64[ch] = h_hist[ch];
-        sab_plan_alphabet(h64, n, lut, &sigma, &base, &k, &key_bits);
-    }
-    S.sigma = sigma;
-    S.bits_per_symbol = (u32)sab_ceil_log2_u64(base);
-    S.symbols_per_key = (u32)k;
-    u16* d_lut = (u16*)(c->d_counters + 16 + 256);
-    memcpy(c->h_small + 384, lut, sizeof(lut));  // pinned staging: the async copy must not read the stack later
-    SAB_CUDA_TRY(cudaMemcpyAsync(d_lut, c->h_small + 384, sizeof(lut), cudaMemcpyHostToDevice, st));
+    SabAlphabet al;
+    SAB_TRY(sab_alphabet_local(c, d_text, n, &al));
 
     // 2. packed keys
-    SAB_TRY(sab_launch_pack(c, d_text, n, n, (const u16*)d_lut, base, k, buf.k[0]));
+    SAB_TRY(sab_launch_pack(c, d_text, n, n, al.d_lut, al.base, al.k, buf.k[0]));
     sab_prof_end(c);
 
     // 3. sort (key, i); the payload of the first pass is generated, not read
     // (the last pass writes the sorted indices straight into sa[1..]: they need no copy afterwards)
     bool sa_written = false;
-    SAB_TRY(sab_radix_sort<u64>(c, buf, n, 0, key_bits, /*iota=*/true, &S.passes[0], d_sa + 1, &sa_written));
+    SAB_TRY(sab_radix_sort<u64>(c, buf, n, 0, al.key_bits, /*iota=*/true, &S.passes[0], d_sa + 1, &sa_written));
 
     // 4. ranks, SA skeleton, active list, bucket directory over the sorted keys
     u32* d_m = c->d_counters;
     const u64* sortedK = buf.k[buf.cur];
-    if (c->want_bkt) SAB_TRY(sab_fused_buckets(c, d_text, n, sortedK, n, (const u16*)d_lut, sigma, base, k));
+    if (c->want_bkt) SAB_TRY(sab_fused_buckets(c, d_text, n, sortedK, n, al));
     const u32* sortedI = sa_written ? d_sa + 1 : buf.v[buf.cur];
-    u64* free_keys = buf.k[buf.cur ^ 1];
     u32* act_idx = buf.v[buf.cur ^ 1];
-    int dir_bits = sab_ceil_log2_u64(n) - SAB_DIR_SHIFT;
-    if (dir_bits > 28) dir_bits = 28;
-    if (dir_bits > key_bits) dir_bits = key_bits;
-    if (dir_bits < 1) dir_bits = 1;
-    const int dir_shift = key_bits - dir_bits;
+    const int dir_bits = sab_dir_bits(n, al.key_bits, SAB_DIR_SHIFT);
+    const int dir_shift = al.key_bits - dir_bits;
     u32* dir = sab_arena_take<u32>(c, ((size_t)1 << dir_bits) + 8);
     u32* split_bitmap = sab_arena_take<u32>(c, (size_t)n / 32 + 8);
     SAB_CUDA_TRY(cudaMemsetAsync(rank, 0xff, n * sizeof(u32), st));
     SAB_CUDA_TRY(cudaMemsetAsync(rank + n, 0, sizeof(u32), st));  // the empty suffix has rank 0
     c->h_small[32] = (u32)n;
     SAB_CUDA_TRY(cudaMemcpyAsync(d_sa, c->h_small + 32, sizeof(u32), cudaMemcpyHostToDevice, st));  // sa[0] = n
-    {
-        const u64 tiles = div_up64(n, SAB_SCAN_TILE);
-        TileState<RankScan> ts = sab_tile_state<RankScan>(c, tiles);
-        sab_prof_begin(c, 3);
-        SAB_LAUNCH(init_ranks_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, st, sortedK, sortedI, n, 1u, rank,
-                   (u32*)nullptr, sa_written ? (u32*)nullptr : d_sa + 1, r1buf, act_idx, d_m, dir, dir_shift, ts);
-        sab_prof_end(c);
-        SAB_LAUNCH_CHECK();
-        S.kernel_launches++;
-    }
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    SAB_CUDA_TRY(cudaStreamSynchronize(st));
-    u64 m = c->h_small[0];
+    u64 m = 0;
+    SAB_TRY(sab_init_ranks(c, sortedK, sortedI, n, 1u, rank, nullptr, sa_written ? nullptr : d_sa + 1, r1buf, act_idx, dir, dir_shift, &m));
     S.active[0] = m;
     if (m == 0) {
         S.rounds = 0;
@@ -596,40 +677,25 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     // 4b. lazy or complete inverse suffix array
     LazyIsa z;
     z.text = d_text;
-    z.lut = d_lut;
+    z.lut = al.d_lut;
     z.dir = dir;
     z.n = n;
-    z.base = base;
-    z.k = k;
+    z.base = al.base;
+    z.k = al.k;
     z.dir_shift = dir_shift;
-    SortBuffers<u64> rb;  // buffers of the rounds
-    u64 key_cap;          // records each of rb.k[0], rb.k[1] can hold
-    if (m <= n / 4) {
-        // keep the sorted keys; the composite keys of the rounds ping-pong inside the other key buffer
-        z.sorted_keys = sortedK;
-        rb.k[0] = free_keys;
-        rb.k[1] = free_keys + sab_align_up((size_t)(n + 8) / 2, 32);
-        key_cap = (n + 8) - sab_align_up((size_t)(n + 8) / 2, 32);
-        rb.v[0] = act_idx;
-        rb.v[1] = buf.v[buf.cur];
-        rb.cur = 0;
-    } else {
-        z.sorted_keys = nullptr;
+    z.sorted_keys = m <= n / 4 ? sortedK : nullptr;  // keep the sorted keys
+    if (!z.sorted_keys) {
         sab_prof_begin(c, 3);
         SAB_LAUNCH(fill_settled_ranks_kernel, (unsigned)div_up64(n, 256), 256, 0, st, sortedK, sortedI, n, rank);
         sab_prof_end(c);
         SAB_LAUNCH_CHECK();
         S.kernel_launches++;
-        rb.k[0] = buf.k[buf.cur ^ 1];
-        rb.k[1] = buf.k[buf.cur];
-        key_cap = n + 8;
-        rb.v[0] = act_idx;
-        rb.v[1] = buf.v[buf.cur];
-        rb.cur = 0;
     }
+    u64 key_cap;  // records each of rb.k[0], rb.k[1] can hold
+    SortBuffers<u64> rb = sab_round_buffers(buf, n, z.sorted_keys != nullptr, &key_cap);
 
     // 5. doubling rounds
-    u64 h = (u64)k;
+    u64 h = (u64)al.k;
     u32 round = 0;
     const int rank_bits = sab_ceil_log2_u64(n + 2);
     // the split filter (5c) pays off while few groups split: repetitive texts, early rounds
@@ -688,16 +754,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
             // the unused tails of the round buffers (keys, payloads) and of r1buf (positions)
             int sorted = 0;
             if (group_sort_on) {
-                const u64 used = sab_align_up(n_sort, 64);
-                const u64 cap_keys = key_cap > used ? key_cap - used : 0;
-                const u64 cap_vals = n + 8 > n_stay + used ? n + 8 - n_stay - used : 0;
-                GroupSortSpare sp;
-                sp.k[0] = sb.k[0] + used;
-                sp.k[1] = sb.k[1] + used;
-                sp.v[0] = sb.v[0] + used;
-                sp.v[1] = sb.v[1] + used;
-                sp.pos = r1buf + n_stay;
-                sp.cap = cap_keys < cap_vals ? cap_keys : cap_vals;
+                const GroupSortSpare sp = sab_group_sort_spare(sb, n_sort, key_cap, n + 8 - n_stay, r1buf + n_stay);
                 // the sweep is tried whenever there is any spare room: it reports how many records belong to
                 // large groups even when they do not fit (then the round takes the radix sort and the sweep
                 // pauses for two rounds -- the list, and with it the need for room, only shrinks)
@@ -716,17 +773,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
                 order_restored = true;
             }
             u32* out_idx = (sb.cur == 0) ? rb.v[rb.cur ^ 1] + n_stay : rb.v[rb.cur];
-            {
-                const u64 tiles = div_up64(n_sort, SAB_SCAN_TILE);
-                TileState<RerankScan> ts = sab_tile_state<RerankScan>(c, tiles);
-                sab_prof_begin(c, 3);
-                SAB_LAUNCH(rerank_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, st, (const u64*)sb.k[sb.cur],
-                           (const u32*)sb.v[sb.cur], n_sort, rank, d_sa, r1buf + n_stay, out_idx, (u32*)nullptr, (u32*)nullptr,
-                           (u32*)nullptr, d_m, ts);
-                sab_prof_end(c);
-                SAB_LAUNCH_CHECK();
-                S.kernel_launches++;
-            }
+            SAB_TRY(sab_launch_rerank(c, sb, n_sort, rank, d_sa, r1buf + n_stay, out_idx, nullptr, nullptr, nullptr));
             SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
             SAB_CUDA_TRY(cudaStreamSynchronize(st));
             kept = c->h_small[0];

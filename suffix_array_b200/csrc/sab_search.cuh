@@ -11,7 +11,6 @@
 #pragma once
 #include "sab_context.cuh"
 
-#define SAB_BKT_LEN 65793u
 // 4 lanes per pattern (16 bytes per compare step): with the prefix directory a query is ~7 probes and most of them
 // differ inside the first 16 bytes; 10 M patterns of 8..64 B on the 1 GiB index: 1.61 / 1.89 G queries/s against
 // 1.25 / 1.47 with 8 lanes (profiles/r02_search_variants.txt)
@@ -24,7 +23,7 @@
 // ------------------------------------------------------------------ enable_buckets
 // Dense path: the byte pairs are counted in a shared table indexed by (code(c0), code'(c1)) of the
 // bytes present in the text; sparse path (large alphabets): global atomics straight into the table.
-// cnt[] has SAB_BKT_LEN u32 slots, zeroed by the caller; slot layout as in src/sa.rs:94,103,107.
+// cnt[] has SAB200_BKT_LEN u32 slots, zeroed by the caller; slot layout as in src/sa.rs:94,103,107.
 __global__ void __launch_bounds__(256)
 bucket_pairs_kernel(const u8* __restrict__ text, u64 n, const u16* __restrict__ lut, u32 sigma, int dense,
                     u32* __restrict__ cnt) {
@@ -68,13 +67,13 @@ bucket_pairs_kernel(const u8* __restrict__ text, u64 n, const u16* __restrict__ 
 // accounts for the empty suffix (src/sa.rs:98).  One block of 1024 threads.
 __global__ void __launch_bounds__(1024) bucket_scan_kernel(u32* __restrict__ bkt) {
     SAB_SHARED_ARRAY(u32, s_w, 32);
-    constexpr u32 PER = (SAB_BKT_LEN + 1023u) / 1024u;  // 65
+    constexpr u32 PER = (SAB200_BKT_LEN + 1023u) / 1024u;  // 65
     const u32 t = threadIdx.x, lane = lane_id(), w = warp_id();
     const u32 b0 = t * PER;
     u32 sum = 0;
     for (u32 i = 0; i < PER; ++i) {
         const u32 j = b0 + i;
-        if (j < SAB_BKT_LEN) sum += bkt[j] + (j == 0 ? 1u : 0u);
+        if (j < SAB200_BKT_LEN) sum += bkt[j] + (j == 0 ? 1u : 0u);
     }
     u32 incl = warp_incl_sum(sum);
     if (lane == 31) s_w[w] = incl;
@@ -88,7 +87,7 @@ __global__ void __launch_bounds__(1024) bucket_scan_kernel(u32* __restrict__ bkt
     u32 run = incl - sum + (w ? s_w[w - 1] : 0u);
     for (u32 i = 0; i < PER; ++i) {
         const u32 j = b0 + i;
-        if (j < SAB_BKT_LEN) {
+        if (j < SAB200_BKT_LEN) {
             run += bkt[j] + (j == 0 ? 1u : 0u);
             bkt[j] = run;
         }
@@ -177,7 +176,7 @@ struct SearchArgs {
     const u8* text;   // n bytes (+ padding)
     u64 n;
     const u32* sa;    // n + 1
-    const u32* bkt;   // SAB_BKT_LEN or null
+    const u32* bkt;   // SAB200_BKT_LEN or null
     const u8* pats;   // concatenated patterns (+ padding)
     const u64* offs;  // np + 1
     u64 np;
