@@ -14,6 +14,7 @@
 
 static_assert(sizeof(SabStats) == sizeof(sab200_stats), "SabStats must mirror sab200_stats");
 static_assert(SAB_MAX_ROUNDS == SAB200_MAX_ROUNDS, "round table size");
+static_assert(SAB_MAX_PASSES * sizeof(u32) <= sizeof(SabScratch::skip), "a skip flag for every radix pass");
 
 // ------------------------------------------------------------------ error string
 static char g_err[1024] = "";
@@ -41,16 +42,11 @@ int sab_context_init(SabContext* c) {
     SAB_CUDA_TRY(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     SAB_CUDA_TRY(cudaMalloc(&c->d_ghist, sizeof(u64) * SAB_MAX_PASSES * SAB_RADIX_BINS));
     SAB_CUDA_TRY(cudaMalloc(&c->d_gbase, sizeof(u64) * SAB_MAX_PASSES * SAB_RADIX_BINS));
-    SAB_CUDA_TRY(cudaMalloc(&c->d_skip, sizeof(u32) * 16));
-    SAB_CUDA_TRY(cudaMallocHost(&c->h_small, sizeof(u32) * 4096));
+    SAB_CUDA_TRY(cudaMallocHost(&c->staging, sizeof(SabStaging)));
     SAB_CUDA_TRY(cudaMalloc(&c->d_ticket, sizeof(u32) * 4));
     SAB_CUDA_TRY(cudaMemset(c->d_ticket, 0, sizeof(u32) * 4));
-    SAB_CUDA_TRY(cudaMalloc(&c->d_counters, sizeof(u32) * 1024));
-    SAB_CUDA_TRY(cudaMemset(c->d_counters, 0, sizeof(u32) * 1024));
-    c->ticket_host = 0;
-    c->lb_epoch = 0;
-    c->scan_epoch = 0;
-    c->ready = true;
+    SAB_CUDA_TRY(cudaMalloc(&c->scratch, sizeof(SabScratch)));
+    SAB_CUDA_TRY(cudaMemset(c->scratch, 0, sizeof(SabScratch)));
     return SAB_OK;
 }
 
@@ -65,8 +61,7 @@ void sab_context_destroy(SabContext* c) {
     for (auto e : c->event_pool) cudaEventDestroy(e);
     cudaFree(c->d_ghist);
     cudaFree(c->d_gbase);
-    cudaFree(c->d_skip);
-    cudaFreeHost(c->h_small);
+    cudaFreeHost(c->staging);
     for (int i = 0; i < 2; ++i) {
         if (c->bounce[i]) cudaFreeHost(c->bounce[i]);
         if (c->bounce_ev[i]) cudaEventDestroy(c->bounce_ev[i]);
@@ -74,7 +69,7 @@ void sab_context_destroy(SabContext* c) {
     cudaFree(c->d_lookback);
     cudaFree(c->d_ticket);
     cudaFree(c->d_scan_slots);
-    cudaFree(c->d_counters);
+    cudaFree(c->scratch);
     cudaFree(c->arena);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
@@ -171,7 +166,7 @@ cudaEvent_t sab_event_get(SabContext* c) {
     cudaEventCreate(&e);
     return e;
 }
-void sab_prof_begin(SabContext* c, int kind) {
+void sab_prof_begin(SabContext* c, SabProfKind kind) {
     if (!c->profiling) return;
     SabEventPair p;
     p.a = sab_event_get(c);
@@ -191,12 +186,12 @@ void sab_prof_collect(SabContext* c) {
         float ms = 0.f;
         cudaEventElapsedTime(&ms, p.a, p.b);
         switch (p.kind) {
-            case 0: c->stats.radix_pass_ms += ms; break;
-            case 1: c->stats.hist_ms += ms; break;
-            case 2: c->stats.pack_ms += ms; break;
-            case 3: c->stats.rank_ms += ms; break;
-            case 4: c->stats.gather_ms += ms; break;
-            case 5: c->stats.group_sort_ms += ms; break;
+            case SAB_PROF_RADIX_PASS: c->stats.radix_pass_ms += ms; break;
+            case SAB_PROF_HIST: c->stats.hist_ms += ms; break;
+            case SAB_PROF_PACK: c->stats.pack_ms += ms; break;
+            case SAB_PROF_RANK: c->stats.rank_ms += ms; break;
+            case SAB_PROF_GATHER: c->stats.gather_ms += ms; break;
+            case SAB_PROF_GROUP_SORT: c->stats.group_sort_ms += ms; break;
         }
         c->event_pool.push_back(p.a);
         c->event_pool.push_back(p.b);
@@ -314,6 +309,13 @@ static double now_ms() {
     return duration<double, std::milli>(steady_clock::now().time_since_epoch()).count();
 }
 
+// a failed launch may have left the ticket counter of the radix passes out of step with its host mirror
+static void sab_reset_after_failure(SabContext* c) {
+    cudaMemsetAsync(c->d_ticket, 0, sizeof(u32) * 4, c->stream);
+    cudaStreamSynchronize(c->stream);
+    c->ticket_host = 0;
+}
+
 static int run_device(SabContext* c, const u8* d_s, u64 n, u32* d_sa) {
     c->profiling = g_profiling;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -329,12 +331,7 @@ static int run_device(SabContext* c, const u8* d_s, u64 n, u32* d_sa) {
     cudaEventDestroy(e1);
     sab_prof_collect(c);
     c->stats.total_ms = ms;
-    if (rc != SAB_OK) {
-        // a failed launch may have left the ticket counter out of step with its host mirror
-        cudaMemsetAsync(c->d_ticket, 0, sizeof(u32) * 4, c->stream);
-        cudaStreamSynchronize(c->stream);
-        c->ticket_host = 0;
-    }
+    if (rc != SAB_OK) sab_reset_after_failure(c);
     return rc;
 }
 
@@ -349,12 +346,10 @@ int32_t sab200_saca_device(const uint8_t* d_s, uint64_t n, uint32_t* d_sa, int32
         sab_set_error("sab200_saca_device: bad arguments (n=%llu)", (unsigned long long)n);
         return SAB_ERR_ARGS;
     }
-    SabContext* c = sab_get_context(device);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
-    int rc = run_device(c, d_s, n, d_sa);
-    g_last_stats = c->stats;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    int rc = run_device(u.c, d_s, n, d_sa);
+    g_last_stats = u.c->stats;
     return rc;
 }
 
@@ -386,19 +381,14 @@ static int32_t saca_host(const uint8_t* s, uint64_t n, uint32_t* sa, uint32_t* b
     }
     if (bkt && n < ((u64)1 << 20)) ngpus = 1;  // tiny texts may pack a single symbol per key: the table then needs the text
     if (ngpus > 1) return sab_saca_multi(s, n, sa, ngpus, bkt);
-    SabContext* c = sab_get_context(0);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
-    // text and SA live at the top of the arena, the construction scratch below them
-    const size_t text_bytes = sab_align_up((size_t)n + 64, 256);
-    const size_t sa_bytes = sab_align_up(((size_t)n + 1) * sizeof(u32), 256);
-    const size_t work = sab_saca_workspace_bytes(n);
-    const size_t bkt_bytes = sab_align_up((size_t)SAB200_BKT_LEN * sizeof(u32), 256);
-    SAB_TRY(sab_arena_reserve(c, work + text_bytes + sa_bytes + bkt_bytes + 512));
-    u8* d_s = (u8*)(c->arena + sab_align_up(work, 256));
-    u32* d_sa = (u32*)((char*)d_s + text_bytes);
-    u32* d_bkt = (u32*)((char*)d_sa + sa_bytes);
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    SabContext* c = u.c;
+    // the construction workspace first (sab_saca_device takes it from the bottom), text, SA and bucket table above it
+    u8* d_s;
+    u32 *d_sa, *d_bkt;
+    SAB_TRY(sab_arena_carve(c, {{nullptr, sab_saca_workspace_bytes(n)}, {&d_s, (size_t)n + 64}, {&d_sa, ((size_t)n + 1) * sizeof(u32)},
+                                {&d_bkt, (size_t)SAB200_BKT_LEN * sizeof(u32)}}));
     c->want_bkt = bkt ? d_bkt : nullptr;
     c->bkt_add_one = 1;
     double t0 = now_ms();
@@ -432,14 +422,12 @@ extern "C" int32_t sab200_enable_buckets(const uint8_t* s, uint64_t n, uint32_t*
         sab_set_error("sab200_enable_buckets: bad arguments");
         return SAB_ERR_ARGS;
     }
-    SabContext* c = sab_get_context(0);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
-    const size_t text_bytes = sab_align_up((size_t)n + 64, 256);
-    SAB_TRY(sab_arena_reserve(c, text_bytes + SAB200_BKT_LEN * sizeof(u32) + 1024));
-    u8* d_s = (u8*)c->arena;
-    u32* d_bkt = (u32*)(c->arena + text_bytes);
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    SabContext* c = u.c;
+    u8* d_s;
+    u32* d_bkt;
+    SAB_TRY(sab_arena_carve(c, {{&d_s, (size_t)n + 64}, {&d_bkt, (size_t)SAB200_BKT_LEN * sizeof(u32)}}));
     if (n) SAB_CUDA_TRY(cudaMemcpyAsync(d_s, s, n, cudaMemcpyHostToDevice, c->stream));
     SabAlphabet al = {};
     if (n) SAB_TRY(sab_alphabet_local(c, d_s, n, &al));
@@ -456,18 +444,15 @@ extern "C" int32_t sab200_check(const uint8_t* s, uint64_t n, const uint32_t* sa
         return SAB_ERR_ARGS;
     }
     if (sa_len != n + 1) return 0;  // src/sa.rs:73-75
-    SabContext* c = sab_get_context(0);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
     const size_t text_bytes = sab_align_up((size_t)n + 64, 256);
     const size_t arr_bytes = sab_align_up(((size_t)n + 2) * sizeof(u32), 256);
-    SAB_TRY(sab_arena_reserve(c, text_bytes + 2 * arr_bytes + 1024));
-    u8* d_s = (u8*)c->arena;
-    u32* d_sa = (u32*)(c->arena + text_bytes);
-    u32* d_isa = (u32*)(c->arena + text_bytes + arr_bytes);
-    u32* d_flag = c->d_counters + 8;
-    cudaStream_t st = c->stream;
+    u8* d_s;
+    u32 *d_sa, *d_isa;
+    SAB_TRY(sab_arena_carve(u.c, {{&d_s, text_bytes}, {&d_sa, arr_bytes}, {&d_isa, arr_bytes}}));
+    u32* d_flag = &u.c->scratch->check_flag;
+    cudaStream_t st = u.c->stream;
     SAB_CUDA_TRY(cudaMemsetAsync(d_s, 0, text_bytes, st));
     if (n) SAB_CUDA_TRY(cudaMemcpyAsync(d_s, s, n, cudaMemcpyHostToDevice, st));
     SAB_CUDA_TRY(cudaMemcpyAsync(d_sa, sa, sa_len * sizeof(u32), cudaMemcpyHostToDevice, st));
@@ -478,9 +463,9 @@ extern "C" int32_t sab200_check(const uint8_t* s, uint64_t n, const uint32_t* sa
     SAB_LAUNCH_CHECK();
     SAB_LAUNCH(sufcheck_order_kernel, blocks, 256, 0, st, (const u8*)d_s, (const u32*)d_sa, sa_len, n, (const u32*)d_isa, d_flag);
     SAB_LAUNCH_CHECK();
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_flag, sizeof(u32), cudaMemcpyDeviceToHost, st));
-    SAB_CUDA_TRY(cudaStreamSynchronize(st));
-    return c->h_small[0] ? 0 : 1;
+    u32 bad;
+    SAB_TRY(sab_read_u32(u.c, d_flag, 1, &bad));
+    return bad ? 0 : 1;
 }
 
 // ---- LCP array ------------------------------------------------------------------------------
@@ -489,18 +474,13 @@ extern "C" int32_t sab200_lcp_array(const uint8_t* s, uint64_t n, const uint32_t
         sab_set_error("sab200_lcp_array: bad arguments (n=%llu, sa_len=%llu)", (unsigned long long)n, (unsigned long long)sa_len);
         return SAB_ERR_ARGS;
     }
-    SabContext* c = sab_get_context(0);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
-    const size_t text_bytes = sab_align_up((size_t)n + 64, 256);
-    const size_t arr_bytes = sab_align_up(((size_t)n + 2) * sizeof(u32), 256);
-    SAB_TRY(sab_arena_reserve(c, text_bytes + 3 * arr_bytes + 1024));
-    u8* d_s = (u8*)c->arena;
-    u32* d_sa = (u32*)(c->arena + text_bytes);
-    u32* d_isa = (u32*)(c->arena + text_bytes + arr_bytes);
-    u32* d_lcp = (u32*)(c->arena + text_bytes + 2 * arr_bytes);
-    cudaStream_t st = c->stream;
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    const size_t arr_bytes = ((size_t)n + 2) * sizeof(u32);
+    u8* d_s;
+    u32 *d_sa, *d_isa, *d_lcp;
+    SAB_TRY(sab_arena_carve(u.c, {{&d_s, (size_t)n + 64}, {&d_sa, arr_bytes}, {&d_isa, arr_bytes}, {&d_lcp, arr_bytes}}));
+    cudaStream_t st = u.c->stream;
     if (n) SAB_CUDA_TRY(cudaMemcpyAsync(d_s, s, n, cudaMemcpyHostToDevice, st));
     SAB_CUDA_TRY(cudaMemcpyAsync(d_sa, sa, sa_len * sizeof(u32), cudaMemcpyHostToDevice, st));
     SAB_LAUNCH(lcp_isa_kernel, (unsigned)div_up64(sa_len, 256), 256, 0, st, (const u32*)d_sa, sa_len, d_isa);
@@ -558,25 +538,19 @@ static void replica_free(SabReplica& r) {
     r = SabReplica();
 }
 
-// The prefix directory over the resident text and suffix array: alphabet from a byte histogram on the device, depth
-// = the most symbols whose codes number at most n / 8 (between 2^16 and 2^27 entries), one sweep over the suffix
-// array.  Running out of memory for it is not an error: the queries then bisect the whole bucket.
+// The prefix directory over the resident text and suffix array, under the context's lock: alphabet from a byte
+// histogram on the device, depth = the most symbols whose codes number at most n / 8 (between 2^16 and 2^27 entries),
+// one sweep over the suffix array.  Running out of memory for it is not an error: the queries then bisect the bucket.
 static int replica_build_prefix_dir(SabReplica& r, u64 n) {
     SabContext* c = r.ctx;
     cudaStream_t st = c->stream;
-    std::lock_guard<std::mutex> lk(c->mu);
-    u32* d_hist = c->d_counters + 16;
-    SAB_CUDA_TRY(cudaMemsetAsync(d_hist, 0, 256 * sizeof(u32), st));
-    u64 blocks = div_up64(n, 256 * 64);
-    if (blocks > (u64)c->sm_count * 8) blocks = (u64)c->sm_count * 8;
-    SAB_LAUNCH(alphabet_hist_kernel, (unsigned)blocks, 256, 0, st, (const u8*)r.d_text, n, d_hist);
-    SAB_LAUNCH_CHECK();
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small + 64, d_hist, 256 * sizeof(u32), cudaMemcpyDeviceToHost, st));
-    SAB_CUDA_TRY(cudaStreamSynchronize(st));
-    u16 lut[256];
+    SAB_TRY(sab_launch_alphabet_hist(c, r.d_text, n, c->scratch->hist));
+    u32 hist[256];
+    SAB_TRY(sab_read_u32(c, c->scratch->hist, 256, hist));
+    u16* lut = c->staging->lut;  // pinned: the upload below is asynchronous
     u32 sigma = 0;
     for (int ch = 0; ch < 256; ++ch) {
-        const bool present = c->h_small[64 + ch] != 0;
+        const bool present = hist[ch] != 0;
         lut[ch] = (u16)(sigma | (present ? 0x8000u : 0u));
         if (present) ++sigma;
     }
@@ -595,12 +569,9 @@ static int replica_build_prefix_dir(SabReplica& r, u64 n) {
         r.d_pdir = nullptr;
         return SAB_OK;
     }
-    SAB_CUDA_TRY(cudaMalloc(&r.d_plut, sizeof(lut)));
-    memcpy(c->h_small + 384, lut, sizeof(lut));  // pinned staging
-    SAB_CUDA_TRY(cudaMemcpyAsync(r.d_plut, c->h_small + 384, sizeof(lut), cudaMemcpyHostToDevice, st));
-    u64 fblocks = div_up64(entries + 1, 256 * 8);
-    if (fblocks > (u64)c->sm_count * 16) fblocks = (u64)c->sm_count * 16;
-    SAB_LAUNCH(fill_u32_kernel, (unsigned)fblocks, 256, 0, st, r.d_pdir, entries + 1, (u32)(n + 1));
+    SAB_CUDA_TRY(cudaMalloc(&r.d_plut, sizeof(c->staging->lut)));
+    SAB_CUDA_TRY(cudaMemcpyAsync(r.d_plut, lut, sizeof(c->staging->lut), cudaMemcpyHostToDevice, st));
+    SAB_LAUNCH(fill_u32_kernel, sab_grid(c, entries + 1, 256 * 8, 16), 256, 0, st, r.d_pdir, entries + 1, (u32)(n + 1));
     SAB_LAUNCH_CHECK();
     SAB_LAUNCH(prefix_dir_kernel, (unsigned)div_up64(n + 1, 256), 256, 0, st, (const u8*)r.d_text, n, (const u32*)r.d_sa, n + 1,
                (const u16*)r.d_plut, base, depth, r.d_pdir);
@@ -616,9 +587,9 @@ static int replica_build_prefix_dir(SabReplica& r, u64 n) {
 }
 
 static int replica_init(SabReplica& r, int device, const u8* s, u64 n, const u32* sa, const u32* bkt) {
-    r.ctx = sab_get_context(device);
-    if (!r.ctx) return SAB_ERR_CUDA;
-    SAB_CUDA_TRY(cudaSetDevice(device));
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    r.ctx = u.c;
     cudaStream_t st = r.ctx->stream;
     const size_t text_bytes = sab_align_up((size_t)n + 64, 256);
     SAB_CUDA_TRY(cudaMalloc(&r.d_text, text_bytes));
@@ -854,15 +825,11 @@ extern "C" int32_t sab200_pack(const uint32_t* sa, uint64_t sa_len, uint8_t* out
         sab_set_error("sab200_pack: output buffer too small (need %llu bytes)", (unsigned long long)(16 + words * 4));
         return SAB_ERR_ARGS;
     }
-    SabContext* c = sab_get_context(0);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
-    const size_t in_bytes = sab_align_up((size_t)sa_len * 4 + 64, 256);
-    SAB_TRY(sab_arena_reserve(c, in_bytes + (size_t)words * 4 + 1024));
-    u32* d_sa = (u32*)c->arena;
-    u32* d_out = (u32*)(c->arena + in_bytes);
-    cudaStream_t st = c->stream;
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    u32 *d_sa, *d_out;
+    SAB_TRY(sab_arena_carve(u.c, {{&d_sa, (size_t)sa_len * 4 + 64}, {&d_out, (size_t)words * 4}}));
+    cudaStream_t st = u.c->stream;
     SAB_CUDA_TRY(cudaMemcpyAsync(d_sa, sa, sa_len * 4, cudaMemcpyHostToDevice, st));
     if (words) {
         SAB_LAUNCH(pack_blocks_kernel, (unsigned)div_up64(words, 256), 256, 0, st, (const u32*)d_sa, sa_len, bits, words, d_out);
@@ -902,15 +869,12 @@ extern "C" int32_t sab200_unpack(const uint8_t* bytes, uint64_t nbytes, uint32_t
                       (unsigned long long)dlen);
         return SAB_ERR_ARGS;
     }
-    SabContext* c = sab_get_context(0);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
     const size_t in_bytes = sab_align_up((size_t)words * 4 + 64, 256);
-    SAB_TRY(sab_arena_reserve(c, in_bytes + (size_t)length * 4 + 1024));
-    u32* d_in = (u32*)c->arena;
-    u32* d_sa = (u32*)(c->arena + in_bytes);
-    cudaStream_t st = c->stream;
+    u32 *d_in, *d_sa;
+    SAB_TRY(sab_arena_carve(u.c, {{&d_in, in_bytes}, {&d_sa, (size_t)length * 4}}));
+    cudaStream_t st = u.c->stream;
     SAB_CUDA_TRY(cudaMemsetAsync(d_in, 0, in_bytes, st));  // re-pads the trimmed tail (src/packed_sa.rs:80-85)
     if (dlen) SAB_CUDA_TRY(cudaMemcpyAsync(d_in, bytes + 16, dlen, cudaMemcpyHostToDevice, st));
     SAB_LAUNCH(unpack_blocks_kernel, (unsigned)div_up64(length, 256), 256, 0, st, (const u32*)d_in, (u64)length, bits, d_sa);

@@ -4,6 +4,8 @@
 #pragma once
 #include <stdarg.h>
 
+#include <cstddef>
+#include <initializer_list>
 #include <mutex>
 #include <vector>
 
@@ -37,22 +39,40 @@ struct SabStats {
     u64 group_big_records;        // ... of which in groups too large for it (radix-sorted)
 };
 
+enum SabProfKind { SAB_PROF_RADIX_PASS, SAB_PROF_HIST, SAB_PROF_PACK, SAB_PROF_RANK, SAB_PROF_GATHER, SAB_PROF_GROUP_SORT };
+
 struct SabEventPair {
     cudaEvent_t a, b;
-    int kind;  // 0 radix pass, 1 hist, 2 pack, 3 rank, 4 gather, 5 group sort
+    SabProfKind kind;  // the SabStats timing the pair adds to (sab_prof_collect)
+};
+
+// Device scalars and small tables of a context: one member per user, so no step overwrites a value another still needs.
+struct SabScratch {
+    u32 count;      // init_ranks / re-rank: records still active
+    u32 filter[2];  // split filter: records to sort, records parked
+    u32 check_flag; // sab200_check: set when the array is not the suffix array of the text
+    u32 big;        // in-group sort: records of groups too large for it
+    u32 nu;         // multi-GPU lazy look-ups: requests that found no rank
+    u32 skip[16];   // radix sort: 1 for each digit place where all keys agree (SAB_MAX_PASSES of them)
+    u32 hist[256];  // byte histogram of a text
+    u16 lut[256];   // code table of the running construction (sab_plan_alphabet)
+};
+
+// Pinned host staging of a context: readbacks land here, and small uploads leave from here, not from the caller's stack.
+struct SabStaging {
+    u32 read[256];  // sab_read_u32
+    u32 sa0;        // sa[0] = n of a single-GPU construction
+    u16 lut[256];   // a code table, built here for its asynchronous upload
+    u64 wide[256];  // u64 rows of the multi-GPU driver, both ways
 };
 
 struct SabContext {
     int device = 0;
-    bool ready = false;
     cudaStream_t stream = 0;
     int sm_count = 148;
     // radix scratch
     u64* d_ghist = nullptr;   // [8][256]
     u64* d_gbase = nullptr;   // [8][256]
-    u32* d_skip = nullptr;    // [8]
-    u32* h_small = nullptr;   // pinned, 4096 words: [0,16) counters read back, [32] sentinel staging, [64,320) byte
-                              // histogram, [384,512) code table staging, [1024,2048) 512 u64 of count / base staging
     u64* d_lookback = nullptr;
     size_t lookback_tiles = 0;
     u32* d_ticket = nullptr;
@@ -62,17 +82,17 @@ struct SabContext {
     ScanSlot* d_scan_slots = nullptr;  // chained-scan status, one 16-byte slot per tile
     size_t scan_tiles = 0;
     u32 scan_epoch = 0;
-    u32* d_counters = nullptr;  // 1024 words: [0,16) device scalars (counts of the scans), [16,272) byte histogram,
-                                // [272,400) code table (256 x u16)
+    SabScratch* scratch = nullptr;  // device
+    SabStaging* staging = nullptr;  // pinned host
     // arena
     char* arena = nullptr;
     size_t arena_bytes = 0;
     size_t arena_used = 0;
-    size_t arena_want_seen = 0;
+    size_t arena_want_seen = 0;  // request the arena was last sized for (it may have been capped by the free memory)
     void* bounce[2] = {nullptr, nullptr};        // pinned bounce buffers for pageable caller memory (sab_copy_*)
     cudaEvent_t bounce_ev[2] = {nullptr, nullptr};
     u32* want_bkt = nullptr;     // device buffer for the fused bucket table of the running construction (or null)
-    u32 bkt_add_one = 1;  // request the arena was last sized for (it may have been capped by the free memory)
+    u32 bkt_add_one = 1;  // added to every boundary of the fused table: 1 counts the empty suffix, 0 for a rank's share
     // profiling
     bool profiling = false;
     std::vector<SabEventPair> events;
@@ -98,10 +118,53 @@ static inline T* sab_arena_take(SabContext* c, size_t count) {
     return (T*)(c->arena + off);
 }
 
+// One buffer of an entry point's arena: *dst receives its address; a null dst reserves the room without handing it out.
+struct SabSlice {
+    void** dst;
+    size_t bytes;
+    template <typename T>
+    SabSlice(T** p, size_t b) : dst((void**)p), bytes(b) {}
+    SabSlice(std::nullptr_t, size_t b) : dst(nullptr), bytes(b) {}
+};
+
+// Reserves the sum of the 256-aligned sizes and hands the buffers out in order from the bottom of the arena.
+static inline int sab_arena_carve(SabContext* c, std::initializer_list<SabSlice> slices) {
+    size_t total = 0;
+    for (const SabSlice& s : slices) total += sab_align_up(s.bytes, 256);
+    SAB_TRY(sab_arena_reserve(c, total));
+    c->arena_used = 0;
+    for (const SabSlice& s : slices) {
+        char* p = sab_arena_take<char>(c, s.bytes);
+        if (s.dst) *s.dst = p;
+    }
+    return SAB_OK;
+}
+
+// The context of `device`, locked and current on the calling thread: the prologue of the entry points.
+struct SabUse {
+    SabContext* c = nullptr;
+    std::unique_lock<std::mutex> lk;
+};
+static inline int sab_use(int device, SabUse* u) {
+    u->c = sab_get_context(device);
+    if (!u->c) return SAB_ERR_CUDA;
+    u->lk = std::unique_lock<std::mutex>(u->c->mu);
+    SAB_CUDA_TRY(cudaSetDevice(u->c->device));
+    return SAB_OK;
+}
+
+// n <= 256 device words into out[] through the pinned staging, with one stream synchronisation
+static inline int sab_read_u32(SabContext* c, const u32* d_src, int n, u32* out) {
+    SAB_CUDA_TRY(cudaMemcpyAsync(c->staging->read, d_src, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    memcpy(out, c->staging->read, (size_t)n * sizeof(u32));
+    return SAB_OK;
+}
+
 cudaEvent_t sab_event_get(SabContext* c);
 int sab_copy_h2d(SabContext* c, void* d_dst, const void* h_src, size_t bytes);
 int sab_copy_d2h(SabContext* c, void* h_dst, const void* d_src, size_t bytes);
-void sab_prof_begin(SabContext* c, int kind);
+void sab_prof_begin(SabContext* c, SabProfKind kind);
 void sab_prof_end(SabContext* c);
 void sab_prof_collect(SabContext* c);
 

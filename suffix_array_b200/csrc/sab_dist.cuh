@@ -499,12 +499,11 @@ struct DistRun {
     // ---- 1. common alphabet / key shape: the byte histograms of all shards add up
     int alphabet() {
         ph.mark(PH_ALPHABET);
-        u32* d_h32 = c->d_counters + 16;
-        SAB_TRY(sab_launch_alphabet_hist(c, d_text, count, d_h32));
-        SAB_LAUNCH(hist_widen_kernel, 1, 256, 0, st, (const u32*)d_h32, c->d_ghist);
+        SAB_TRY(sab_launch_alphabet_hist(c, d_text, count, c->scratch->hist));
+        SAB_LAUNCH(hist_widen_kernel, 1, 256, 0, st, (const u32*)c->scratch->hist, c->d_ghist);
         SAB_LAUNCH_CHECK();
         SAB_TRY(sab_comm_all_reduce_u64(cm, st, c->d_ghist, 256));
-        u64* h64 = (u64*)(c->h_small + 1024);
+        u64* h64 = c->staging->wide;
         SAB_CUDA_TRY(cudaMemcpyAsync(h64, c->d_ghist, 256 * sizeof(u64), cudaMemcpyDeviceToHost, st));
         SAB_CUDA_TRY(cudaStreamSynchronize(st));
         return sab_plan_alphabet(c, h64, n, &al);
@@ -516,7 +515,7 @@ struct DistRun {
         u64* keysA = A.top<u64>(count + 8);
         SAB_ARENA_CHECK(A);
         if (count) {
-            sab_prof_begin(c, 2);
+            sab_prof_begin(c, SAB_PROF_PACK);
             SAB_TRY(sab_launch_pack(c, d_text, sh.len, count, al.d_lut, al.base, al.k, keysA));
             sab_prof_end(c);
         }
@@ -594,7 +593,7 @@ struct DistRun {
             // stores, and the all_reduce below orders the stores before the local sort.
             PeerOut po;
             memset(&po, 0, sizeof(po));
-            u64* h = (u64*)(c->h_small + 1024);
+            u64* h = c->staging->wide;
             for (int i = 0; i < 256; ++i) h[i] = 0;
             for (int d = 0; d < P; ++d) {
                 u64 Rd = 0, before = 0;
@@ -728,7 +727,7 @@ struct DistRun {
         const u64 rebal_min = (u64)sab_env_int("SAB_REBALANCE_MIN", 1 << 20);
         if (M < rebal_min * (u64)P || (double)mx * P <= 1.1 * (double)M) return SAB_OK;
         const u64 Q = div_up64(M, (u64)P);
-        u64* h = (u64*)(c->h_small + 1024);
+        u64 *h_cuts = c->staging->wide, *h_found = c->staging->wide + SAB_MAX_RANKS;  // as d_cuts, d_found below
         u64 cuts[SAB_MAX_RANKS], found[SAB_MAX_RANKS];
         for (int j = 1; j < P; ++j) {
             const u64 want = (u64)j * Q;
@@ -737,8 +736,8 @@ struct DistRun {
         }
         u64* d_cuts = c->d_ghist;  // [P-1] cuts, then [P-1] results
         unsigned long long* d_found = (unsigned long long*)(c->d_ghist + SAB_MAX_RANKS);
-        memcpy(h, cuts, sizeof(u64) * (P - 1));
-        SAB_CUDA_TRY(cudaMemcpyAsync(d_cuts, h, sizeof(u64) * (P - 1), cudaMemcpyHostToDevice, st));
+        memcpy(h_cuts, cuts, sizeof(u64) * (P - 1));
+        SAB_CUDA_TRY(cudaMemcpyAsync(d_cuts, h_cuts, sizeof(u64) * (P - 1), cudaMemcpyHostToDevice, st));
         u64 woff = 0, window = 1 << 16;
         for (;;) {
             bool open = false;
@@ -749,11 +748,11 @@ struct DistRun {
             SAB_LAUNCH(find_boundary_kernel, bpc * (unsigned)(P - 1), 256, 0, st, (const u32*)r1buf, m, (const u64*)d_cuts, bpc, woff,
                        window, d_found);
             SAB_LAUNCH_CHECK();
-            SAB_CUDA_TRY(cudaMemcpyAsync(h + 32, d_found, sizeof(u64) * (P - 1), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaMemcpyAsync(h_found, d_found, sizeof(u64) * (P - 1), cudaMemcpyDeviceToHost, st));
             SAB_CUDA_TRY(cudaStreamSynchronize(st));
             for (int j = 0; j < P - 1; ++j) {
                 if (found[j] != ~0ull) continue;
-                if (h[32 + j] != ~0ull) found[j] = h[32 + j];
+                if (h_found[j] != ~0ull) found[j] = h_found[j];
                 else if (cuts[j] + woff + window >= m) found[j] = m;  // the group runs to the end of the list
             }
             woff += window;
@@ -828,7 +827,7 @@ struct DistRun {
             lead_barrier = false;
         }
         if (m) {
-            sab_prof_begin(c, 4);
+            sab_prof_begin(c, SAB_PROF_GATHER);
             SAB_LAUNCH(dist_gather_p2p_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u32*)r1buf, (const u32*)rb.v[rb.cur], m,
                        (u32)h, lay, pt, lazy ? 1 : 0, al.d_lut, al.base, al.k, dir_shift, sdop, rb.k[rb.cur]);
             sab_prof_end(c);
@@ -861,7 +860,7 @@ struct DistRun {
         SAB_ARENA_CHECK(A);
         SAB_TRY(sab_comm_exchange(cm, st, pr, ipart, q, sizeof(u32)));
         if (nq) {
-            sab_prof_begin(c, 4);
+            sab_prof_begin(c, SAB_PROF_GATHER);
             SAB_LAUNCH(dist_gather_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, (const u32*)q, nq, (u32)h, (u32)sh.lo, lay,
                        (const u32*)rank_local, ans);
             sab_prof_end(c);
@@ -875,7 +874,7 @@ struct DistRun {
             u64* keys_u = A.top<u64>(nq + 8);
             u32* slot_u = A.top<u32>(nq + 8);
             SAB_ARENA_CHECK(A);
-            u32* d_nu = c->d_counters + 12;
+            u32* d_nu = &c->scratch->nu;
             SAB_CUDA_TRY(cudaMemsetAsync(d_nu, 0, sizeof(u32), st));
             if (nq) {
                 SAB_LAUNCH(dist_lazy_collect_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, q, (const u32*)ans, nq, (u32)h, sh.lo, d_text,
@@ -938,7 +937,7 @@ struct DistRun {
         sorted_idx = nullptr;
         sorted_in = 0;
         SAB_ARENA_CHECK(A);
-        SAB_CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, sizeof(u32), st));  // kept = 0 unless the re-rank says otherwise
+        SAB_CUDA_TRY(cudaMemsetAsync(&c->scratch->count, 0, sizeof(u32), st));  // kept = 0 unless the re-rank says otherwise
         if (m == 0) return SAB_OK;
         const int rank_bits = sab_ceil_log2_u64(n + 2);
         SortBuffers<u64> sb;
@@ -1001,7 +1000,7 @@ struct DistRun {
     // over all ranks).  The survivors here become the next list.
     int rank_updates(bool p2p_round) {
         u64 kept = 0;
-        u32* d_m = c->d_counters;
+        u32* d_m = &c->scratch->count;
         ph.mark(PH_RANK_UPDATES);
         if (p2p_round) {
             // all_reduce #1: the survivors add up (termination) and every rank has finished LOADING ranks;
@@ -1016,10 +1015,10 @@ struct DistRun {
             }
             SAB_TRY(sab_comm_all_reduce_u64(cm, st, cm->d_small + 8, 1));
             SAB_CUDA_TRY(cudaMemcpyAsync(cm->h_small, cm->d_small, sizeof(u64), cudaMemcpyDeviceToHost, st));
-            SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            SAB_CUDA_TRY(cudaStreamSynchronize(st));
+            u32 survivors;
+            SAB_TRY(sab_read_u32(c, d_m, 1, &survivors));  // its synchronisation also lands the total
             tot = cm->h_small[0];
-            kept = c->h_small[0];
+            kept = survivors;
             ds->p2p_rounds++;
         } else {
             u64 rows_k[SAB_MAX_RANKS * 32];
@@ -1213,10 +1212,9 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
         return SAB_ERR_ARGS;
     }
     const double w0 = now_ms();
-    SabContext* c = sab_get_context(cm->device);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
+    SabUse u;
+    SAB_TRY(sab_use(cm->device, &u));
+    SabContext* c = u.c;
     memset(&c->stats, 0, sizeof(c->stats));
     c->profiling = g_profiling;
     sab200_dist_stats& ds = cm->last;
@@ -1265,9 +1263,7 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
     c->want_bkt = nullptr;
     c->bkt_add_one = 1;
     if (rc != SAB_OK) {
-        cudaMemsetAsync(c->d_ticket, 0, sizeof(u32) * 4, st);  // a failed launch may have left the ticket out of step
-        cudaStreamSynchronize(st);
-        c->ticket_host = 0;
+        sab_reset_after_failure(c);
         return rc;
     }
     if (slice_len) *slice_len = res.slice_len;
@@ -1277,10 +1273,7 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
     if (h_bkt_part) SAB_CUDA_TRY(cudaMemcpyAsync(h_bkt_part, d_bkt, (size_t)SAB200_BKT_LEN * sizeof(u32), cudaMemcpyDeviceToHost, st));
     if (host_out_base) {
         if (res.slice_len) SAB_TRY(sab_copy_d2h(c, host_out_base + res.sa_off, res.d_slice, res.slice_len * sizeof(u32)));
-        if (cm->rank == 0) {
-            c->h_small[32] = (u32)n;
-            memcpy(host_out_base, c->h_small + 32, sizeof(u32));  // sa[0] = n (src/saca.rs:13)
-        }
+        if (cm->rank == 0) host_out_base[0] = (u32)n;  // src/saca.rs:13
     } else if (out) {
         if (out_cap < res.slice_len) {
             sab_set_error("sab200_saca_sharded: the slice has %llu entries, the buffer holds %llu", (unsigned long long)res.slice_len,
@@ -1315,11 +1308,9 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
 
 extern "C" int32_t sab200_sort_pairs_device(uint64_t* d_k0, uint64_t* d_k1, uint32_t* d_v0, uint32_t* d_v1, uint64_t count,
                                             int32_t key_bits, int32_t device) {
-    SabContext* c = sab_get_context(device);
-    if (!c) return SAB_ERR_CUDA;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
     if (key_bits < 0 || key_bits > 64) return SAB_ERR_ARGS;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
     SortBuffers<u64> buf;
     buf.k[0] = d_k0;
     buf.k[1] = d_k1;
@@ -1327,30 +1318,22 @@ extern "C" int32_t sab200_sort_pairs_device(uint64_t* d_k0, uint64_t* d_k1, uint
     buf.v[1] = d_v1;
     buf.cur = 0;
     u32 passes = 0;
-    const int rc = sab_radix_sort<u64>(c, buf, count, 0, key_bits, false, &passes);
+    const int rc = sab_radix_sort<u64>(u.c, buf, count, 0, key_bits, false, &passes);
     if (rc != SAB_OK) return rc;
-    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(u.c->stream));
     return buf.cur;
 }
 
 extern "C" int32_t sab200_group_sort_device(uint64_t* d_k0, uint64_t* d_k1, uint32_t* d_v0, uint32_t* d_v1, uint64_t count,
                                             int32_t key_bits, int32_t ascending, int32_t device, uint64_t* nbig_out) {
-    SabContext* c = sab_get_context(device);
-    if (!c) return SAB_ERR_CUDA;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
     if (key_bits < 32 || key_bits > 64 || count > 0xfffffff0ull) return SAB_ERR_ARGS;
     if (nbig_out) *nbig_out = 0;
     if (count == 0) return 0;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
     const u64 cap = sab_align_up((size_t)count * 2 + 64, 64);  // room for every record, and for the position sort
-    SAB_TRY(sab_arena_reserve(c, (size_t)cap * (2 * 8 + 3 * 4) + 8 * 256));
-    c->arena_used = 0;
     GroupSortSpare sp;
-    sp.k[0] = sab_arena_take<u64>(c, cap);
-    sp.k[1] = sab_arena_take<u64>(c, cap);
-    sp.v[0] = sab_arena_take<u32>(c, cap);
-    sp.v[1] = sab_arena_take<u32>(c, cap);
-    sp.pos = sab_arena_take<u32>(c, cap);
+    SAB_TRY(sab_arena_carve(u.c, {{&sp.k[0], cap * 8}, {&sp.k[1], cap * 8}, {&sp.v[0], cap * 4}, {&sp.v[1], cap * 4}, {&sp.pos, cap * 4}}));
     sp.cap = cap;
     SortBuffers<u64> sb;
     sb.k[0] = d_k0;
@@ -1360,25 +1343,23 @@ extern "C" int32_t sab200_group_sort_device(uint64_t* d_k0, uint64_t* d_k1, uint
     sb.cur = 0;
     u32 passes = 0;
     u64 nbig = 0;
-    const int rc = sab_group_sort(c, sb, count, key_bits, sp, &passes, &nbig, ascending != 0);
+    const int rc = sab_group_sort(u.c, sb, count, key_bits, sp, &passes, &nbig, ascending != 0);
     if (rc < 0) return rc;
     if (rc == 0) {
         sab_set_error("group sort: the records of large groups did not fit the spare buffers");
         return SAB_ERR_INTERNAL;
     }
-    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(u.c->stream));
     if (nbig_out) *nbig_out = nbig;
     return sb.cur;
 }
 
 extern "C" int32_t sab200_copy_from_device(void* dst, const void* d_src, uint64_t bytes, int32_t device) {
     if (!dst || !d_src) return bytes ? SAB_ERR_ARGS : SAB_OK;
-    SabContext* c = sab_get_context(device);
-    if (!c) return SAB_ERR_CUDA;
-    std::lock_guard<std::mutex> lk(c->mu);
-    SAB_CUDA_TRY(cudaSetDevice(c->device));
-    SAB_CUDA_TRY(cudaMemcpyAsync(dst, d_src, bytes, cudaMemcpyDeviceToHost, c->stream));
-    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    SAB_CUDA_TRY(cudaMemcpyAsync(dst, d_src, bytes, cudaMemcpyDeviceToHost, u.c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(u.c->stream));
     return SAB_OK;
 }
 

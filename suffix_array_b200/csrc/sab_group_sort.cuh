@@ -376,20 +376,18 @@ static int sab_group_sort(SabContext* c, SortBuffers<u64>& sb, u64 cnt, int key_
     const u64 tiles = div_up64(cnt, SAB_GSORT_TILE);
     SAB_TRY(sab_ensure_scan(c, (size_t)tiles));
     TileState<u32> ts = sab_tile_state<u32>(c, tiles);
-    u32* d_nbig = c->d_counters + 10;
     const u32 cap = sp.cap > 0xffffffffull ? 0xffffffffu : (u32)sp.cap;
 #ifndef SAB_EMU
     SAB_CUDA_TRY(cudaFuncSetAttribute(group_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SAB_GSORT_SMEM));
 #endif
-    sab_prof_begin(c, 5);
+    sab_prof_begin(c, SAB_PROF_GROUP_SORT);
     SAB_LAUNCH(group_sort_kernel, (unsigned)tiles, SAB_GSORT_THREADS, SAB_GSORT_SMEM, c->stream, (const u64*)sb.k[0],
-               (const u32*)sb.v[0], cnt, sb.k[1], sb.v[1], sp.k[0], sp.v[0], sp.pos, cap, d_nbig, ts);
+               (const u32*)sb.v[0], cnt, sb.k[1], sb.v[1], sp.k[0], sp.v[0], sp.pos, cap, &c->scratch->big, ts);
     sab_prof_end(c);
     SAB_LAUNCH_CHECK();
     c->stats.kernel_launches++;
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small + 10, d_nbig, sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
-    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
-    const u64 nbig = c->h_small[10];
+    u32 nbig;
+    SAB_TRY(sab_read_u32(c, &c->scratch->big, 1, &nbig));
     c->stats.group_sort_records += cnt;
     c->stats.group_big_records += nbig;
     *nbig_out = nbig;
@@ -420,7 +418,7 @@ static int sab_group_sort(SabContext* c, SortBuffers<u64>& sb, u64 cnt, int key_
             SAB_TRY(sab_radix_sort<u64>(c, pb, nbig, 32, key_bits, /*iota=*/false, &pos_passes));
             sorted_pos = pb.v[pb.cur];
         }
-        sab_prof_begin(c, 5);
+        sab_prof_begin(c, SAB_PROF_GROUP_SORT);
         SAB_LAUNCH(scatter_back_kernel, (unsigned)div_up64(nbig, 256), 256, 0, c->stream, (const u64*)bb.k[bb.cur],
                    (const u32*)bb.v[bb.cur], sorted_pos, (u32)nbig, sb.k[1], sb.v[1]);
         sab_prof_end(c);

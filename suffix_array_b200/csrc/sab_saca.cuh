@@ -409,7 +409,7 @@ struct SabAlphabet {
 // probability ~ n * 2^-(k*H2) (H2 = order-0 collision entropy; higher-order structure only makes the
 // estimate optimistic, never the result wrong).
 static int sab_plan_alphabet(SabContext* c, const u64* hist, u64 n, SabAlphabet* a) {
-    u16 lut[256];
+    u16* lut = c->staging->lut;  // pinned: the upload at the end is asynchronous
     u32 sigma = 0;
     double sum_p2 = 0.0;
     for (int ch = 0; ch < 256; ++ch) {
@@ -470,21 +470,18 @@ static int sab_plan_alphabet(SabContext* c, const u64* hist, u64 n, SabAlphabet*
     c->stats.sigma = sigma;
     c->stats.bits_per_symbol = (u32)sab_ceil_log2_u64(base);
     c->stats.symbols_per_key = (u32)k;
-    u16* d_lut = (u16*)(c->d_counters + 16 + 256);
-    memcpy(c->h_small + 384, lut, sizeof(lut));  // pinned staging: the async copy must not read the stack later
-    SAB_CUDA_TRY(cudaMemcpyAsync(d_lut, c->h_small + 384, sizeof(lut), cudaMemcpyHostToDevice, c->stream));
-    a->d_lut = d_lut;
+    SAB_CUDA_TRY(cudaMemcpyAsync(c->scratch->lut, lut, sizeof(c->staging->lut), cudaMemcpyHostToDevice, c->stream));
+    a->d_lut = c->scratch->lut;
     return SAB_OK;
 }
 
 // The alphabet of a text of n > 0 bytes resident on this GPU.
 static int sab_alphabet_local(SabContext* c, const u8* d_text, u64 n, SabAlphabet* a) {
-    u32* d_hist = c->d_counters + 16;  // 256 words inside the counters block
-    SAB_TRY(sab_launch_alphabet_hist(c, d_text, n, d_hist));
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small + 64, d_hist, 256 * sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
-    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    SAB_TRY(sab_launch_alphabet_hist(c, d_text, n, c->scratch->hist));
+    u32 h32[256];
+    SAB_TRY(sab_read_u32(c, c->scratch->hist, 256, h32));
     u64 hist[256];
-    for (int ch = 0; ch < 256; ++ch) hist[ch] = c->h_small[64 + ch];
+    for (int ch = 0; ch < 256; ++ch) hist[ch] = h32[ch];
     return sab_plan_alphabet(c, hist, n, a);
 }
 
@@ -579,26 +576,26 @@ static int sab_init_ranks(SabContext* c, const u64* sortedK, const u32* sortedI,
                           u32* sa_out, u32* act_r1, u32* act_idx, u32* dir, int dir_shift, u64* m) {
     const u64 tiles = div_up64(cnt, SAB_SCAN_TILE);
     TileState<RankScan> ts = sab_tile_state<RankScan>(c, tiles);
-    sab_prof_begin(c, 3);
+    sab_prof_begin(c, SAB_PROF_RANK);
     SAB_LAUNCH(init_ranks_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, c->stream, sortedK, sortedI, cnt, rank_base, rank, rank_seq,
-               sa_out, act_r1, act_idx, c->d_counters, dir, dir_shift, ts);
+               sa_out, act_r1, act_idx, &c->scratch->count, dir, dir_shift, ts);
     sab_prof_end(c);
     SAB_LAUNCH_CHECK();
     c->stats.kernel_launches++;
-    SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, c->d_counters, sizeof(u32), cudaMemcpyDeviceToHost, c->stream));
-    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
-    *m = c->h_small[0];
+    u32 active;
+    SAB_TRY(sab_read_u32(c, &c->scratch->count, 1, &active));
+    *m = active;
     return SAB_OK;
 }
 
-// re-rank (5) of the cnt sorted records of a round; the number of survivors is left in c->d_counters[0]
+// re-rank (5) of the cnt sorted records of a round; the number of survivors is left in c->scratch->count
 static int sab_launch_rerank(SabContext* c, const SortBuffers<u64>& sb, u64 cnt, u32* rank, u32* sa, u32* out_r1, u32* out_idx,
                              u32* upd_idx, u32* upd_r, u32* set_pos) {
     const u64 tiles = div_up64(cnt, SAB_SCAN_TILE);
     TileState<RerankScan> ts = sab_tile_state<RerankScan>(c, tiles);
-    sab_prof_begin(c, 3);
+    sab_prof_begin(c, SAB_PROF_RANK);
     SAB_LAUNCH(rerank_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, c->stream, (const u64*)sb.k[sb.cur], (const u32*)sb.v[sb.cur], cnt,
-               rank, sa, out_r1, out_idx, upd_idx, upd_r, set_pos, c->d_counters, ts);
+               rank, sa, out_r1, out_idx, upd_idx, upd_r, set_pos, &c->scratch->count, ts);
     sab_prof_end(c);
     SAB_LAUNCH_CHECK();
     c->stats.kernel_launches++;
@@ -639,7 +636,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     SAB_TRY(sab_ensure_scan(c, (size_t)div_up64(n, SAB_SCAN_TILE)));
 
     // 1. alphabet
-    sab_prof_begin(c, 2);
+    sab_prof_begin(c, SAB_PROF_PACK);
     SabAlphabet al;
     SAB_TRY(sab_alphabet_local(c, d_text, n, &al));
 
@@ -653,7 +650,6 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     SAB_TRY(sab_radix_sort<u64>(c, buf, n, 0, al.key_bits, /*iota=*/true, &S.passes[0], d_sa + 1, &sa_written));
 
     // 4. ranks, SA skeleton, active list, bucket directory over the sorted keys
-    u32* d_m = c->d_counters;
     const u64* sortedK = buf.k[buf.cur];
     if (c->want_bkt) SAB_TRY(sab_fused_buckets(c, d_text, n, sortedK, n, al));
     const u32* sortedI = sa_written ? d_sa + 1 : buf.v[buf.cur];
@@ -664,8 +660,8 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     u32* split_bitmap = sab_arena_take<u32>(c, (size_t)n / 32 + 8);
     SAB_CUDA_TRY(cudaMemsetAsync(rank, 0xff, n * sizeof(u32), st));
     SAB_CUDA_TRY(cudaMemsetAsync(rank + n, 0, sizeof(u32), st));  // the empty suffix has rank 0
-    c->h_small[32] = (u32)n;
-    SAB_CUDA_TRY(cudaMemcpyAsync(d_sa, c->h_small + 32, sizeof(u32), cudaMemcpyHostToDevice, st));  // sa[0] = n
+    c->staging->sa0 = (u32)n;
+    SAB_CUDA_TRY(cudaMemcpyAsync(d_sa, &c->staging->sa0, sizeof(u32), cudaMemcpyHostToDevice, st));  // sa[0] = n
     u64 m = 0;
     SAB_TRY(sab_init_ranks(c, sortedK, sortedI, n, 1u, rank, nullptr, sa_written ? nullptr : d_sa + 1, r1buf, act_idx, dir, dir_shift, &m));
     S.active[0] = m;
@@ -685,7 +681,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     z.dir_shift = dir_shift;
     z.sorted_keys = m <= n / 4 ? sortedK : nullptr;  // keep the sorted keys
     if (!z.sorted_keys) {
-        sab_prof_begin(c, 3);
+        sab_prof_begin(c, SAB_PROF_RANK);
         SAB_LAUNCH(fill_settled_ranks_kernel, (unsigned)div_up64(n, 256), 256, 0, st, sortedK, sortedI, n, rank);
         sab_prof_end(c);
         SAB_LAUNCH_CHECK();
@@ -714,7 +710,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
                           (unsigned long long)m);
             return SAB_ERR_INTERNAL;
         }
-        sab_prof_begin(c, 4);
+        sab_prof_begin(c, SAB_PROF_GATHER);
         SAB_LAUNCH(gather_rank2_kernel, (unsigned)div_up64(m, (u64)SAB_GATHER_THREADS * SAB_GATHER_ITEMS), SAB_GATHER_THREADS,
                    0, st, (const u32*)r1buf, (const u32*)rb.v[rb.cur], m, h, rank, z, rb.k[rb.cur]);
         sab_prof_end(c);
@@ -724,22 +720,22 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
         if (filter_on && m >= SAB_FILTER_MIN) {
             const u64 tiles = div_up64(m, SAB_SCAN_TILE);
             TileState<FilterScan> ts = sab_tile_state<FilterScan>(c, tiles);
-            sab_prof_begin(c, 3);
+            sab_prof_begin(c, SAB_PROF_RANK);
             SAB_CUDA_TRY(cudaMemsetAsync(split_bitmap, 0, ((size_t)n / 32 + 8) * sizeof(u32), st));
             SAB_LAUNCH(mark_split_groups_kernel, (unsigned)div_up64(m, 256), 256, 0, st, (const u64*)rb.k[rb.cur], m, split_bitmap);
             SAB_LAUNCH_CHECK();
             SAB_LAUNCH(split_filter_kernel, (unsigned)tiles, SAB_SCAN_THREADS, 0, st, rb.k[rb.cur], rb.v[rb.cur], m,
-                       (const u32*)split_bitmap, r1buf, rb.v[rb.cur ^ 1], d_m + 2, ts);
+                       (const u32*)split_bitmap, r1buf, rb.v[rb.cur ^ 1], c->scratch->filter, ts);
             sab_prof_end(c);
             SAB_LAUNCH_CHECK();
             S.kernel_launches += 2;
-            SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m + 2, 2 * sizeof(u32), cudaMemcpyDeviceToHost, st));
-            SAB_CUDA_TRY(cudaStreamSynchronize(st));
-            n_sort = c->h_small[0];
-            n_stay = c->h_small[1];
+            u32 split[2];
+            SAB_TRY(sab_read_u32(c, c->scratch->filter, 2, split));
+            n_sort = split[0];
+            n_stay = split[1];
             if (n_sort * 10 > m * 7) filter_on = false;  // from here on most groups split every round
         }
-        u64 kept = 0;
+        u32 kept = 0;
         bool order_restored = false;  // the round's records went through the full radix sort: ascending in r1 again
         if (n_sort > 0) {
             // sort the n_sort records at the front of (k[cur], v[cur]); the spare payload buffer starts
@@ -774,9 +770,7 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
             }
             u32* out_idx = (sb.cur == 0) ? rb.v[rb.cur ^ 1] + n_stay : rb.v[rb.cur];
             SAB_TRY(sab_launch_rerank(c, sb, n_sort, rank, d_sa, r1buf + n_stay, out_idx, nullptr, nullptr, nullptr));
-            SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, d_m, sizeof(u32), cudaMemcpyDeviceToHost, st));
-            SAB_CUDA_TRY(cudaStreamSynchronize(st));
-            kept = c->h_small[0];
+            SAB_TRY(sab_read_u32(c, &c->scratch->count, 1, &kept));
             if (sb.cur != 0 && kept > 0)  // the survivors were written to the other buffer: append them to the parked ones
                 SAB_CUDA_TRY(cudaMemcpyAsync(rb.v[rb.cur ^ 1] + n_stay, rb.v[rb.cur], kept * sizeof(u32), cudaMemcpyDeviceToDevice, st));
         }

@@ -49,7 +49,7 @@ static int sab_launch_pass_op(SabContext* c, const KeyT* kin, KeyT* kout, const 
 #ifndef SAB_EMU
     SAB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));  // per device
 #endif
-    sab_prof_begin(c, 0);
+    sab_prof_begin(c, SAB_PROF_RADIX_PASS);
     SAB_LAUNCH(kern, (unsigned)tiles, THREADS, Cfg::SMEM, c->stream, kin, kout, vin, vout, n, dop, gbase,
                c->d_lookback, c->d_ticket, c->ticket_host, epoch, po, iota_base);
     sab_prof_end(c);
@@ -98,19 +98,17 @@ static int sab_radix_sort(SabContext* c, SortBuffers<KeyT>& buf, u64 n, int begi
         u64 hblocks = div_up64(n, htile);
         const u64 hmax = (u64)c->sm_count * 4;
         if (hblocks > hmax) hblocks = hmax;
-        sab_prof_begin(c, 1);
+        sab_prof_begin(c, SAB_PROF_HIST);
         SAB_LAUNCH(radix_hist_kernel<KeyT>, (unsigned)hblocks, SAB_HIST_THREADS, 0, c->stream, (const KeyT*)buf.k[buf.cur], n,
                    begin_bit, npass, c->d_ghist);
         SAB_LAUNCH_CHECK();
         SAB_LAUNCH(radix_scan_kernel, 1, SAB_RADIX_BINS, 0, c->stream, (const u64*)c->d_ghist, n, npass, c->d_gbase,
-                   c->d_skip);
+                   c->scratch->skip);
         sab_prof_end(c);
         SAB_LAUNCH_CHECK();
         c->stats.kernel_launches += 2;
-        SAB_CUDA_TRY(cudaMemcpyAsync(c->h_small, c->d_skip, sizeof(u32) * SAB_MAX_PASSES, cudaMemcpyDeviceToHost, c->stream));
-        SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
         u32 skip[SAB_MAX_PASSES];
-        memcpy(skip, c->h_small, sizeof(skip));
+        SAB_TRY(sab_read_u32(c, c->scratch->skip, SAB_MAX_PASSES, skip));
         int last = -1;
         for (int p = 0; p < npass; ++p)
             if (!skip[p]) last = p;
