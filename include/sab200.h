@@ -107,6 +107,27 @@ int32_t sab200_check(const uint8_t* s, uint64_t n, const uint32_t* sa, uint64_t 
  * first position of a chunk compares from scratch, the others extend the previous length minus one. */
 int32_t sab200_lcp_array(const uint8_t* s, uint64_t n, const uint32_t* sa, uint64_t sa_len, uint32_t* lcp);
 
+/* ---- Burrows-Wheeler transform ----------------------------------------------------------------
+ * libdivsufsort's divbwt / inverse_bw_transform, which the reference does not expose.  Over the n+1 rows of the
+ * suffix array sab200_saca builds (sa[0] = n): the last column is L[j] = s[sa[j]-1] where sa[j] > 0, and L[p] = '$' at
+ * the single row p with sa[p] = 0, the PRIMARY INDEX (1 <= p <= n for n >= 1).  The transform is L without row p:
+ * n bytes, bwt[0] = s[n-1].  The empty text gives an empty transform and p = 0.  Example: "banana" -> ("annbaa", 4).
+ * This is the layout libdivsufsort documents for divbwt; libdivsufsort is not in the tree, so byte parity with it is
+ * pinned only by this definition (like the pack bytes above).
+ *
+ * sab200_bwt builds the suffix array on the GPU as sab200_saca does (its statistics stay readable through
+ * sab200_get_stats), gathers L there, and moves only the n bytes of the transform back.  It takes no device memory
+ * beyond what sab200_saca takes.
+ * sab200_inverse_bwt returns the text of (bwt, primary).  A primary outside [1, n] (outside {0} when n = 0), or a bwt
+ * that is the transform of no text, returns SAB200_ERR_ARGS with sab200_last_error saying which; `s` is then left
+ * unwritten.  Device memory: about 25 bytes per byte of text.
+ * Host buffers, pageable or pinned; one GPU. */
+int32_t sab200_bwt(const uint8_t* s, uint64_t n, uint8_t* bwt, uint64_t* primary);
+int32_t sab200_inverse_bwt(const uint8_t* bwt, uint64_t n, uint64_t primary, uint8_t* s);
+/* The same with DEVICE buffers already resident on `device` (n bytes each), to time the device work without PCIe. */
+int32_t sab200_bwt_device(const uint8_t* d_s, uint64_t n, uint8_t* d_bwt, uint64_t* primary, int32_t device);
+int32_t sab200_inverse_bwt_device(const uint8_t* d_bwt, uint64_t n, uint64_t primary, uint8_t* d_s, int32_t device);
+
 /* ---- batched queries -----------------------------------------------------------------------
  * A resident copy of (text, SA, optional bucket table) on `ngpus` GPUs (replicated; queries are
  * sharded across the replicas, no collective).  bkt_or_null = NULL means "buckets not enabled"

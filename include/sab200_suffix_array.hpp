@@ -46,6 +46,26 @@ inline void saca(const std::uint8_t* s, std::size_t n, std::vector<std::uint32_t
     check(sab200_saca(s, n, sa.data(), ngpus), "sab200_saca");
 }
 
+// Burrows-Wheeler transform (sab200.h): the n bytes of the last column without the row of '$', and that row's index
+// (the primary index).  bwt("banana") = ("annbaa", 4).
+inline std::pair<std::vector<std::uint8_t>, std::uint64_t> bwt(const std::uint8_t* s, std::size_t n) {
+    if (n > MAX_LENGTH) throw std::length_error("text longer than MAX_LENGTH");
+    std::pair<std::vector<std::uint8_t>, std::uint64_t> r(std::vector<std::uint8_t>(n), 0);
+    check(sab200_bwt(s, n, r.first.data(), &r.second), "sab200_bwt");
+    return r;
+}
+
+// The text whose transform is (u, primary); std::invalid_argument when there is none or the primary index is out of
+// range.
+inline std::vector<std::uint8_t> inverse_bwt(const std::uint8_t* u, std::size_t n, std::uint64_t primary) {
+    if (n > MAX_LENGTH) throw std::length_error("transform longer than MAX_LENGTH");
+    std::vector<std::uint8_t> s(n);
+    const std::int32_t rc = sab200_inverse_bwt(u, n, primary, s.data());
+    if (rc == SAB200_ERR_ARGS) throw std::invalid_argument(std::string("sab200_inverse_bwt: ") + sab200_last_error());
+    check(rc, "sab200_inverse_bwt");
+    return s;
+}
+
 class SuffixArray {
   public:
     // src/sa.rs:23-27

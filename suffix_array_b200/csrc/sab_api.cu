@@ -6,6 +6,7 @@
 #include "sab_saca.cuh"
 #include "sab_search.cuh"
 #include "sab_pack.cuh"
+#include "sab_bwt.cuh"
 
 #include <chrono>
 #include <cstdlib>
@@ -491,6 +492,95 @@ extern "C" int32_t sab200_lcp_array(const uint8_t* s, uint64_t n, const uint32_t
     SAB_CUDA_TRY(cudaMemcpyAsync(lcp, d_lcp, sa_len * sizeof(u32), cudaMemcpyDeviceToHost, st));
     SAB_CUDA_TRY(cudaStreamSynchronize(st));
     return SAB_OK;
+}
+
+// ---- Burrows-Wheeler transform --------------------------------------------------------------
+// The construction, then the last column L of its n+1 rows into d_L (n+1 bytes; the bottom of the construction
+// workspace is free for it once the construction is done).  The construction's statistics stay readable.
+static int bwt_forward(SabContext* c, const u8* d_s, u64 n, u32* d_sa, u8* d_L, u64* primary) {
+    const int rc = run_device(c, d_s, n, d_sa);
+    g_last_stats = c->stats;
+    SAB_TRY(rc);
+    return sab_bwt_gather(c, d_s, n, d_sa, d_L, primary);
+}
+
+static bool bwt_bad_args(const char* who, const void* in, uint64_t n, const void* out) {
+    if ((n > 0 && (!in || !out)) || n > SAB200_MAX_LENGTH) {
+        sab_set_error("%s: bad arguments (n=%llu)", who, (unsigned long long)n);
+        return true;
+    }
+    return false;
+}
+
+static bool bwt_bad_primary(const char* who, uint64_t n, uint64_t primary) {
+    if (n == 0 ? primary != 0 : (primary < 1 || primary > n)) {
+        sab_set_error("%s: primary index %llu outside [1, %llu] (0 for the empty text)", who, (unsigned long long)primary,
+                      (unsigned long long)n);
+        return true;
+    }
+    return false;
+}
+
+extern "C" int32_t sab200_bwt(const uint8_t* s, uint64_t n, uint8_t* bwt, uint64_t* primary) {
+    if (!primary || bwt_bad_args("sab200_bwt", s, n, bwt)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    SabContext* c = u.c;
+    u8 *d_L, *d_s;
+    u32* d_sa;
+    SAB_TRY(sab_arena_carve(c, {{&d_L, sab_saca_workspace_bytes(n)}, {&d_s, (size_t)n + 64}, {&d_sa, ((size_t)n + 1) * sizeof(u32)}}));
+    SAB_TRY(sab_copy_h2d(c, d_s, s, n));
+    u64 p;
+    SAB_TRY(bwt_forward(c, d_s, n, d_sa, d_L, &p));
+    SAB_TRY(sab_copy_d2h(c, bwt, d_L, p));  // U = L without row p: two pieces of L, no compaction
+    SAB_TRY(sab_copy_d2h(c, bwt + p, d_L + p + 1, n - p));
+    *primary = p;
+    return SAB_OK;
+}
+
+extern "C" int32_t sab200_bwt_device(const uint8_t* d_s, uint64_t n, uint8_t* d_bwt, uint64_t* primary, int32_t device) {
+    if (!primary || bwt_bad_args("sab200_bwt_device", d_s, n, d_bwt)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    SabContext* c = u.c;
+    u8* d_L;
+    u32* d_sa;
+    SAB_TRY(sab_arena_carve(c, {{&d_L, sab_saca_workspace_bytes(n)}, {&d_sa, ((size_t)n + 1) * sizeof(u32)}}));
+    u64 p;
+    SAB_TRY(bwt_forward(c, d_s, n, d_sa, d_L, &p));
+    if (p > 0) SAB_CUDA_TRY(cudaMemcpyAsync(d_bwt, d_L, p, cudaMemcpyDeviceToDevice, c->stream));
+    if (n > p) SAB_CUDA_TRY(cudaMemcpyAsync(d_bwt + p, d_L + p + 1, n - p, cudaMemcpyDeviceToDevice, c->stream));
+    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    *primary = p;
+    return SAB_OK;
+}
+
+static int inverse_bwt_run(SabContext* c, const u8* d_u, u64 n, u64 primary, u8* d_s) {
+    const int rc = sab_inverse_bwt_run(c, d_u, n, (u32)primary, d_s);
+    if (rc != SAB_OK) sab_reset_after_failure(c);
+    return rc;
+}
+
+extern "C" int32_t sab200_inverse_bwt(const uint8_t* bwt, uint64_t n, uint64_t primary, uint8_t* s) {
+    if (bwt_bad_args("sab200_inverse_bwt", bwt, n, s) || bwt_bad_primary("sab200_inverse_bwt", n, primary)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    if (n == 0) return SAB_OK;
+    SabContext* c = u.c;
+    u8* d_u;  // the transform in, the text out: U is dead once it has been widened into the sort records
+    SAB_TRY(sab_arena_carve(c, {{nullptr, sab_inverse_bwt_workspace_bytes(n)}, {&d_u, (size_t)n + 64}}));
+    SAB_TRY(sab_copy_h2d(c, d_u, bwt, n));
+    SAB_TRY(inverse_bwt_run(c, d_u, n, primary, d_u));
+    return sab_copy_d2h(c, s, d_u, n);
+}
+
+extern "C" int32_t sab200_inverse_bwt_device(const uint8_t* d_bwt, uint64_t n, uint64_t primary, uint8_t* d_s, int32_t device) {
+    if (bwt_bad_args("sab200_inverse_bwt_device", d_bwt, n, d_s) || bwt_bad_primary("sab200_inverse_bwt_device", n, primary))
+        return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    if (n == 0) return SAB_OK;
+    return inverse_bwt_run(u.c, d_bwt, n, primary, d_s);
 }
 
 // ---- resident index + batched queries ------------------------------------------------------

@@ -56,6 +56,7 @@ struct SabScratch {
     u32 skip[16];   // radix sort: 1 for each digit place where all keys agree (SAB_MAX_PASSES of them)
     u32 hist[256];  // byte histogram of a text
     u16 lut[256];   // code table of the running construction (sab_plan_alphabet)
+    u32 bwt[2];     // sab200_bwt: the primary index; sab200_inverse_bwt: sample rows, list position of row p
 };
 
 // Pinned host staging of a context: readbacks land here, and small uploads leave from here, not from the caller's stack.

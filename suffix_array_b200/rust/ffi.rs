@@ -22,6 +22,11 @@ extern "C" {
     pub fn sab200_pack_bound(sa_len: u64) -> u64;
     pub fn sab200_pack(sa: *const u32, sa_len: u64, out: *mut u8, out_cap: u64, out_len: *mut u64) -> i32;
     pub fn sab200_unpack(bytes: *const u8, nbytes: u64, sa: *mut u32, sa_cap: u64, sa_len: *mut u64) -> i32;
+    // Burrows-Wheeler transform (libdivsufsort's divbwt / inverse_bw_transform layout; include/sab200.h)
+    pub fn sab200_bwt(s: *const u8, n: u64, bwt: *mut u8, primary: *mut u64) -> i32;
+    pub fn sab200_inverse_bwt(bwt: *const u8, n: u64, primary: u64, s: *mut u8) -> i32;
+    pub fn sab200_bwt_device(d_s: *const u8, n: u64, d_bwt: *mut u8, primary: *mut u64, device: i32) -> i32;
+    pub fn sab200_inverse_bwt_device(d_bwt: *const u8, n: u64, primary: u64, d_s: *mut u8, device: i32) -> i32;
     pub fn sab200_device_count() -> i32;
     pub fn sab200_last_error() -> *const c_char;
     pub fn sab200_shutdown();

@@ -45,6 +45,35 @@ def saca(s, sa, ngpus=1):
     _lib.check(L.sab200_saca(_ptr(s), s.size, sa.ctypes.data_as(C.c_void_p), ngpus), "sab200_saca")
 
 
+def bwt(s):
+    """Burrows-Wheeler transform of `s` (include/sab200.h): -> (uint8 array of n bytes, primary index).  The last
+    column of the n+1 sorted rotations of s$ without the row of '$'; bwt(b"banana") gives (b"annbaa", 4).  The suffix
+    array is built and used on the GPU; only the n bytes come back."""
+    t = _as_text(s)
+    assert t.size <= MAX_LENGTH
+    out = np.empty(t.size, dtype=np.uint8)
+    p = C.c_uint64()
+    L = _lib.require_gpu()
+    _lib.check(L.sab200_bwt(_ptr(t), t.size, _ptr(out), C.byref(p)), "sab200_bwt")
+    return out, int(p.value)
+
+
+def inverse_bwt(u, primary):
+    """The text whose transform is (u, primary), as a uint8 array.  Raises ValueError when `primary` is outside
+    [1, n] (0 for the empty transform) or `u` is the transform of no text."""
+    t = _as_text(u)
+    primary = int(primary)
+    if t.size > MAX_LENGTH or not 0 <= primary < 2 ** 64:
+        raise ValueError("bad transform length or primary index")
+    out = np.empty(t.size, dtype=np.uint8)
+    L = _lib.require_gpu()
+    rc = L.sab200_inverse_bwt(_ptr(t), t.size, primary, _ptr(out))
+    if rc == -1:
+        raise ValueError(L.sab200_last_error().decode("utf-8", "replace"))
+    _lib.check(rc, "sab200_inverse_bwt")
+    return out
+
+
 class SuffixArray:
     """Suffix array for a byte string (src/sa.rs:14-19): text `s`, `sa` of n+1 u32, optional buckets."""
 
