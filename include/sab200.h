@@ -159,6 +159,29 @@ int32_t sab200_search_lcp_batch(sab200_index* ix, const uint8_t* pats, const uin
 int32_t sab200_search_all_batch_device(sab200_index* ix, const uint8_t* d_pats, const uint64_t* d_offs, uint64_t np,
                                        uint32_t* d_lo, uint32_t* d_hi);
 
+/* ---- matching statistics ---------------------------------------------------------------------
+ * No reference counterpart.  Queries are passed like patterns: query q is qs[offs[q] .. offs[q+1]) (nq+1 offsets,
+ * non-decreasing, else SAB200_ERR_ARGS; at most 2^31-1 queries).  For every byte position i of a query Q of m bytes
+ * (i local to the query):
+ *   len[i]          the largest l <= m - i such that Q[i .. i+l) is a substring of s (l = 0 allowed): a match never
+ *                   runs past the end of its own query.  If i + len[i] < m, Q[i .. i+len[i]+1) does not occur in s.
+ *   [lo[i], hi[i])  the GLOBAL suffix-array indices j in [0, n] whose suffix starts with Q[i .. i+len[i]): for
+ *                   len[i] >= 1 exactly what sab200_search_all_batch returns for that pattern (hi - lo occurrences at
+ *                   sa[lo .. hi)); [0, n+1) for len[i] = 0.
+ * The outputs are indexed by the absolute byte offset in qs: each holds offs[nq] entries (entries before offs[0] are
+ * not written).  With several replicas every replica receives the whole concatenation and walks an equal share of
+ * the positions.  Host buffers, pageable or pinned.
+ * The first call on an index extends it on every replica with the inverse suffix array, the LCP array and block
+ * minima over it: 8(n+2) + about n/64 bytes per replica, at the cost of one integrity check and one LCP build per
+ * replica.  A suffix array that is not the text's (reachable through unchecked_from_parts) returns SAB200_ERR_ARGS
+ * and keeps no extension; an extension that does not fit returns SAB200_ERR_OOM.  The index stays usable either way. */
+int32_t sab200_matching_statistics_batch(sab200_index* ix, const uint8_t* qs, const uint64_t* offs, uint64_t nq,
+                                         uint32_t* len, uint32_t* lo, uint32_t* hi);
+/* the same with DEVICE buffers on the GPU of replica 0 (kernel-only timing); d_qs is indexed by the absolute offsets
+ * and must be followed by at least 8 readable bytes */
+int32_t sab200_matching_statistics_batch_device(sab200_index* ix, const uint8_t* d_qs, const uint64_t* d_offs, uint64_t nq,
+                                                uint32_t* d_len, uint32_t* d_lo, uint32_t* d_hi);
+
 /* Introspection of a resident index (bench and tests).  sab200_index_create also builds a PREFIX DIRECTORY over the
  * resident text and suffix array (csrc/sab_search.cuh: number of suffixes below every code of `depth` leading symbols
  * in base `sigma`), from which search_all / contains start their bisection instead of from the whole two-byte

@@ -187,6 +187,24 @@ class SuffixArray {
         check(sab200_search_lcp_batch(index(), pats, offs, np, start, end), "sab200_search_lcp_batch");
     }
 
+    // ---- matching statistics (include/sab200.h): len / lo / hi receive offs[nq] entries each, indexed by the absolute
+    // offset in qs; a suffix array that is not the text's throws std::invalid_argument
+    void matching_statistics_batch(const std::uint8_t* qs, const std::uint64_t* offs, std::size_t nq, std::uint32_t* len,
+                                   std::uint32_t* lo, std::uint32_t* hi) {
+        const std::int32_t rc = sab200_matching_statistics_batch(index(), qs, offs, nq, len, lo, hi);
+        if (rc == SAB200_ERR_ARGS) throw std::invalid_argument(std::string("sab200_matching_statistics_batch: ") + sab200_last_error());
+        check(rc, "sab200_matching_statistics_batch");
+    }
+    struct MatchingStatistics {
+        std::vector<std::uint32_t> len, lo, hi;
+    };
+    MatchingStatistics matching_statistics(const std::uint8_t* q, std::size_t m) {
+        const std::uint64_t offs[2] = {0, m};
+        MatchingStatistics r{std::vector<std::uint32_t>(m), std::vector<std::uint32_t>(m), std::vector<std::uint32_t>(m)};
+        matching_statistics_batch(q, offs, 1, r.len.data(), r.lo.data(), r.hi.data());
+        return r;
+    }
+
     // ---- per-pattern queries (src/sa.rs:164-253)
     bool contains(const std::uint8_t* pat, std::size_t m) {
         const std::uint64_t offs[2] = {0, m};

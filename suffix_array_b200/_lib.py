@@ -138,6 +138,8 @@ def _bind(L):
         "sab200_contains_batch": ([vp, vp, vp, u64, vp], i32),
         "sab200_search_lcp_batch": ([vp, vp, vp, u64, vp, vp], i32),
         "sab200_search_all_batch_device": ([vp, vp, vp, u64, vp, vp], i32),
+        "sab200_matching_statistics_batch": ([vp, vp, vp, u64, vp, vp, vp], i32),
+        "sab200_matching_statistics_batch_device": ([vp, vp, vp, u64, vp, vp, vp], i32),
         "sab200_index_directory": ([vp, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)], u64),
         "sab200_index_probes": ([vp, i32], u64),
         "sab200_pack_bound": ([u64], u64),

@@ -5,6 +5,7 @@
 #include "sab_context.cuh"
 #include "sab_saca.cuh"
 #include "sab_search.cuh"
+#include "sab_ms.cuh"
 #include "sab_pack.cuh"
 #include "sab_bwt.cuh"
 
@@ -602,11 +603,18 @@ struct SabReplica {
     u32* d_out0 = nullptr;
     u32* d_out1 = nullptr;
     size_t np_cap = 0;
+    // matching-statistics extension, built by the first sab200_matching_statistics_batch* call on the index
+    u32* d_isa = nullptr;
+    u32* d_lcp = nullptr;
+    u32* d_lmin = nullptr;  // the levels of block minima above the LCP array, one after the other
+    u32* d_ms = nullptr;    // len / lo / hi of the positions of a call, ms_cap each (grow-only)
+    size_t ms_cap = 0;
 };
 struct sab200_index {
     u64 n = 0;
     bool has_bkt = false;
     bool count_probes = false;
+    bool has_ms = false;  // every replica holds the matching-statistics extension
     std::vector<SabReplica> rep;
     std::mutex mu;
 };
@@ -624,6 +632,10 @@ static void replica_free(SabReplica& r) {
     cudaFree(r.d_offs);
     cudaFree(r.d_out0);
     cudaFree(r.d_out1);
+    cudaFree(r.d_isa);
+    cudaFree(r.d_lcp);
+    cudaFree(r.d_lmin);
+    cudaFree(r.d_ms);
     if (r.stream2) cudaStreamDestroy(r.stream2);
     r = SabReplica();
 }
@@ -898,6 +910,247 @@ extern "C" uint64_t sab200_index_directory(sab200_index* ix, uint32_t* sigma, ui
     if (sigma) *sigma = ix->rep[0].pd.sigma;
     if (depth) *depth = ix->rep[0].pd.depth;
     return ix->rep[0].pd.pw[ix->rep[0].pd.depth];
+}
+
+// ---- matching statistics ----------------------------------------------------------------------
+// Entries of every level of the block-minimum hierarchy (cnt[0] = n + 1, the LCP array itself) up to the first level
+// of at most 256 entries; returns that level's index, *extra = the entries of the levels above the LCP array.
+static u32 ms_levels(u64 n, u64 cnt[SAB_MS_LEVELS], u64* extra) {
+    u32 top = 0;
+    cnt[0] = n + 1;
+    *extra = 0;
+    while (cnt[top] > 256) {
+        cnt[top + 1] = div_up64(cnt[top], 256);
+        *extra += cnt[++top];
+    }
+    return top;
+}
+
+static void replica_free_ms(SabReplica& r) {
+    cudaFree(r.d_isa);
+    cudaFree(r.d_lcp);
+    cudaFree(r.d_lmin);
+    r.d_isa = r.d_lcp = r.d_lmin = nullptr;
+}
+
+// isa by the integrity kernels (a wrong suffix array is refused here, before anything scatters through it), the LCP
+// array by Kasai from that isa, then the block minima level by level.
+static int replica_build_ms_run(SabReplica& r, u64 n) {
+    SabUse u;
+    SAB_TRY(sab_use(r.ctx->device, &u));
+    SabContext* c = u.c;
+    cudaStream_t st = c->stream;
+    u64 cnt[SAB_MS_LEVELS], extra;
+    const u32 top = ms_levels(n, cnt, &extra);
+    const size_t arr = ((size_t)n + 2) * sizeof(u32);
+    if (cudaMalloc(&r.d_isa, arr) != cudaSuccess || cudaMalloc(&r.d_lcp, arr) != cudaSuccess ||
+        cudaMalloc(&r.d_lmin, (size_t)(extra + 1) * sizeof(u32)) != cudaSuccess) {
+        cudaGetLastError();
+        sab_set_error("matching statistics: the index extension (%zu bytes) does not fit on device %d",
+                      2 * arr + (size_t)(extra + 1) * sizeof(u32), c->device);
+        return SAB_ERR_OOM;
+    }
+    u32* flag = &c->scratch->check_flag;
+    SAB_CUDA_TRY(cudaMemsetAsync(r.d_isa, 0xff, arr, st));
+    SAB_CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(u32), st));
+    const unsigned blocks = (unsigned)div_up64(n + 1, 256);
+    SAB_LAUNCH(sufcheck_scatter_kernel, blocks, 256, 0, st, (const u32*)r.d_sa, n + 1, n, r.d_isa, flag);
+    SAB_LAUNCH_CHECK();
+    SAB_LAUNCH(sufcheck_order_kernel, blocks, 256, 0, st, (const u8*)r.d_text, (const u32*)r.d_sa, n + 1, n, (const u32*)r.d_isa, flag);
+    SAB_LAUNCH_CHECK();
+    u32 bad;
+    SAB_TRY(sab_read_u32(c, flag, 1, &bad));
+    if (bad) {
+        sab_set_error("matching statistics: the index's suffix array is not the suffix array of its text");
+        return SAB_ERR_ARGS;
+    }
+    const u64 chunks = div_up64(n ? n : 1, SAB_LCP_CHUNK);
+    SAB_LAUNCH(lcp_kasai_kernel, (unsigned)div_up64(chunks, 256), 256, 0, st, (const u8*)r.d_text, n, (const u32*)r.d_sa,
+               (const u32*)r.d_isa, r.d_lcp);
+    SAB_LAUNCH_CHECK();
+    const u32* in = r.d_lcp;
+    u32* out = r.d_lmin;
+    for (u32 k = 1; k <= top; ++k) {
+        SAB_LAUNCH(lcp_block_min_kernel, (unsigned)div_up64(cnt[k] * 32, 256), 256, 0, st, in, cnt[k - 1], out, cnt[k]);
+        SAB_LAUNCH_CHECK();
+        in = out;
+        out += cnt[k];
+    }
+    SAB_CUDA_TRY(cudaStreamSynchronize(st));
+    return SAB_OK;
+}
+
+// The extension on every replica, built once per index (under ix->mu); on failure none is kept.
+static int ms_prepare(sab200_index* ix) {
+    if (ix->has_ms) return SAB_OK;
+    for (auto& r : ix->rep) {
+        const int rc = replica_build_ms_run(r, ix->n);
+        if (rc != SAB_OK) {
+            for (auto& q : ix->rep) replica_free_ms(q);
+            return rc;
+        }
+    }
+    ix->has_ms = true;
+    return SAB_OK;
+}
+
+static MsArgs ms_args(const SabReplica& r, u64 n, const u8* d_qs_adj, const u64* d_offs, u64 nq) {
+    MsArgs a;
+    memset(&a, 0, sizeof(a));
+    a.s.pd = r.pd;
+    a.s.text = r.d_text;
+    a.s.n = n;
+    a.s.sa = r.d_sa;
+    a.s.pats = d_qs_adj;
+    a.s.offs = d_offs;
+    a.s.np = nq;
+    a.isa = r.d_isa;
+    u64 extra;
+    a.top = ms_levels(n, a.cnt, &extra);
+    a.lvl[0] = r.d_lcp;
+    for (u32 k = 1, off = 0; k <= a.top; off += (u32)a.cnt[k], ++k) a.lvl[k] = r.d_lmin + off;
+    // the directory narrows a from-scratch search to ~16 suffixes; below its depth a carried interval is no narrower
+    a.fresh_below = r.pd.dir ? r.pd.depth : 1;
+    return a;
+}
+
+static int launch_ms(MsArgs a, u64 p0, u64 p1, u32* len_adj, u32* lo_adj, u32* hi_adj, cudaStream_t st) {
+    a.p0 = p0;
+    a.p1 = p1;
+    a.len = len_adj;
+    a.lo = lo_adj;
+    a.hi = hi_adj;
+    const u64 warps = div_up64(p1 - p0, SAB_MS_CHUNK);
+    SAB_LAUNCH(ms_kernel, (unsigned)div_up64(warps * 32, SAB_MS_THREADS), SAB_MS_THREADS, 0, st, a);
+    SAB_LAUNCH_CHECK();
+    return SAB_OK;
+}
+
+#ifndef SAB_MS_SUB
+#define SAB_MS_SUB ((u64)SAB_MS_CHUNK << 12)  // positions per pipelined launch (4 Mi: 48 MiB of results)
+#endif
+
+extern "C" int32_t sab200_matching_statistics_batch(sab200_index* ix, const uint8_t* qs, const uint64_t* offs, uint64_t nq,
+                                                    uint32_t* len, uint32_t* lo, uint32_t* hi) {
+    if (!ix || (nq > 0 && !offs)) {
+        sab_set_error("matching statistics: bad arguments");
+        return SAB_ERR_ARGS;
+    }
+    if (nq == 0) return SAB_OK;
+    if (nq > 0x7fffffffull) {
+        sab_set_error("matching statistics: at most 2^31-1 queries per call");
+        return SAB_ERR_ARGS;
+    }
+    for (u64 q = 0; q < nq; ++q)
+        if (offs[q + 1] < offs[q]) {
+            sab_set_error("matching statistics: the offsets decrease at query %llu", (unsigned long long)q);
+            return SAB_ERR_ARGS;
+        }
+    const u64 b0 = offs[0], b1 = offs[nq];
+    if (b1 > b0 && (!qs || !len || !lo || !hi)) {
+        sab_set_error("matching statistics: bad arguments");
+        return SAB_ERR_ARGS;
+    }
+    std::lock_guard<std::mutex> lk(ix->mu);
+    SAB_TRY(ms_prepare(ix));
+    if (b1 == b0) return SAB_OK;
+    // every replica holds the whole concatenation (a match may run past its share) and walks an equal share of the
+    // positions, cut at chunk boundaries
+    const int P = (int)ix->rep.size();
+    const u64 per = div_up64(div_up64(b1 - b0, SAB_MS_CHUNK), (u64)P) * SAB_MS_CHUNK;
+    for (int d = 0; d < P; ++d) {
+        const u64 s0 = b0 + (u64)d * per;
+        if (s0 >= b1) continue;
+        const u64 share = b1 - s0 < per ? b1 - s0 : per;
+        SabReplica& r = ix->rep[d];
+        SAB_CUDA_TRY(cudaSetDevice(r.ctx->device));
+        SAB_TRY(replica_reserve(r, (size_t)(b1 - b0), (size_t)nq));
+        if (r.ms_cap < share) {
+            cudaFree(r.d_ms);
+            r.d_ms = nullptr;
+            r.ms_cap = 0;
+            SAB_CUDA_TRY(cudaMalloc(&r.d_ms, (size_t)share * 3 * sizeof(u32)));
+            r.ms_cap = share;
+        }
+        SAB_CUDA_TRY(cudaMemcpyAsync(r.d_pats, qs + b0, b1 - b0, cudaMemcpyHostToDevice, r.ctx->stream));
+        SAB_CUDA_TRY(cudaMemcpyAsync(r.d_offs, offs, (nq + 1) * sizeof(u64), cudaMemcpyHostToDevice, r.ctx->stream));
+    }
+    for (int d = 0; d < P; ++d) {
+        const u64 s0 = b0 + (u64)d * per;
+        if (s0 >= b1) continue;
+        const u64 s1 = b1 - s0 < per ? b1 : s0 + per;
+        SabReplica& r = ix->rep[d];
+        SAB_CUDA_TRY(cudaSetDevice(r.ctx->device));
+        SAB_CUDA_TRY(cudaStreamSynchronize(r.ctx->stream));
+        const MsArgs a = ms_args(r, ix->n, r.d_pats - b0, r.d_offs, nq);
+        u32 *dl = r.d_ms - s0, *dlo = dl + r.ms_cap, *dhi = dlo + r.ms_cap;  // indexed by absolute position
+        // Sub-ranges alternate between two streams: the download of one runs under the kernel of the next, which is
+        // launched first so that a pageable destination (a synchronous copy) does not leave the device idle.
+        auto download = [&](u64 p0, u64 p1, cudaStream_t st) -> int {
+            SAB_CUDA_TRY(cudaMemcpyAsync(len + p0, dl + p0, (p1 - p0) * sizeof(u32), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaMemcpyAsync(lo + p0, dlo + p0, (p1 - p0) * sizeof(u32), cudaMemcpyDeviceToHost, st));
+            SAB_CUDA_TRY(cudaMemcpyAsync(hi + p0, dhi + p0, (p1 - p0) * sizeof(u32), cudaMemcpyDeviceToHost, st));
+            return SAB_OK;
+        };
+        u64 prev0 = 0, prev1 = 0;
+        cudaStream_t prev_st = nullptr;
+        int which = 0;
+        for (u64 p0 = s0; p0 < s1; p0 += SAB_MS_SUB, which ^= 1) {
+            const u64 p1 = s1 - p0 < SAB_MS_SUB ? s1 : p0 + SAB_MS_SUB;
+            cudaStream_t st = (which && r.stream2) ? r.stream2 : r.ctx->stream;
+            SAB_TRY(launch_ms(a, p0, p1, dl, dlo, dhi, st));
+            if (prev1 > prev0) SAB_TRY(download(prev0, prev1, prev_st));
+            prev0 = p0;
+            prev1 = p1;
+            prev_st = st;
+        }
+        SAB_TRY(download(prev0, prev1, prev_st));
+    }
+    for (int d = 0; d < P; ++d) {
+        SabReplica& r = ix->rep[d];
+        SAB_CUDA_TRY(cudaSetDevice(r.ctx->device));
+        SAB_CUDA_TRY(cudaStreamSynchronize(r.ctx->stream));
+        if (r.stream2) SAB_CUDA_TRY(cudaStreamSynchronize(r.stream2));
+    }
+    return SAB_OK;
+}
+
+// Device-resident form on the GPU of replica 0: d_qs is indexed by the absolute offsets and followed by at least
+// 8 readable bytes; d_len / d_lo / d_hi are indexed by absolute position.
+extern "C" int32_t sab200_matching_statistics_batch_device(sab200_index* ix, const uint8_t* d_qs, const uint64_t* d_offs, uint64_t nq,
+                                                           uint32_t* d_len, uint32_t* d_lo, uint32_t* d_hi) {
+    if (!ix || (nq > 0 && (!d_offs || !d_qs || !d_len || !d_lo || !d_hi))) {
+        sab_set_error("matching statistics: bad arguments");
+        return SAB_ERR_ARGS;
+    }
+    if (nq == 0) return SAB_OK;
+    if (nq > 0x7fffffffull) {
+        sab_set_error("matching statistics: at most 2^31-1 queries per call");
+        return SAB_ERR_ARGS;
+    }
+    std::lock_guard<std::mutex> lk(ix->mu);
+    SAB_TRY(ms_prepare(ix));
+    SabReplica& r = ix->rep[0];
+    SabUse u;
+    SAB_TRY(sab_use(r.ctx->device, &u));
+    cudaStream_t st = u.c->stream;
+    u32* flag = &u.c->scratch->ms_offs;
+    SAB_CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(u32), st));
+    SAB_LAUNCH(ms_offs_check_kernel, (unsigned)div_up64(nq, 256), 256, 0, st, (const u64*)d_offs, nq, flag);
+    SAB_LAUNCH_CHECK();
+    u64 ends[2];
+    SAB_CUDA_TRY(cudaMemcpyAsync(&ends[0], d_offs, sizeof(u64), cudaMemcpyDeviceToHost, st));
+    SAB_CUDA_TRY(cudaMemcpyAsync(&ends[1], d_offs + nq, sizeof(u64), cudaMemcpyDeviceToHost, st));
+    u32 bad;
+    SAB_TRY(sab_read_u32(u.c, flag, 1, &bad));
+    if (bad) {
+        sab_set_error("matching statistics: the offsets decrease");
+        return SAB_ERR_ARGS;
+    }
+    if (ends[1] == ends[0]) return SAB_OK;
+    SAB_TRY(launch_ms(ms_args(r, ix->n, d_qs, d_offs, nq), ends[0], ends[1], d_len, d_lo, d_hi, st));
+    SAB_CUDA_TRY(cudaStreamSynchronize(st));
+    return SAB_OK;
 }
 
 // ---- pack serialisation ---------------------------------------------------------------------

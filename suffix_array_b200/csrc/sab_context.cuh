@@ -50,13 +50,14 @@ struct SabEventPair {
 struct SabScratch {
     u32 count;      // init_ranks / re-rank: records still active
     u32 filter[2];  // split filter: records to sort, records parked
-    u32 check_flag; // sab200_check: set when the array is not the suffix array of the text
+    u32 check_flag; // sab200_check, matching-statistics extension: set when the array is not the suffix array of the text
     u32 big;        // in-group sort: records of groups too large for it
     u32 nu;         // multi-GPU lazy look-ups: requests that found no rank
     u32 skip[16];   // radix sort: 1 for each digit place where all keys agree (SAB_MAX_PASSES of them)
     u32 hist[256];  // byte histogram of a text
     u16 lut[256];   // code table of the running construction (sab_plan_alphabet)
     u32 bwt[2];     // sab200_bwt: the primary index; sab200_inverse_bwt: sample rows, list position of row p
+    u32 ms_offs;    // sab200_matching_statistics_batch_device: set when the query offsets decrease
 };
 
 // Pinned host staging of a context: readbacks land here, and small uploads leave from here, not from the caller's stack.

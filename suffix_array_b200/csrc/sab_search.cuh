@@ -129,6 +129,34 @@ __device__ __forceinline__ u64 prefix_code(const u8* __restrict__ text, u64 n, u
     return c;
 }
 
+// Narrows [*lo, *hi) to the directory range of the pattern's first `depth` symbols (pd.dir must be set).  The lower
+// bound of the pattern lies in the narrowed range (or at its end when it is empty) whatever the pattern's length.
+__device__ __forceinline__ void prefix_dir_narrow(const PrefixDir& pd, const u8* __restrict__ pat, u64 m, u64* lo, u64* hi) {
+    const u32 depth = pd.depth, sigma = pd.sigma;
+    u64 code = 0;
+    u32 t = 0, e = 0x8000u;
+    for (; t < depth && t < m; ++t) {
+        e = pd.lut[pat[t]];
+        if (!(e & 0x8000u)) break;
+        code = code * sigma + (e & 0x1ffu);
+    }
+    u64 clo, chi;
+    if (e & 0x8000u) {  // t symbols of the pattern, all present in the text: every code that starts with them
+        clo = code * pd.pw[depth - t];
+        chi = clo + pd.pw[depth - t];
+    } else {
+        // byte t of the pattern does not occur in the text: the pattern falls between two neighbouring codes --
+        // unless it is smaller than every symbol, where it still follows the suffixes that END after the t
+        // symbols (they are padded with the minimum symbol and share the first code of the prefix)
+        clo = (code * sigma + (e & 0x1ffu)) * pd.pw[depth - t - 1];
+        chi = clo + ((e & 0x1ffu) == 0 ? 1u : 0u);
+    }
+    const u64 dlo = pd.dir[clo], dhi = pd.dir[chi];
+    if (dlo > *lo) *lo = dlo;
+    if (dhi < *hi) *hi = dhi;
+    if (*hi < *lo) *hi = *lo;
+}
+
 __global__ void __launch_bounds__(256) fill_u32_kernel(u32* __restrict__ out, u64 count, u32 value) {
     const u64 stride = (u64)gridDim.x * blockDim.x;
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride) out[i] = value;
@@ -263,33 +291,9 @@ __global__ void __launch_bounds__(SAB_SEARCH_THREADS) search_kernel(SearchArgs a
         }
         return;
     }
-    if (MODE != 2 && a.pd.dir) {
-        // narrow [lo, hi) to the suffixes that share the pattern's first symbols (search_lcp keeps the reference's
-        // range: its answer depends on the borders of the two-byte bucket, src/sa.rs:224-252)
-        const u32 depth = a.pd.depth, sigma = a.pd.sigma;
-        u64 code = 0;
-        u32 t = 0, e = 0x8000u;
-        for (; t < depth && t < m; ++t) {
-            e = a.pd.lut[pat[t]];
-            if (!(e & 0x8000u)) break;
-            code = code * sigma + (e & 0x1ffu);
-        }
-        u64 clo, chi;
-        if (e & 0x8000u) {  // t symbols of the pattern, all present in the text: every code that starts with them
-            clo = code * a.pd.pw[depth - t];
-            chi = clo + a.pd.pw[depth - t];
-        } else {
-            // byte t of the pattern does not occur in the text: the pattern falls between two neighbouring codes --
-            // unless it is smaller than every symbol, where it still follows the suffixes that END after the t
-            // symbols (they are padded with the minimum symbol and share the first code of the prefix)
-            clo = (code * sigma + (e & 0x1ffu)) * a.pd.pw[depth - t - 1];
-            chi = clo + ((e & 0x1ffu) == 0 ? 1u : 0u);
-        }
-        const u64 dlo = a.pd.dir[clo], dhi = a.pd.dir[chi];
-        if (dlo > lo) lo = dlo;
-        if (dhi < hi) hi = dhi;
-        if (hi < lo) hi = lo;
-    }
+    // narrow [lo, hi) to the suffixes that share the pattern's first symbols (search_lcp keeps the reference's
+    // range: its answer depends on the borders of the two-byte bucket, src/sa.rs:224-252)
+    if (MODE != 2 && a.pd.dir) prefix_dir_narrow(a.pd, pat, m, &lo, &hi);
     u32 nprobe = 0;
     // lower bound: first index whose suffix is not < pat   (src/sa.rs:181-190)
     u64 i = lo, k = hi;

@@ -18,6 +18,9 @@ extern "C" {
     pub fn sab200_search_all_batch(ix: *mut Sab200Index, pats: *const u8, offs: *const u64, np: u64, lo: *mut u32, hi: *mut u32) -> i32;
     pub fn sab200_contains_batch(ix: *mut Sab200Index, pats: *const u8, offs: *const u64, np: u64, out: *mut u8) -> i32;
     pub fn sab200_search_lcp_batch(ix: *mut Sab200Index, pats: *const u8, offs: *const u64, np: u64, start: *mut u32, end: *mut u32) -> i32;
+    // matching statistics: len / lo / hi hold offs[nq] entries each, indexed by the absolute offset in qs (include/sab200.h)
+    pub fn sab200_matching_statistics_batch(ix: *mut Sab200Index, qs: *const u8, offs: *const u64, nq: u64, len: *mut u32, lo: *mut u32, hi: *mut u32) -> i32;
+    pub fn sab200_matching_statistics_batch_device(ix: *mut Sab200Index, d_qs: *const u8, d_offs: *const u64, nq: u64, d_len: *mut u32, d_lo: *mut u32, d_hi: *mut u32) -> i32;
     // feature "pack": GPU forms of PackedSuffixArray::from_sa + dump_bytes / load_bytes + into_sa (src/packed_sa.rs)
     pub fn sab200_pack_bound(sa_len: u64) -> u64;
     pub fn sab200_pack(sa: *const u32, sa_len: u64, out: *mut u8, out_cap: u64, out_len: *mut u64) -> i32;

@@ -233,6 +233,29 @@ class SuffixArray:
                    "sab200_search_lcp_batch")
         return st, en
 
+    # ---- matching statistics (no reference counterpart; include/sab200.h)
+    def matching_statistics_batch(self, queries, offs=None):
+        """-> (len, lo, hi) uint32 arrays with one entry per byte of the concatenated queries.  At position i of a
+        query Q, len[i] is the longest prefix of the rest of Q that occurs in the text, and sa[lo[i]:hi[i]] are the
+        positions where it occurs ([0, n+1) when len[i] = 0).  The first call on an index builds its extension
+        (integrity check, inverse suffix array, LCP array); a suffix array that is not the text's raises ValueError."""
+        flat, offs = (queries, offs) if offs is not None else _pack_patterns(queries)
+        flat = np.ascontiguousarray(flat, dtype=np.uint8)
+        offs = np.ascontiguousarray(offs, dtype=np.uint64)
+        nq = offs.size - 1
+        total = int(offs[-1]) if nq > 0 else 0
+        out = [np.empty(total, dtype=np.uint32) for _ in range(3)]
+        L = _lib.lib()
+        rc = L.sab200_matching_statistics_batch(self._get_index(), _ptr(flat), _ptr(offs), max(nq, 0), *[_ptr(o) for o in out])
+        if rc == -1:
+            raise ValueError(L.sab200_last_error().decode("utf-8", "replace"))
+        _lib.check(rc, "sab200_matching_statistics_batch")
+        return tuple(out)
+
+    def matching_statistics(self, query):
+        """matching_statistics_batch of the single query"""
+        return self.matching_statistics_batch([query])
+
     # ---- per-pattern queries (src/sa.rs:164-253)
     def contains(self, pat):
         return bool(self.contains_batch([pat])[0])
