@@ -68,6 +68,12 @@ struct SabStaging {
     u64 wide[256];  // u64 rows of the multi-GPU driver, both ways
 };
 
+// A grow-only device buffer that an entry point carves into the buffers of one call.
+struct SabArena {
+    char* base = nullptr;
+    size_t bytes = 0, used = 0;
+};
+
 struct SabContext {
     int device = 0;
     cudaStream_t stream = 0;
@@ -86,10 +92,7 @@ struct SabContext {
     u32 scan_epoch = 0;
     SabScratch* scratch = nullptr;  // device
     SabStaging* staging = nullptr;  // pinned host
-    // arena
-    char* arena = nullptr;
-    size_t arena_bytes = 0;
-    size_t arena_used = 0;
+    SabArena arena;
     size_t arena_want_seen = 0;  // request the arena was last sized for (it may have been capped by the free memory)
     void* bounce[2] = {nullptr, nullptr};        // pinned bounce buffers for pageable caller memory (sab_copy_*)
     cudaEvent_t bounce_ev[2] = {nullptr, nullptr};
@@ -106,7 +109,8 @@ struct SabContext {
 SabContext* sab_get_context(int device);
 int sab_context_init(SabContext* c);
 void sab_context_destroy(SabContext* c);
-int sab_arena_reserve(SabContext* c, size_t bytes);
+int sab_arena_reserve(SabArena* a, cudaStream_t st, size_t bytes);
+static inline int sab_arena_reserve(SabContext* c, size_t bytes) { return sab_arena_reserve(&c->arena, c->stream, bytes); }
 int sab_ensure_lookback(SabContext* c, size_t tiles);
 int sab_ensure_scan(SabContext* c, size_t tiles);
 
@@ -114,10 +118,10 @@ static inline size_t sab_align_up(size_t x, size_t a) { return (x + a - 1) / a *
 
 // bump allocation inside the arena (call sab_arena_reserve first)
 template <typename T>
-static inline T* sab_arena_take(SabContext* c, size_t count) {
-    size_t off = sab_align_up(c->arena_used, 256);
-    c->arena_used = off + count * sizeof(T);
-    return (T*)(c->arena + off);
+static inline T* sab_arena_take(SabArena* a, size_t count) {
+    size_t off = sab_align_up(a->used, 256);
+    a->used = off + count * sizeof(T);
+    return (T*)(a->base + off);
 }
 
 // One buffer of an entry point's arena: *dst receives its address; a null dst reserves the room without handing it out.
@@ -130,16 +134,20 @@ struct SabSlice {
 };
 
 // Reserves the sum of the 256-aligned sizes and hands the buffers out in order from the bottom of the arena.
-static inline int sab_arena_carve(SabContext* c, std::initializer_list<SabSlice> slices) {
+// A reallocation first waits for `st`, the stream that last used the arena.
+static inline int sab_arena_carve(SabArena* a, cudaStream_t st, std::initializer_list<SabSlice> slices) {
     size_t total = 0;
     for (const SabSlice& s : slices) total += sab_align_up(s.bytes, 256);
-    SAB_TRY(sab_arena_reserve(c, total));
-    c->arena_used = 0;
+    SAB_TRY(sab_arena_reserve(a, st, total));
+    a->used = 0;
     for (const SabSlice& s : slices) {
-        char* p = sab_arena_take<char>(c, s.bytes);
+        char* p = sab_arena_take<char>(a, s.bytes);
         if (s.dst) *s.dst = p;
     }
     return SAB_OK;
+}
+static inline int sab_arena_carve(SabContext* c, std::initializer_list<SabSlice> slices) {
+    return sab_arena_carve(&c->arena, c->stream, slices);
 }
 
 // The context of `device`, locked and current on the calling thread: the prologue of the entry points.

@@ -277,7 +277,7 @@ struct DistArena {
 #define SAB_ARENA_CHECK(A)                                                                                     \
     do {                                                                                                       \
         if (!(A).ok) {                                                                                         \
-            sab_set_error("%s:%d: device arena exhausted (%zu bytes)", __FILE__, __LINE__, c->arena_bytes);    \
+            sab_set_error("%s:%d: device arena exhausted (%zu bytes)", __FILE__, __LINE__, c->arena.bytes);    \
             return SAB_ERR_OOM;                                                                                \
         }                                                                                                      \
     } while (0)
@@ -325,11 +325,11 @@ static inline size_t sab_dist_want(u64 B) {
 }
 static int sab_dist_reserve(SabContext* c, u64 B) {
     size_t want = sab_dist_want(B);
-    if (c->arena_bytes >= want || c->arena_want_seen == want) return SAB_OK;  // steady state: no driver call at all
+    if (c->arena.bytes >= want || c->arena_want_seen == want) return SAB_OK;  // steady state: no driver call at all
     c->arena_want_seen = want;
     size_t free_b = 0, total_b = 0;
     SAB_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
-    const size_t avail = (size_t)((double)(free_b + c->arena_bytes) * 0.94);
+    const size_t avail = (size_t)((double)(free_b + c->arena.bytes) * 0.94);
     if (want > avail) want = avail;
     return sab_arena_reserve(c, want);
 }
@@ -353,7 +353,7 @@ static int sab_peers_update(sab200_comm* cm, SabContext* c, const u64* rows, int
     cudaIpcMemHandle_t mine;
     memset(&mine, 0, sizeof(mine));
     u64 fail = 0;
-    if (cudaIpcGetMemHandle(&mine, c->arena) != cudaSuccess) {
+    if (cudaIpcGetMemHandle(&mine, c->arena.base) != cudaSuccess) {
         cudaGetLastError();
         fail = 1;
     }
@@ -375,7 +375,7 @@ static int sab_peers_update(sab200_comm* cm, SabContext* c, const u64* rows, int
         p.base = nullptr;
         p.ipc = false;
         if (s == g) {
-            p.base = c->arena;
+            p.base = c->arena.base;
             continue;
         }
         if (p.pid == mypid) {
@@ -558,7 +558,7 @@ struct DistRun {
         // the count exchange also carries what the peers need to address this rank's receive buffers directly
         // (fused exchange, below): process, device, arena, offset of the key buffer inside it
         const u64 k0_off = sab_align_up(A.lo, 256);
-        u64 extra[5] = {(u64)getpid(), (u64)c->device, (u64)(uintptr_t)c->arena, (u64)c->arena_bytes, k0_off};
+        u64 extra[5] = {(u64)getpid(), (u64)c->device, (u64)(uintptr_t)c->arena.base, (u64)c->arena.bytes, k0_off};
         constexpr int NX = 5;
         u64 rows[SAB_MAX_RANKS * 32];
         SAB_TRY((sab_plan_exchange<u64, SplitterDigit>(cm, c, keysA, count, nullptr, sdop, nullptr, 0, extra, NX, &pk, rows)));
@@ -603,7 +603,7 @@ struct DistRun {
                 }
                 const u64 koff = rows[(size_t)d * W + P + 4];
                 const u64 voff = sab_align_up(koff + (Rd + 8) * sizeof(u64), 256);
-                char* base = d == g ? c->arena : (char*)cm->peers[d].base;
+                char* base = d == g ? c->arena.base : (char*)cm->peers[d].base;
                 po.k[d] = (u64)(uintptr_t)(base + koff);
                 po.v[d] = (u64)(uintptr_t)(base + voff);
                 h[d] = before;
@@ -791,21 +791,21 @@ struct DistRun {
         if (!fused || rebalanced) return SAB_OK;
         // row: offsets of rank_local, text, sorted keys, directory inside the arena; directory origin, slice length, offset
         u64* hrow = cm->h_small + 32;
-        hrow[0] = (u64)((char*)rank_local - c->arena);
-        hrow[1] = (u64)((const char*)d_text - c->arena);
-        hrow[2] = (u64)((const char*)sortedK - c->arena);
-        hrow[3] = (u64)((char*)dir - c->arena);
+        hrow[0] = (u64)((char*)rank_local - c->arena.base);
+        hrow[1] = (u64)((const char*)d_text - c->arena.base);
+        hrow[2] = (u64)((const char*)sortedK - c->arena.base);
+        hrow[3] = (u64)((char*)dir - c->arena.base);
         hrow[4] = dlo;
         hrow[5] = R;
         hrow[6] = sa_off;
-        hrow[7] = ((const char*)d_text >= c->arena && (const char*)d_text < c->arena + c->arena_bytes) ? 1 : 0;
+        hrow[7] = ((const char*)d_text >= c->arena.base && (const char*)d_text < c->arena.base + c->arena.bytes) ? 1 : 0;
         SAB_CUDA_TRY(cudaMemcpyAsync(cm->d_small, hrow, 8 * sizeof(u64), cudaMemcpyHostToDevice, st));
         u64 prow[SAB_MAX_RANKS * 8];
         SAB_TRY(sab_comm_gather_rows(cm, st, 8, prow));  // also orders every rank's ISA scatter before the first gather
         bool ok = true;
         for (int d = 0; d < P; ++d) {
             const u64* r = prow + (size_t)d * 8;
-            char* pb = d == g ? c->arena : (char*)cm->peers[d].base;
+            char* pb = d == g ? c->arena.base : (char*)cm->peers[d].base;
             ok = ok && r[7] == 1 && pb != nullptr;
             pt.rank_local[d] = (u32*)(pb + r[0]);
             pt.text[d] = (const u8*)(pb + r[1]);
@@ -1230,9 +1230,9 @@ static int sab_sharded_run(sab200_comm* cm, const u8* shard, u64 shard_len, u64 
     }
     SAB_TRY(sab_dist_reserve(c, B));
     DistArena A;
-    A.base = c->arena;
+    A.base = c->arena.base;
     A.lo = 0;
-    A.hi = c->arena_bytes & ~(size_t)255;
+    A.hi = c->arena.bytes & ~(size_t)255;
     A.ok = true;
     cudaStream_t st = c->stream;
     const u8* d_text = shard;

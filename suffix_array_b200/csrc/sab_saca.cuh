@@ -624,14 +624,14 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
         return SAB_OK;
     }
     SAB_TRY(sab_arena_reserve(c, sab_saca_workspace_bytes(n)));
-    c->arena_used = 0;
+    c->arena.used = 0;
     SortBuffers<u64> buf;
-    buf.k[0] = sab_arena_take<u64>(c, n + 8);
-    buf.k[1] = sab_arena_take<u64>(c, n + 8);
-    buf.v[0] = sab_arena_take<u32>(c, n + 8);
-    buf.v[1] = sab_arena_take<u32>(c, n + 8);
-    u32* r1buf = sab_arena_take<u32>(c, n + 8);
-    u32* rank = sab_arena_take<u32>(c, n + 9);
+    buf.k[0] = sab_arena_take<u64>(&c->arena, n + 8);
+    buf.k[1] = sab_arena_take<u64>(&c->arena, n + 8);
+    buf.v[0] = sab_arena_take<u32>(&c->arena, n + 8);
+    buf.v[1] = sab_arena_take<u32>(&c->arena, n + 8);
+    u32* r1buf = sab_arena_take<u32>(&c->arena, n + 8);
+    u32* rank = sab_arena_take<u32>(&c->arena, n + 9);
     buf.cur = 0;
     SAB_TRY(sab_ensure_scan(c, (size_t)div_up64(n, SAB_SCAN_TILE)));
 
@@ -656,8 +656,8 @@ static int sab_saca_device(SabContext* c, const u8* d_text, u64 n, u32* d_sa) {
     u32* act_idx = buf.v[buf.cur ^ 1];
     const int dir_bits = sab_dir_bits(n, al.key_bits, SAB_DIR_SHIFT);
     const int dir_shift = al.key_bits - dir_bits;
-    u32* dir = sab_arena_take<u32>(c, ((size_t)1 << dir_bits) + 8);
-    u32* split_bitmap = sab_arena_take<u32>(c, (size_t)n / 32 + 8);
+    u32* dir = sab_arena_take<u32>(&c->arena, ((size_t)1 << dir_bits) + 8);
+    u32* split_bitmap = sab_arena_take<u32>(&c->arena, (size_t)n / 32 + 8);
     SAB_CUDA_TRY(cudaMemsetAsync(rank, 0xff, n * sizeof(u32), st));
     SAB_CUDA_TRY(cudaMemsetAsync(rank + n, 0, sizeof(u32), st));  // the empty suffix has rank 0
     c->staging->sa0 = (u32)n;

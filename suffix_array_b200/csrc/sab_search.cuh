@@ -426,6 +426,12 @@ lcp_kasai_kernel(const u8* __restrict__ s, u64 n, const u32* __restrict__ sa, co
         if (h) --h;
     }
 }
+static int sab_launch_kasai(SabContext* c, const u8* d_s, u64 n, const u32* d_sa, const u32* d_isa, u32* d_lcp) {
+    const u64 chunks = div_up64(n ? n : 1, SAB_LCP_CHUNK);
+    SAB_LAUNCH(lcp_kasai_kernel, (unsigned)div_up64(chunks, 256), 256, 0, c->stream, d_s, n, d_sa, d_isa, d_lcp);
+    SAB_LAUNCH_CHECK();
+    return SAB_OK;
+}
 
 // ------------------------------------------------------------------ linear-time integrity check
 // flags[0] != 0 -> not a suffix array.  isa must be pre-filled with 0xFFFFFFFF.
@@ -460,4 +466,19 @@ sufcheck_order_kernel(const u8* __restrict__ text, const u32* __restrict__ sa, u
     }
     const u8 cx = text[x], cb = text[b];
     if (cx > cb || (cx == cb && isa[x + 1] >= isa[b + 1])) flags[0] = 1;
+}
+
+// *bad = 0 when d_sa (sa_len entries) is the suffix array of the text; d_isa (n + 2 words) then holds its inverse.
+// Waits for c->stream.
+static int sab_isa_check(SabContext* c, const u8* d_s, u64 n, const u32* d_sa, u64 sa_len, u32* d_isa, u32* bad) {
+    cudaStream_t st = c->stream;
+    u32* flag = &c->scratch->check_flag;
+    SAB_CUDA_TRY(cudaMemsetAsync(d_isa, 0xff, ((size_t)n + 2) * sizeof(u32), st));
+    SAB_CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(u32), st));
+    const unsigned blocks = (unsigned)div_up64(sa_len, 256);
+    SAB_LAUNCH(sufcheck_scatter_kernel, blocks, 256, 0, st, d_sa, sa_len, n, d_isa, flag);
+    SAB_LAUNCH_CHECK();
+    SAB_LAUNCH(sufcheck_order_kernel, blocks, 256, 0, st, d_s, d_sa, sa_len, n, (const u32*)d_isa, flag);
+    SAB_LAUNCH_CHECK();
+    return sab_read_u32(c, flag, 1, bad);
 }

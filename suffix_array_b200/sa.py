@@ -37,6 +37,14 @@ def _pack_patterns(pats):
     return flat, offs
 
 
+def _batch_input(pats, offs):
+    """(concatenation, offsets) as given, or packed from a list of bytes-like -> (flat, offs, number of patterns)"""
+    flat, offs = (pats, offs) if offs is not None else _pack_patterns(pats)
+    flat = np.ascontiguousarray(flat, dtype=np.uint8)
+    offs = np.ascontiguousarray(offs, dtype=np.uint64)
+    return flat, offs, offs.size - 1
+
+
 def saca(s, sa, ngpus=1):
     """src/saca.rs:9-15.  Asserts mirror the reference's (`:10-11`), with the new MAX_LENGTH."""
     assert s.size <= MAX_LENGTH
@@ -202,10 +210,7 @@ class SuffixArray:
     # ---- batched queries (the GPU side door next to the per-pattern methods)
     def search_all_batch(self, pats, offs=None):
         """-> (lo, hi) uint32 arrays; the reference's slice for pattern q is sa[lo[q]:hi[q]]."""
-        flat, offs = (pats, offs) if offs is not None else _pack_patterns(pats)
-        flat = np.ascontiguousarray(flat, dtype=np.uint8)
-        offs = np.ascontiguousarray(offs, dtype=np.uint64)
-        np_ = offs.size - 1
+        flat, offs, np_ = _batch_input(pats, offs)
         lo = np.empty(np_, dtype=np.uint32)
         hi = np.empty(np_, dtype=np.uint32)
         _lib.check(_lib.lib().sab200_search_all_batch(self._get_index(), _ptr(flat), _ptr(offs), np_, _ptr(lo), _ptr(hi)),
@@ -213,20 +218,14 @@ class SuffixArray:
         return lo, hi
 
     def contains_batch(self, pats, offs=None):
-        flat, offs = (pats, offs) if offs is not None else _pack_patterns(pats)
-        flat = np.ascontiguousarray(flat, dtype=np.uint8)
-        offs = np.ascontiguousarray(offs, dtype=np.uint64)
-        np_ = offs.size - 1
+        flat, offs, np_ = _batch_input(pats, offs)
         out = np.empty(np_, dtype=np.uint8)
         _lib.check(_lib.lib().sab200_contains_batch(self._get_index(), _ptr(flat), _ptr(offs), np_, _ptr(out)),
                    "sab200_contains_batch")
         return out.astype(bool)
 
     def search_lcp_batch(self, pats, offs=None):
-        flat, offs = (pats, offs) if offs is not None else _pack_patterns(pats)
-        flat = np.ascontiguousarray(flat, dtype=np.uint8)
-        offs = np.ascontiguousarray(offs, dtype=np.uint64)
-        np_ = offs.size - 1
+        flat, offs, np_ = _batch_input(pats, offs)
         st = np.empty(np_, dtype=np.uint32)
         en = np.empty(np_, dtype=np.uint32)
         _lib.check(_lib.lib().sab200_search_lcp_batch(self._get_index(), _ptr(flat), _ptr(offs), np_, _ptr(st), _ptr(en)),
@@ -239,10 +238,7 @@ class SuffixArray:
         query Q, len[i] is the longest prefix of the rest of Q that occurs in the text, and sa[lo[i]:hi[i]] are the
         positions where it occurs ([0, n+1) when len[i] = 0).  The first call on an index builds its extension
         (integrity check, inverse suffix array, LCP array); a suffix array that is not the text's raises ValueError."""
-        flat, offs = (queries, offs) if offs is not None else _pack_patterns(queries)
-        flat = np.ascontiguousarray(flat, dtype=np.uint8)
-        offs = np.ascontiguousarray(offs, dtype=np.uint64)
-        nq = offs.size - 1
+        flat, offs, nq = _batch_input(queries, offs)
         total = int(offs[-1]) if nq > 0 else 0
         out = [np.empty(total, dtype=np.uint32) for _ in range(3)]
         L = _lib.lib()
