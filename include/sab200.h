@@ -128,6 +128,37 @@ int32_t sab200_inverse_bwt(const uint8_t* bwt, uint64_t n, uint64_t primary, uin
 int32_t sab200_bwt_device(const uint8_t* d_s, uint64_t n, uint8_t* d_bwt, uint64_t* primary, int32_t device);
 int32_t sab200_inverse_bwt_device(const uint8_t* d_bwt, uint64_t n, uint64_t primary, uint8_t* d_s, int32_t device);
 
+/* ---- Lempel-Ziv (LZ77) factorization ------------------------------------------------------------
+ * No reference counterpart.  For a text s of n bytes, LPF[i] is the largest l with s[i .. i+l) = s[p .. p+l) for some
+ * p < i (the two may overlap: p + l > i is allowed), 0 when s[i] does not occur before i.  The greedy factorization
+ * has the starts b_0 = 0, b_{t+1} = b_t + max(1, LPF[b_t]), and z factors in all (b_z = n).  Factor t is
+ * (pos[t], len[t]) with len[t] = LPF[b_t]; pos[t] = s[b_t] when len[t] = 0 (a literal), else the SOURCE, fixed so that
+ * the output is deterministic: over the suffix array of sab200_saca (row 0, the empty suffix, is never chosen), with
+ * j the row of suffix b_t, PSV / NSV are the nearest rows before / after j whose suffix starts before b_t, and the source
+ * is whichever of sa[PSV], sa[NSV] shares the longer prefix with suffix b_t, sa[PSV] on a tie.  (LPF[i] is the longer
+ * of these two common prefixes, Crochemore-Ilie.)  Examples:
+ *   "banana" -> (b,0) (a,0) (n,0) (1,3), z = 4;   "aaaa" -> (a,0) (0,3), z = 2;   the empty text -> z = 0.
+ *
+ * sab200_lz77 builds the suffix array on the GPU as sab200_saca does (its statistics stay readable through
+ * sab200_get_stats), then the inverse suffix array, the LCP array (comparing text only where the permuted LCP array is
+ * irreducible: O(n log n) bytes, also on runs such as all-'a' text), LPF and sources at every position, the parse and the
+ * compaction, all in the construction's workspace once the construction is done: device memory is what sab200_saca
+ * takes (the construction workspace, the text and n + 1 suffix-array words: about 37 bytes per byte of text), and the
+ * 8z bytes of output are carved from that workspace.  *z always receives the factor count; when cap < z the call returns SAB200_ERR_ARGS and writes no
+ * factor.  cap = n always suffices.
+ * sab200_lz77_decode returns the n bytes of any valid parse, greedy or not.  It returns SAB200_ERR_ARGS, with
+ * sab200_last_error saying which rule failed, and leaves s unwritten, when the lengths max(1, len[t]) do not sum to n,
+ * a literal has pos > 255, a copy has pos >= b_t, z > n, or n > SAB200_MAX_LENGTH.  Device memory: the input, the
+ * output and 4(z + n) bytes.
+ * Host buffers, pageable or pinned; one GPU. */
+int32_t sab200_lz77(const uint8_t* s, uint64_t n, uint32_t* pos, uint32_t* len, uint64_t cap, uint64_t* z);
+int32_t sab200_lz77_decode(const uint32_t* pos, const uint32_t* len, uint64_t z, uint64_t n, uint8_t* s);
+/* The same with DEVICE buffers already resident on `device`, to time the device work without PCIe. */
+int32_t sab200_lz77_device(const uint8_t* d_s, uint64_t n, uint32_t* d_pos, uint32_t* d_len, uint64_t cap,
+                           uint64_t* z, int32_t device);
+int32_t sab200_lz77_decode_device(const uint32_t* d_pos, const uint32_t* d_len, uint64_t z, uint64_t n,
+                                  uint8_t* d_s, int32_t device);
+
 /* ---- batched queries -----------------------------------------------------------------------
  * A resident copy of (text, SA, optional bucket table) on `ngpus` GPUs (replicated; queries are
  * sharded across the replicas, no collective).  bkt_or_null = NULL means "buckets not enabled"

@@ -13,6 +13,7 @@
 #include <cstdint>
 #include <fstream>
 #include <iterator>
+#include <memory>
 #include <optional>
 #include <stdexcept>
 #include <string>
@@ -63,6 +64,28 @@ inline std::vector<std::uint8_t> inverse_bwt(const std::uint8_t* u, std::size_t 
     const std::int32_t rc = sab200_inverse_bwt(u, n, primary, s.data());
     if (rc == SAB200_ERR_ARGS) throw std::invalid_argument(std::string("sab200_inverse_bwt: ") + sab200_last_error());
     check(rc, "sab200_inverse_bwt");
+    return s;
+}
+
+// Greedy LZ77 factorization (sab200.h): the z factors (pos[t], len[t]); len = 0 is a literal with pos = the byte,
+// otherwise a copy of len bytes from the earlier position pos.  lz77("banana") = (b,0) (a,0) (n,0) (1,3).
+inline std::pair<std::vector<std::uint32_t>, std::vector<std::uint32_t>> lz77(const std::uint8_t* s, std::size_t n) {
+    if (n > MAX_LENGTH) throw std::length_error("text longer than MAX_LENGTH");
+    // cap = n suffices; uninitialised, so only the pages of the z factors are ever touched
+    std::unique_ptr<std::uint32_t[]> pos(new std::uint32_t[n ? n : 1]), len(new std::uint32_t[n ? n : 1]);
+    std::uint64_t z = 0;
+    check(sab200_lz77(s, n, pos.get(), len.get(), n, &z), "sab200_lz77");
+    return {std::vector<std::uint32_t>(pos.get(), pos.get() + z), std::vector<std::uint32_t>(len.get(), len.get() + z)};
+}
+
+// The n bytes of the parse (pos, len), greedy or not; std::invalid_argument when the factors do not parse n bytes.
+inline std::vector<std::uint8_t> lz77_decode(const std::vector<std::uint32_t>& pos, const std::vector<std::uint32_t>& len,
+                                             std::size_t n) {
+    if (pos.size() != len.size()) throw std::invalid_argument("lz77_decode: pos and len differ in length");
+    std::vector<std::uint8_t> s(n);
+    const std::int32_t rc = sab200_lz77_decode(pos.data(), len.data(), pos.size(), n, s.data());
+    if (rc == SAB200_ERR_ARGS) throw std::invalid_argument(std::string("sab200_lz77_decode: ") + sab200_last_error());
+    check(rc, "sab200_lz77_decode");
     return s;
 }
 

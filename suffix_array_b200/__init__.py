@@ -4,6 +4,6 @@ src/sa.rs).  The CUDA engine (csrc/, sm_100a) sits behind the C ABI of include/s
 package is the thin host mirror of the reference's `SuffixArray` interface.
 """
 from ._lib import MAX_LENGTH, BKT_LEN, SabError, build, last_stats, lib, require_gpu
-from .sa import SuffixArray, bwt, inverse_bwt, saca
+from .sa import SuffixArray, bwt, inverse_bwt, lz77, lz77_decode, saca
 
-__all__ = ["SuffixArray", "saca", "bwt", "inverse_bwt", "MAX_LENGTH", "BKT_LEN", "SabError", "build", "last_stats", "lib", "require_gpu"]
+__all__ = ["SuffixArray", "saca", "bwt", "inverse_bwt", "lz77", "lz77_decode", "MAX_LENGTH", "BKT_LEN", "SabError", "build", "last_stats", "lib", "require_gpu"]

@@ -132,6 +132,10 @@ def _bind(L):
         "sab200_inverse_bwt": ([vp, u64, u64, vp], i32),
         "sab200_bwt_device": ([vp, u64, vp, C.POINTER(u64), i32], i32),
         "sab200_inverse_bwt_device": ([vp, u64, u64, vp, i32], i32),
+        "sab200_lz77": ([vp, u64, vp, vp, u64, C.POINTER(u64)], i32),
+        "sab200_lz77_decode": ([vp, vp, u64, u64, vp], i32),
+        "sab200_lz77_device": ([vp, u64, vp, vp, u64, C.POINTER(u64), i32], i32),
+        "sab200_lz77_decode_device": ([vp, vp, u64, u64, vp, i32], i32),
         "sab200_index_create": ([vp, u64, vp, u64, vp, i32], vp),
         "sab200_index_destroy": ([vp], None),
         "sab200_search_all_batch": ([vp, vp, vp, u64, vp, vp], i32),

@@ -7,6 +7,7 @@
 #include "sab_search.cuh"
 #include "sab_pack.cuh"
 #include "sab_bwt.cuh"
+#include "sab_lz.cuh"
 
 #include <chrono>
 #include <cstdlib>
@@ -571,6 +572,121 @@ extern "C" int32_t sab200_inverse_bwt_device(const uint8_t* d_bwt, uint64_t n, u
     SAB_TRY(sab_use(device, &u));
     if (n == 0) return SAB_OK;
     return inverse_bwt_run(u.c, d_bwt, n, primary, d_s);
+}
+
+// ---- Lempel-Ziv factorization ----------------------------------------------------------------
+// The construction, then the parse in its workspace d_work (dead once the construction is done).  The construction's
+// statistics stay readable.  *d_pos / *d_len: the z factors, inside the workspace.
+static int lz77_forward(SabContext* c, const u8* d_s, u64 n, u32* d_sa, char* d_work, u32** d_pos, u32** d_len, u64* z) {
+    const int rc = run_device(c, d_s, n, d_sa);
+    g_last_stats = c->stats;
+    SAB_TRY(rc);
+    *z = 0;
+    if (n == 0) return SAB_OK;
+    return sab_lz77_parse(c, d_s, n, d_sa, d_work, d_pos, d_len, z);
+}
+
+static bool lz77_bad_args(const char* who, const void* s, uint64_t n, const void* pos, const void* len, uint64_t cap, const void* z) {
+    if (!z || (n > 0 && !s) || (cap > 0 && (!pos || !len)) || n > SAB200_MAX_LENGTH) {
+        sab_set_error("%s: bad arguments (n=%llu, cap=%llu)", who, (unsigned long long)n, (unsigned long long)cap);
+        return true;
+    }
+    return false;
+}
+
+static bool lz77_short_cap(const char* who, uint64_t z, uint64_t cap) {
+    if (cap >= z) return false;
+    sab_set_error("%s: %llu factors, room for %llu", who, (unsigned long long)z, (unsigned long long)cap);
+    return true;
+}
+
+extern "C" int32_t sab200_lz77(const uint8_t* s, uint64_t n, uint32_t* pos, uint32_t* len, uint64_t cap, uint64_t* z) {
+    if (lz77_bad_args("sab200_lz77", s, n, pos, len, cap, z)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    SabContext* c = u.c;
+    char* d_work;
+    u8* d_s;
+    u32* d_sa;
+    SAB_TRY(sab_arena_carve(c, {{&d_work, sab_saca_workspace_bytes(n)}, {&d_s, (size_t)n + 64}, {&d_sa, ((size_t)n + 1) * sizeof(u32)}}));
+    SAB_TRY(sab_copy_h2d(c, d_s, s, n));
+    u32 *d_pos = nullptr, *d_len = nullptr;
+    SAB_TRY(lz77_forward(c, d_s, n, d_sa, d_work, &d_pos, &d_len, z));
+    if (lz77_short_cap("sab200_lz77", *z, cap)) return SAB_ERR_ARGS;
+    SAB_TRY(sab_copy_d2h(c, pos, d_pos, *z * sizeof(u32)));
+    return sab_copy_d2h(c, len, d_len, *z * sizeof(u32));
+}
+
+extern "C" int32_t sab200_lz77_device(const uint8_t* d_s, uint64_t n, uint32_t* d_pos, uint32_t* d_len, uint64_t cap, uint64_t* z,
+                                      int32_t device) {
+    if (lz77_bad_args("sab200_lz77_device", d_s, n, d_pos, d_len, cap, z)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    SabContext* c = u.c;
+    char* d_work;
+    u32* d_sa;
+    SAB_TRY(sab_arena_carve(c, {{&d_work, sab_saca_workspace_bytes(n)}, {&d_sa, ((size_t)n + 1) * sizeof(u32)}}));
+    u32 *w_pos = nullptr, *w_len = nullptr;
+    SAB_TRY(lz77_forward(c, d_s, n, d_sa, d_work, &w_pos, &w_len, z));
+    if (lz77_short_cap("sab200_lz77_device", *z, cap)) return SAB_ERR_ARGS;
+    if (*z) {
+        SAB_CUDA_TRY(cudaMemcpyAsync(d_pos, w_pos, *z * sizeof(u32), cudaMemcpyDeviceToDevice, c->stream));
+        SAB_CUDA_TRY(cudaMemcpyAsync(d_len, w_len, *z * sizeof(u32), cudaMemcpyDeviceToDevice, c->stream));
+    }
+    SAB_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return SAB_OK;
+}
+
+// the checks the host can make before any device work
+static bool lz77_decode_bad_args(const char* who, const void* pos, const void* len, uint64_t z, uint64_t n, const void* s) {
+    if ((z > 0 && (!pos || !len)) || (n > 0 && !s)) {
+        sab_set_error("%s: bad arguments (z=%llu, n=%llu)", who, (unsigned long long)z, (unsigned long long)n);
+        return true;
+    }
+    if (n > SAB200_MAX_LENGTH) {
+        sab_set_error("%s: n = %llu exceeds SAB200_MAX_LENGTH", who, (unsigned long long)n);
+        return true;
+    }
+    if (z > n) {
+        sab_set_error("%s: %llu factors cannot parse %llu bytes (z > n)", who, (unsigned long long)z, (unsigned long long)n);
+        return true;
+    }
+    if (z == 0 && n > 0) {
+        sab_set_error("%s: the factor lengths (max(1, len) each) sum to 0, not to n = %llu", who, (unsigned long long)n);
+        return true;
+    }
+    return false;
+}
+
+static int lz77_decode_run(SabContext* c, const u32* d_pos, const u32* d_len, u64 z, u64 n, u8* d_s) {
+    const int rc = sab_lz77_decode_run(c, d_pos, d_len, z, n, d_s);
+    if (rc != SAB_OK && rc != SAB_ERR_ARGS) sab_reset_after_failure(c);
+    return rc;
+}
+
+extern "C" int32_t sab200_lz77_decode(const uint32_t* pos, const uint32_t* len, uint64_t z, uint64_t n, uint8_t* s) {
+    if (lz77_decode_bad_args("sab200_lz77_decode", pos, len, z, n, s)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(0, &u));
+    if (n == 0) return SAB_OK;
+    SabContext* c = u.c;
+    u32 *d_pos, *d_len;
+    u8* d_s;
+    SAB_TRY(sab_arena_carve(c, {{nullptr, sab_lz77_decode_workspace_bytes(z, n)}, {&d_pos, (size_t)z * 4}, {&d_len, (size_t)z * 4},
+                                {&d_s, (size_t)n + 64}}));
+    SAB_TRY(sab_copy_h2d(c, d_pos, pos, z * 4));
+    SAB_TRY(sab_copy_h2d(c, d_len, len, z * 4));
+    SAB_TRY(lz77_decode_run(c, d_pos, d_len, z, n, d_s));
+    return sab_copy_d2h(c, s, d_s, n);
+}
+
+extern "C" int32_t sab200_lz77_decode_device(const uint32_t* d_pos, const uint32_t* d_len, uint64_t z, uint64_t n, uint8_t* d_s,
+                                             int32_t device) {
+    if (lz77_decode_bad_args("sab200_lz77_decode_device", d_pos, d_len, z, n, d_s)) return SAB_ERR_ARGS;
+    SabUse u;
+    SAB_TRY(sab_use(device, &u));
+    if (n == 0) return SAB_OK;
+    return lz77_decode_run(u.c, d_pos, d_len, z, n, d_s);
 }
 
 // ---- pack serialisation ---------------------------------------------------------------------

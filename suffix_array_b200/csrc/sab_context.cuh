@@ -58,6 +58,7 @@ struct SabScratch {
     u16 lut[256];   // code table of the running construction (sab_plan_alphabet)
     u32 bwt[2];     // sab200_bwt: the primary index; sab200_inverse_bwt: sample rows, list position of row p
     u32 ms_offs;    // sab200_matching_statistics_batch_device: set when the query offsets decrease
+    u32 lz[4];      // sab200_lz77: the factor count; sab200_lz77_decode: rule flags, factor total (2 words), round changed
 };
 
 // Pinned host staging of a context: readbacks land here, and small uploads leave from here, not from the caller's stack.

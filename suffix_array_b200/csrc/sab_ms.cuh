@@ -83,8 +83,11 @@ __device__ __forceinline__ u64 ms_first_below(const u32* __restrict__ v, u64 lo,
 }
 
 // LCP interval [a, b) of length l >= 1 around rank r (the suffix at r has at least l bytes): a = largest j <= r with
-// lcp[j] < l (lcp[0] = 0, so it exists), b = smallest j > r with lcp[j] < l, or n + 1
-__device__ __forceinline__ u64 ms_left(const MsArgs& a, u64 r, u64 l, u32 lane) {
+// lcp[j] < l (lcp[0] = 0, so it exists), b = smallest j > r with lcp[j] < l, or n + 1.
+// Levels: any type with the lvl / cnt / top members of MsArgs, a block-minimum hierarchy over lvl[0].  Over another
+// array ms_left returns 0 when no entry of [0, r] is below l.
+template <typename Levels>
+__device__ __forceinline__ u64 ms_left(const Levels& a, u64 r, u64 l, u32 lane) {
     u64 j = ms_last_below(a.lvl[0], r & ~255ull, r, l, lane);
     if (j != SAB_MS_NONE) return j;
     u32 k = 1;
@@ -99,7 +102,8 @@ __device__ __forceinline__ u64 ms_left(const MsArgs& a, u64 r, u64 l, u32 lane) 
     return j;
 }
 
-__device__ __forceinline__ u64 ms_right(const MsArgs& a, u64 r, u64 l, u32 lane) {
+template <typename Levels>
+__device__ __forceinline__ u64 ms_right(const Levels& a, u64 r, u64 l, u32 lane) {
     const u64 end0 = (r | 255) < a.cnt[0] ? (r | 255) : a.cnt[0] - 1;
     u64 j = r < end0 ? ms_first_below(a.lvl[0], r + 1, end0, l, lane) : SAB_MS_NONE;
     if (j != SAB_MS_NONE) return j;

@@ -30,6 +30,11 @@ extern "C" {
     pub fn sab200_inverse_bwt(bwt: *const u8, n: u64, primary: u64, s: *mut u8) -> i32;
     pub fn sab200_bwt_device(d_s: *const u8, n: u64, d_bwt: *mut u8, primary: *mut u64, device: i32) -> i32;
     pub fn sab200_inverse_bwt_device(d_bwt: *const u8, n: u64, primary: u64, d_s: *mut u8, device: i32) -> i32;
+    // LZ77 factorization: z factors (pos, len), len = 0 a literal; *z is reported even when cap < z (include/sab200.h)
+    pub fn sab200_lz77(s: *const u8, n: u64, pos: *mut u32, len: *mut u32, cap: u64, z: *mut u64) -> i32;
+    pub fn sab200_lz77_decode(pos: *const u32, len: *const u32, z: u64, n: u64, s: *mut u8) -> i32;
+    pub fn sab200_lz77_device(d_s: *const u8, n: u64, d_pos: *mut u32, d_len: *mut u32, cap: u64, z: *mut u64, device: i32) -> i32;
+    pub fn sab200_lz77_decode_device(d_pos: *const u32, d_len: *const u32, z: u64, n: u64, d_s: *mut u8, device: i32) -> i32;
     pub fn sab200_device_count() -> i32;
     pub fn sab200_last_error() -> *const c_char;
     pub fn sab200_shutdown();

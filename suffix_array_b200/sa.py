@@ -82,6 +82,40 @@ def inverse_bwt(u, primary):
     return out
 
 
+def lz77(s):
+    """Greedy LZ77 factorization of `s` (include/sab200.h): -> (pos, len), uint32 arrays of the z factors.  Factor t
+    is a literal (pos = the byte) when len = 0, else a copy of len bytes from the earlier position pos (the source may
+    overlap the factor).  lz77(b"banana") gives pos [98, 97, 110, 1], len [0, 0, 0, 3].  Suffix array, LPF and parse
+    are computed on the GPU; only the factors come back."""
+    t = _as_text(s)
+    assert t.size <= MAX_LENGTH
+    pos = np.empty(t.size, dtype=np.uint32)  # cap = n always suffices; untouched pages are never committed
+    ln = np.empty(t.size, dtype=np.uint32)
+    z = C.c_uint64()
+    L = _lib.require_gpu()
+    _lib.check(L.sab200_lz77(_ptr(t), t.size, _ptr(pos), _ptr(ln), t.size, C.byref(z)), "sab200_lz77")
+    return pos[:z.value].copy(), ln[:z.value].copy()
+
+
+def lz77_decode(pos, len, n):
+    """The n bytes of the parse (pos, len), greedy or not, as a uint8 array.  Raises ValueError when the factors do not
+    parse n bytes: lengths max(1, len) not summing to n, a literal above 255, a copy whose source is not before it."""
+    p = np.ascontiguousarray(pos, dtype=np.uint32)
+    ln = np.ascontiguousarray(len, dtype=np.uint32)
+    n = int(n)
+    if p.shape != ln.shape or p.ndim != 1:
+        raise ValueError("pos and len must be 1-D arrays of the same length")
+    if not 0 <= n <= MAX_LENGTH:
+        raise ValueError("n = %d outside [0, MAX_LENGTH]" % n)
+    out = np.empty(n, dtype=np.uint8)
+    L = _lib.require_gpu()
+    rc = L.sab200_lz77_decode(_ptr(p), _ptr(ln), p.size, n, _ptr(out))
+    if rc == -1:
+        raise ValueError(L.sab200_last_error().decode("utf-8", "replace"))
+    _lib.check(rc, "sab200_lz77_decode")
+    return out
+
+
 class SuffixArray:
     """Suffix array for a byte string (src/sa.rs:14-19): text `s`, `sa` of n+1 u32, optional buckets."""
 
